@@ -142,6 +142,22 @@ def executed_table(workload):
         return None
 
 
+def dump_outputs(out_dir, frame, max_pixels=1 << 21):
+    """Writes the frame the last timed step rendered so that two builds can be compared output for output:
+    frame_rgb.npy (float32 [n, 3], the 0..255 R, G, B of each pixel) and frame_pixel_index.npy (float64 [n], y * W + x).
+    n is every pixel up to max_pixels, else a fixed seeded sample of that many (40 MiB in all at most)."""
+    os.makedirs(out_dir, exist_ok=True)
+    flat = frame.reshape(-1)
+    if flat.size <= max_pixels:
+        idx = np.arange(flat.size)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(flat.size, max_pixels, replace=False))
+    px = flat[idx]
+    rgb = np.stack([(px >> 16) & 255, (px >> 8) & 255, px & 255], axis=1).astype(np.float32)
+    np.save(os.path.join(out_dir, "frame_rgb.npy"), rgb)
+    np.save(os.path.join(out_dir, "frame_pixel_index.npy"), idx.astype(np.float64))
+
+
 def dist_env():
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -229,7 +245,12 @@ def main():
     ap.add_argument("--diag-local-frames", action="store_true",
                     help="diagnostic, N > 1: every rank stores its rows into its own memory instead of the presenter's frame "
                          "(no NVLink stores; the frame is never assembled and the line says so)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours: after the timed steps, write the frame the last of them rendered to DIR/*.npy "
+                         "(see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.emulate_world > 1 or args.diag_local_frames):
+        ap.error("--dump-outputs writes whole frames; --emulate-world and --diag-local-frames never assemble one")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, local, world = dist_env()
 
@@ -346,6 +367,12 @@ def main():
     barrier()
     t_end = time.perf_counter()
     clocks = sampler.stop(t_begin, t_end)
+    last_frame = None
+    if args.dump_outputs and rank == 0:
+        # the presenter's ring slot of the last timed frame: every rank's rows have landed (barrier above) and no
+        # later frame has been submitted yet
+        last_frame = np.empty((H, W), dtype=np.uint32)
+        r.copy_to_host(last_frame, peer.ptrs[(peer.submitted - 1) % peer.n_buffers])
     my_ms = ev_start.elapsed_time(ev_end)
     per_rank_ms = [my_ms]
     total_ms = torch.tensor([my_ms], dtype=torch.float64, device=dev)
@@ -722,6 +749,8 @@ def main():
             "cpu_baseline": cpu,
         }
         line.update(extras)
+        if last_frame is not None:
+            dump_outputs(args.dump_outputs, last_frame)
         sys.stdout.flush()
         os.dup2(saved_stdout, 1)
         print(json.dumps(line))

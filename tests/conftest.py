@@ -32,7 +32,8 @@ def oracle_ref():
     import oraclelib
 
     if not oraclelib.have_ref():
-        pytest.skip("oracle/_ref not built (the reference tree only exists in the build container)")
+        pytest.skip("oracle/_ref not built: build() makes it where it finds the original project's source "
+                    "(ORE_REFERENCE_DIR, see oracle/ref_build/make_ref.py)")
     return oraclelib.load("ref")
 
 

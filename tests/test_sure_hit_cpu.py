@@ -8,6 +8,8 @@ numpy restatement of that function (itself checked against the C oracle on a sub
 adversarial families: grazing rays, origins on / just off the surface, tiny and huge spheres, far origins,
 directions whose squared length is off by up to 5e-6 (the kernel's admission limit).
 """
+import os
+
 import numpy as np
 import pytest
 
@@ -91,6 +93,18 @@ def test_numpy_restatement_matches_the_references_own_code(oracle_ref):
     for name, O, D, Cn, rad in families(rng, 400):
         want = np.array([oracle_ref.sphere_intersect(O[i], D[i], Cn[i], rad[i])[0] for i in range(len(rad))])
         assert np.array_equal(ref_hit(O, D, Cn, rad), want), name
+
+
+def test_numpy_restatement_and_sure_hits_agree_with_the_stored_reference_answers():
+    """ref_hit and sure_hit against the answers the reference's own sphere::intersect gave for the 4096 rays of
+    tests/golden/intersect_kat.npz (stored, so this runs without the reference's source).  Those rays are generic, not
+    the adversarial families: on the families sure_hit is checked against ref_hit, and ref_hit against the C oracle."""
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "intersect_kat.npz"))
+    O, D, Cn, rad, hit = g["org"], g["dir"], g["centre"], g["radius"], g["hit"].astype(bool)
+    assert np.array_equal(ref_hit(O, D, Cn, rad), hit)
+    sure = sure_hit(O, D, Cn, rad)
+    assert np.count_nonzero(sure) > 500
+    assert not np.any(sure & ~hit)
 
 
 def test_every_sure_hit_sample_is_a_hit_of_the_references_own_code(oracle_ref):
