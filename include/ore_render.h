@@ -135,6 +135,21 @@ int ore_set_spheres(ore_context* ctx, const float* xyz_radius, int32_t n);
 /* Same, from the reference's own 32-byte AoS records (vptr@0, orgin@8, reflective@20,
  * radius@24; `sizeof(float)*8` per sphere, kernel.cu:1218-1220). */
 int ore_set_spheres_aos32(ore_context* ctx, const void* records, int32_t n);
+/* Stream-ordered sphere update from DEVICE memory (an animated scene: a simulation or a torch model moving the spheres
+ * on the GPU).  `xyz_radius_dev`: n records of cx, cy, cz, radius member - the meaning of ore_set_spheres - in device
+ * memory of the context's GPU, 16-byte aligned (NULL allowed when n == 0).  Host memory, another GPU's memory, a
+ * misaligned pointer or n < 0 return ORE_ERR_INVALID and change nothing.
+ *   Ordering: the update is enqueued on `stream` (a cudaStream_t, NULL = the context's render stream).  It runs after
+ *   every render already submitted through this context and after the previous update, on whatever streams they ran,
+ *   and every render or scene setter submitted afterwards, on any stream, sees the new spheres.
+ *   Host blocking: none, unless n needs more room than every earlier upload of this context: the scene buffers then
+ *   grow, which first waits on the host for the last render and the last update.  A caller that sizes the buffers
+ *   once with its largest n (one call with that n) never blocks afterwards.
+ *   Caller's buffer: it must stay allocated and unchanged until the update has run on `stream` (the rules of
+ *   cudaMemcpyAsync); the context does not keep it.
+ *   Result: the device arrays are bit-identical to what ore_set_spheres builds for the same values, so every result
+ *   guarantee of the render calls holds unchanged. */
+int ore_set_spheres_device(ore_context* ctx, const float* xyz_radius_dev, int32_t n, void* stream);
 /* "Next" primitives of castRay / castLightRay (SURVEY.md 8f N1).  The reference ships both counts at 0
  * (kernel.cu:1231).  Hit ids continue after the spheres: cube i -> n_spheres + i, plane i -> n_spheres +
  * n_cubes + i.  Exact tests, no filters: meant for the handful of objects the reference would hold.
@@ -255,6 +270,12 @@ int ore_measure_fp32_peak(ore_context* ctx, double* tflops, double* sm_clock_mhz
  * op 0 cosf(a), 1 sinf(a), 2 acosf(a), 3 atan2f(a, b).  The path's versions return glibc's bits (ore_libm.cuh).
  * op 4, 5, 6: x, y, z of the path's normalise() applied to (a[i], b[i], a[(i + 1) % n]) - IEEE x / |v| bit for bit. */
 int ore_debug_libm(ore_context* ctx, int op, int n, const float* a_host, const float* b_host, float* out_host);
+/* Tests only: synchronises the device and copies one array of the sphere hierarchy to the host.  which: 0 records in
+ * original order (max(n, 1) float4), 1 exact records sorted (n_sort float4), 2 shadow records cx,cy,cz,R' sorted
+ * (n_sort float4), 3 sorted position -> original index (n_sort int32), 4 leaf balls (n_leaves_pad float4), 5 super-
+ * cluster balls (n_supers_pad float4); n_sort = 32 ceil(n / 32) (32 when n = 0), n_leaves_pad = ceil(n / 8) rounded up
+ * to a multiple of 32, n_supers_pad = ceil(n / 256) rounded up to a multiple of 4.  n_items must be that length. */
+int ore_debug_sphere_tree(ore_context* ctx, int32_t which, void* host_out, int32_t n_items);
 
 #ifdef __cplusplus
 }

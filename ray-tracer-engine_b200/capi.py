@@ -29,7 +29,20 @@ EXPORTS = [
     "ore_dev_alloc", "ore_dev_free", "ore_ipc_export", "ore_ipc_import", "ore_ipc_close", "ore_copy_to_host",
     "ore_render_async_signal", "ore_host_register", "ore_host_unregister", "ore_flag_write", "ore_flag_wait_geq",
     "ore_flag_write_after", "ore_get_stream", "ore_render_batch_device", "ore_render_batch_async",
+    "ore_set_spheres_device", "ore_debug_sphere_tree",
 ]
+
+# ore_debug_sphere_tree: which array of the sphere hierarchy, and its element type
+SPHERE_TREE_ARRAYS = {"sph_exact": 0, "sph_xsort": 1, "sph_sort": 2, "sort_index": 3, "leaf_sph": 4, "super_sph": 5}
+
+
+def sphere_tree_lengths(n: int) -> dict:
+    """item counts of the six hierarchy arrays for n spheres (include/ore_render.h, ore_debug_sphere_tree)"""
+    n_sort = max(1, (n + 31) // 32) * 32
+    n_leaf = (n + 7) // 8
+    n_sup = (n_leaf + 31) // 32
+    return {"sph_exact": max(n, 1), "sph_xsort": n_sort, "sph_sort": n_sort, "sort_index": n_sort,
+            "leaf_sph": (n_leaf + 31) // 32 * 32, "super_sph": (n_sup + 3) // 4 * 4}
 
 
 class OreCamera(C.Structure):
@@ -72,6 +85,8 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.ore_last_error.restype = C.c_char_p
     lib.ore_set_spheres.argtypes = [vp, fp, i32]
     lib.ore_set_spheres_aos32.argtypes = [vp, vp, i32]
+    lib.ore_set_spheres_device.argtypes = [vp, vp, i32, vp]
+    lib.ore_debug_sphere_tree.argtypes = [vp, i32, vp, i32]
     lib.ore_set_lights.argtypes = [vp, fp, i32]
     lib.ore_set_cubes.argtypes = [vp, fp, i32]
     lib.ore_set_planes.argtypes = [vp, fp, i32]
@@ -160,6 +175,35 @@ class Renderer:
         a = np.ascontiguousarray(records)
         assert a.nbytes % 32 == 0
         self._check(self.lib.ore_set_spheres_aos32(self.ctx, a.ctypes.data, a.nbytes // 32), "ore_set_spheres_aos32")
+
+    def set_spheres_device(self, t, stream: int = 0):
+        """Stream-ordered sphere update from a torch CUDA float32 tensor of shape (n, 4) (cx, cy, cz, radius member) on
+        this context's GPU.  `stream`: a raw cudaStream_t (e.g. torch.cuda.current_stream().cuda_stream; 0 = the
+        context's render stream).  Keep `t` alive and unchanged until the update has run on that stream."""
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"set_spheres_device: expected a torch.Tensor, got {type(t).__name__}")
+        if t.dtype != torch.float32:
+            raise TypeError(f"set_spheres_device: expected dtype torch.float32, got {t.dtype}")
+        if t.dim() != 2 or t.shape[1] != 4:
+            raise ValueError(f"set_spheres_device: expected shape (n, 4), got {tuple(t.shape)}")
+        if t.device.type != "cuda" or t.device.index != self.device:
+            raise ValueError(f"set_spheres_device: the tensor must live on cuda:{self.device}, not {t.device}")
+        if not t.is_contiguous():
+            raise ValueError("set_spheres_device: the tensor must be contiguous")
+        n = int(t.shape[0])
+        ptr = t.data_ptr() if n else 0
+        self._check(self.lib.ore_set_spheres_device(self.ctx, C.c_void_p(ptr) if ptr else None, n,
+                                                     C.c_void_p(stream) if stream else None), "ore_set_spheres_device")
+
+    def debug_sphere_tree(self, which: str, n: int) -> np.ndarray:
+        """one array of the sphere hierarchy of the current n-sphere scene, read back after a device synchronise
+        (tests): float32 (len, 4), or int32 (len,) for sort_index"""
+        length = sphere_tree_lengths(n)[which]
+        out = np.zeros(length, np.int32) if which == "sort_index" else np.zeros((length, 4), np.float32)
+        self._check(self.lib.ore_debug_sphere_tree(self.ctx, SPHERE_TREE_ARRAYS[which], out.ctypes.data if length else None,
+                                                   length), "ore_debug_sphere_tree")
+        return out
 
     def set_cubes(self, c1_c2: np.ndarray):
         a = np.ascontiguousarray(c1_c2, dtype=np.float32).reshape(-1, 6)

@@ -9,6 +9,7 @@
 //   shadow_sweep_kernel (ore_sweep.cuh)   stage B: any-hit sweep per light, light accumulation, packed pixel
 //                                         (kernel.cu:1470-1544, 1673-1684)
 #pragma once
+#include "ore_clusters.h"   // ORE_KAPPA_SHADOW (the margin R' is rounded up for)
 #include "ore_device.cuh"
 
 namespace ore {
@@ -27,7 +28,6 @@ constexpr int STAGE_A_THREADS = ORE_STAGE_A_THREADS;
 constexpr int TILE_P = ORE_TILE_P;
 
 // conservative filter margins (see DESIGN.md "Filter soundness")
-#define ORE_KAPPA_SHADOW 3.814697265625e-06f /* 2^-18 */
 #define ORE_KAPPA_PRIMARY 7.62939453125e-06  /* 2^-17 */
 #define ORE_BIG 3.0e38f
 
