@@ -170,6 +170,20 @@ int ore_set_planes(ore_context* ctx, const float* pos_normal, int32_t n);
  * Exact tests, linear scan over the leaves per ray like the reference (kernel.cu:1293-1328,1475-1497). */
 int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tris, int32_t has_normals, const float* box_bounds6,
                  const int32_t* box_offsets, const int32_t* box_indices, int32_t n_boxes);
+/* Stream-ordered update of the mesh's triangles from DEVICE memory (a deforming mesh: skinning, cloth, a displaced
+ * height field computed on the GPU).  `tris27_dev`: n_tris x 27 floats - the meaning of ore_set_mesh's tris27 - in
+ * device memory of the context's GPU, 4-byte aligned.  The topology of the last ore_set_mesh stays: has_normals,
+ * box_offsets and box_indices; n_tris must equal its triangle count.  No mesh set, a wrong n_tris, a NULL, misaligned
+ * or host pointer, or another GPU's memory return ORE_ERR_INVALID and change nothing.
+ *   Leaf boxes: recomputed on the GPU from the new triangles by the reference builder's rule (getMinMaxP,
+ *   kernel.cu:973-997): lo seeded with the first listed triangle's first vertex, hi with the last listed triangle's
+ *   first vertex, then every vertex of every listed triangle grows them in list order with strict > / <.  A leaf that
+ *   lists no triangle keeps its box.  Their bounding spheres follow by the formula ore_set_mesh uses.
+ *   Ordering and host blocking: as ore_set_spheres_device (the same events).  The update is enqueued on `stream`
+ *   (NULL = the context's render stream) after every render already submitted and the previous update; renders
+ *   submitted afterwards, on any stream, see the new triangles.  The host never blocks: nothing grows.
+ *   Caller's buffer: it must stay allocated and unchanged until the update has run on `stream`. */
+int ore_set_mesh_triangles_device(ore_context* ctx, const float* tris27_dev, int32_t n_tris, void* stream);
 /* Replaces cudaMalloc+cudaMemcpy of `lights` in update() (kernel.cu:1776-1778):
  * n x {pos.xyz, size, r, g, b} (kernel.cu:1246-1261). */
 int ore_set_lights(ore_context* ctx, const float* lights7, int32_t n);
@@ -276,6 +290,10 @@ int ore_debug_libm(ore_context* ctx, int op, int n, const float* a_host, const f
  * cluster balls (n_supers_pad float4); n_sort = 32 ceil(n / 32) (32 when n = 0), n_leaves_pad = ceil(n / 8) rounded up
  * to a multiple of 32, n_supers_pad = ceil(n / 256) rounded up to a multiple of 4.  n_items must be that length. */
 int ore_debug_sphere_tree(ore_context* ctx, int32_t which, void* host_out, int32_t n_items);
+/* Tests only: synchronises the device and copies one array of the mesh to the host.  which: 0 triangles (n_tris * 27
+ * floats), 1 leaf boxes lo, hi (2 * n_boxes float4, .w = 0), 2 leaf bounding spheres (n_boxes float4).  n_items must be
+ * that length. */
+int ore_debug_mesh(ore_context* ctx, int32_t which, void* host_out, int32_t n_items);
 
 #ifdef __cplusplus
 }

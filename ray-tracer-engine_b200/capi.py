@@ -29,11 +29,15 @@ EXPORTS = [
     "ore_dev_alloc", "ore_dev_free", "ore_ipc_export", "ore_ipc_import", "ore_ipc_close", "ore_copy_to_host",
     "ore_render_async_signal", "ore_host_register", "ore_host_unregister", "ore_flag_write", "ore_flag_wait_geq",
     "ore_flag_write_after", "ore_get_stream", "ore_render_batch_device", "ore_render_batch_async",
-    "ore_set_spheres_device", "ore_debug_sphere_tree",
+    "ore_set_spheres_device", "ore_debug_sphere_tree", "ore_set_mesh_triangles_device", "ore_debug_mesh",
 ]
 
 # ore_debug_sphere_tree: which array of the sphere hierarchy, and its element type
 SPHERE_TREE_ARRAYS = {"sph_exact": 0, "sph_xsort": 1, "sph_sort": 2, "sort_index": 3, "leaf_sph": 4, "super_sph": 5}
+
+
+# ore_debug_mesh: which array of the mesh
+MESH_ARRAYS = {"tris": 0, "boxes": 1, "box_sph": 2}
 
 
 def sphere_tree_lengths(n: int) -> dict:
@@ -92,6 +96,8 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.ore_set_planes.argtypes = [vp, fp, i32]
     ip = C.POINTER(C.c_int32)
     lib.ore_set_mesh.argtypes = [vp, fp, i32, i32, fp, ip, ip, i32]
+    lib.ore_set_mesh_triangles_device.argtypes = [vp, vp, i32, vp]
+    lib.ore_debug_mesh.argtypes = [vp, i32, vp, i32]
     lib.ore_set_texture.argtypes = [vp, fp, fp, fp, i32, i32]
     lib.ore_set_sky.argtypes = [vp, fp, fp, fp, i32, i32, C.c_float]
     lib.ore_render.argtypes = [vp, C.POINTER(OreCamera), C.POINTER(OreFrame), vp]
@@ -218,10 +224,43 @@ class Renderer:
         ip = C.POINTER(C.c_int32)
         if mesh is None or mesh.n_tris == 0:
             self._check(self.lib.ore_set_mesh(self.ctx, None, 0, 0, None, None, None, 0), "ore_set_mesh")
+            self._mesh_counts = (0, 0)
             return
         self._check(self.lib.ore_set_mesh(self.ctx, _fptr(mesh.tris.reshape(-1)), mesh.n_tris, int(mesh.has_normals),
                                           _fptr(mesh.box_bounds.reshape(-1)), mesh.box_offsets.ctypes.data_as(ip),
                                           mesh.box_indices.ctypes.data_as(ip), mesh.n_boxes), "ore_set_mesh")
+        self._mesh_counts = (mesh.n_tris, mesh.n_boxes) if mesh.n_boxes else (0, 0)   # (no leaves: no mesh)
+
+    def set_mesh_triangles_device(self, t, stream: int = 0):
+        """Stream-ordered update of the mesh's triangles from a torch CUDA float32 tensor of shape (n_tris, 27) (the
+        records of set_mesh) on this context's GPU; the leaf boxes and their spheres are recomputed on the GPU and the
+        topology of the last set_mesh stays.  `stream`: a raw cudaStream_t (0 = the context's render stream).  Keep `t`
+        alive and unchanged until the update has run on that stream."""
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"set_mesh_triangles_device: expected a torch.Tensor, got {type(t).__name__}")
+        if t.dtype != torch.float32:
+            raise TypeError(f"set_mesh_triangles_device: expected dtype torch.float32, got {t.dtype}")
+        n_tris = getattr(self, "_mesh_counts", (0, 0))[0]
+        if t.dim() != 2 or t.shape[1] != 27 or t.shape[0] != n_tris:
+            raise ValueError(f"set_mesh_triangles_device: expected shape ({n_tris}, 27), got {tuple(t.shape)}")
+        if t.device.type != "cuda" or t.device.index != self.device:
+            raise ValueError(f"set_mesh_triangles_device: the tensor must live on cuda:{self.device}, not {t.device}")
+        if not t.is_contiguous():
+            raise ValueError("set_mesh_triangles_device: the tensor must be contiguous")
+        self._check(self.lib.ore_set_mesh_triangles_device(self.ctx, C.c_void_p(t.data_ptr()), n_tris,
+                                                           C.c_void_p(stream) if stream else None),
+                    "ore_set_mesh_triangles_device")
+
+    def debug_mesh(self, which: str) -> np.ndarray:
+        """one array of the current mesh, read back after a device synchronise (tests): tris float32 (n_tris, 27), boxes
+        float32 (2 * n_boxes, 4) (lo, hi per leaf), box_sph float32 (n_boxes, 4)"""
+        n_tris, n_boxes = getattr(self, "_mesh_counts", (0, 0))
+        out = {"tris": lambda: np.zeros((n_tris, 27), np.float32), "boxes": lambda: np.zeros((2 * n_boxes, 4), np.float32),
+               "box_sph": lambda: np.zeros((n_boxes, 4), np.float32)}[which]()
+        self._check(self.lib.ore_debug_mesh(self.ctx, MESH_ARRAYS[which], out.ctypes.data if out.size else None,
+                                            out.size if which == "tris" else out.shape[0]), "ore_debug_mesh")
+        return out
 
     def set_lights(self, lights7: np.ndarray):
         a = np.ascontiguousarray(lights7, dtype=np.float32).reshape(-1, 7)

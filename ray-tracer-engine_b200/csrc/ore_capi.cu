@@ -19,6 +19,7 @@
 #include "../../include/ore_render.h"
 #include "ore_clusters.h"
 #include "ore_kernels.cuh"
+#include "ore_mesh_refit.h"
 #include "ore_scene_build.h"
 
 using namespace ore;
@@ -143,8 +144,8 @@ struct ore_context {
     // end of the last render on whichever stream it ran (scene setters wait for it before touching scene buffers)
     cudaEvent_t ev_done = nullptr;
     bool ev_done_set = false;
-    // end of the last stream-ordered scene update (ore_set_spheres_device) on whichever stream it ran: every render
-    // and every host setter enqueued later waits for it on the device
+    // end of the last stream-ordered scene update (ore_set_spheres_device, ore_set_mesh_triangles_device) on whichever
+    // stream it ran: every render and every host setter enqueued later waits for it on the device
     cudaEvent_t ev_scene = nullptr;
     bool ev_scene_set = false;
     // ordered flag writes (ore_flag_write_after)
@@ -483,6 +484,15 @@ extern "C" int ore_set_spheres_aos32(ore_context* ctx, const void* records, int3
     return upload_spheres(ctx, tmp.data(), 4, 0, n);
 }
 
+// the records of a stream-ordered update: device (or managed) memory of the context's GPU - not host, pinned or another
+// GPU's memory
+static bool on_context_gpu(ore_context* ctx, const void* p) {
+    cudaPointerAttributes at;
+    const cudaError_t e = cudaPointerGetAttributes(&at, p);
+    (void)cudaGetLastError();
+    return e == cudaSuccess && (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == ctx->device;
+}
+
 extern "C" int ore_set_spheres_device(ore_context* ctx, const float* xyz_radius_dev, int32_t n, void* stream) {
     if (!ctx) return ORE_ERR_INVALID;
     if (n < 0) return fail(ctx, ORE_ERR_INVALID, "ore_set_spheres_device: n < 0");
@@ -490,10 +500,7 @@ extern "C" int ore_set_spheres_device(ore_context* ctx, const float* xyz_radius_
     if (n > 0) {
         if (!xyz_radius_dev || ((uintptr_t)xyz_radius_dev & 15))
             return fail(ctx, ORE_ERR_INVALID, "ore_set_spheres_device: the records must be 16-byte aligned");
-        cudaPointerAttributes at;
-        const cudaError_t e = cudaPointerGetAttributes(&at, xyz_radius_dev);
-        (void)cudaGetLastError();
-        if (e != cudaSuccess || (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
+        if (!on_context_gpu(ctx, xyz_radius_dev))
             return fail(ctx, ORE_ERR_INVALID, "ore_set_spheres_device: the records must be device memory of the context's GPU");
     }
     const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
@@ -570,6 +577,8 @@ extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tri
         return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: null array");
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
     if (int rcw = wait_last_render(ctx)) return rcw;
+    // a pending ore_set_mesh_triangles_device still writes tris, boxes and box_sph
+    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaEventSynchronize(ctx->ev_scene));
     void* old[] = {ctx->tris, ctx->boxes, ctx->box_offsets, ctx->box_indices, ctx->box_sph, ctx->box_cone};
     for (void* p : old)
         if (p) ORE_CUDA(ctx, cudaFree(p));
@@ -591,25 +600,17 @@ extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tri
     const size_t ob = (size_t)(n_boxes + 1) * sizeof(int), ib = (size_t)(n_idx > 0 ? n_idx : 1) * sizeof(int);
     int rc;
     const size_t sb = (size_t)n_boxes * sizeof(float4);
-    // pinned staging layout: the two float4 sections first (16-byte aligned: bb and sb are multiples of 16 and the
-    // pinned base is page aligned), then the 4-byte-aligned sections
-    const size_t off_b = 0, off_s = bb, off_t = bb + sb, off_o = off_t + tb, off_i = off_o + ob;
+    // pinned staging layout: the float4 section first (16-byte aligned: bb is a multiple of 16 and the pinned base is
+    // page aligned), then the 4-byte-aligned sections
+    const size_t off_b = 0, off_t = bb, off_o = off_t + tb, off_i = off_o + ob;
     if ((rc = ensure_pinned(ctx, off_i + ib))) return rc;
     char* h = (char*)ctx->pinned;
     float4* hb = (float4*)(h + off_b);
-    float4* hs = (float4*)(h + off_s);
     memcpy(h + off_t, tris27, tb);
     for (int j = 0; j < n_boxes; j++) {
         const float* b = box_bounds6 + 6 * (size_t)j;
         hb[2 * j] = make_float4(b[0], b[1], b[2], 0.f);
         hb[2 * j + 1] = make_float4(b[3], b[4], b[5], 0.f);
-        // bounding sphere for the conservative cone filters: centre, half diagonal + 0.1 % + a little absolute slack
-        // (the float slab test can accept a ray that misses the true box by rounding)
-        const double cx = 0.5 * ((double)b[0] + b[3]), cy = 0.5 * ((double)b[1] + b[4]), cz = 0.5 * ((double)b[2] + b[5]);
-        const double dx = (double)b[3] - b[0], dy = (double)b[4] - b[1], dz = (double)b[5] - b[2];
-        const double rad = 0.5 * sqrt(dx * dx + dy * dy + dz * dz);
-        const double mag = fabs(cx) + fabs(cy) + fabs(cz) + rad;
-        hs[j] = make_float4((float)cx, (float)cy, (float)cz, (float)(rad * 1.001 + 1e-5 * mag + 1e-6));
     }
     memcpy(h + off_o, box_offsets, ob);
     memcpy(h + off_i, box_indices, (size_t)n_idx * sizeof(int));
@@ -619,15 +620,39 @@ extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tri
     ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_indices, ib));
     ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_sph, sb));
     ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_cone, sb * MAX_BATCH));
-    ORE_CUDA(ctx, cudaMemcpyAsync(ctx->box_sph, hs, sb, cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->tris, h + off_t, tb, cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->boxes, hb, bb, cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->box_offsets, h + off_o, ob, cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->box_indices, h + off_i, ib, cudaMemcpyHostToDevice, ctx->stream));
+    // the leaf balls by the kernel the device update runs too (ore_mesh_refit.cu): one code path for box_sph
+    ORE_CUDA(ctx, ore_mesh_balls(ctx->boxes, ctx->box_sph, n_boxes, ctx->stream));
     ORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->n_tris = n_tris;
     ctx->n_boxes = n_boxes;
     ctx->mesh_has_normals = has_normals ? 1 : 0;
+    return ORE_OK;
+}
+
+extern "C" int ore_set_mesh_triangles_device(ore_context* ctx, const float* tris27_dev, int32_t n_tris, void* stream) {
+    if (!ctx) return ORE_ERR_INVALID;
+    if (ctx->n_tris == 0) return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_triangles_device: no mesh set (ore_set_mesh first)");
+    if (n_tris != ctx->n_tris)
+        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_triangles_device: n_tris must equal the mesh's triangle count");
+    if (!tris27_dev || ((uintptr_t)tris27_dev & 3))
+        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_triangles_device: the triangles must be 4-byte aligned");
+    ORE_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!on_context_gpu(ctx, tris27_dev))
+        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_triangles_device: the triangles must be device memory of the context's GPU");
+    const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+    // after every render submitted so far and the previous update, on whatever streams they ran; the host never waits
+    if (ctx->ev_done_set) ORE_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_done, 0));
+    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_scene, 0));
+    ORE_CUDA(ctx, cudaMemcpyAsync(ctx->tris, tris27_dev, (size_t)n_tris * ore_host::TRI_FLOATS * sizeof(float),
+                                  cudaMemcpyDeviceToDevice, st));
+    ORE_CUDA(ctx, ore_mesh_refit(ctx->tris, ctx->box_offsets, ctx->box_indices, ctx->boxes, ctx->n_boxes, st));
+    ORE_CUDA(ctx, ore_mesh_balls(ctx->boxes, ctx->box_sph, ctx->n_boxes, st));
+    ORE_CUDA(ctx, cudaEventRecord(ctx->ev_scene, st));
+    ctx->ev_scene_set = true;
     return ORE_OK;
 }
 
@@ -1516,6 +1541,19 @@ extern "C" int ore_debug_sphere_tree(ore_context* ctx, int32_t which, void* host
     if ((size_t)n_items != count[which]) return fail(ctx, ORE_ERR_INVALID, "ore_debug_sphere_tree: n_items must be the array's length");
     if (n_items > 0)
         ORE_CUDA(ctx, cudaMemcpy(host_out, src[which], (size_t)n_items * (which == 3 ? sizeof(int) : sizeof(float4)), cudaMemcpyDeviceToHost));
+    return ORE_OK;
+}
+
+extern "C" int ore_debug_mesh(ore_context* ctx, int32_t which, void* host_out, int32_t n_items) {
+    if (!ctx || which < 0 || which > 2 || n_items < 0 || (n_items > 0 && !host_out)) return ORE_ERR_INVALID;
+    ORE_CUDA(ctx, cudaSetDevice(ctx->device));
+    ORE_CUDA(ctx, cudaDeviceSynchronize());
+    if (ctx->n_tris == 0) return fail(ctx, ORE_ERR_INVALID, "ore_debug_mesh: no mesh set");
+    const void* src[3] = {ctx->tris, ctx->boxes, ctx->box_sph};
+    const size_t count[3] = {(size_t)ctx->n_tris * ore_host::TRI_FLOATS, 2 * (size_t)ctx->n_boxes, (size_t)ctx->n_boxes};
+    if ((size_t)n_items != count[which]) return fail(ctx, ORE_ERR_INVALID, "ore_debug_mesh: n_items must be the array's length");
+    if (n_items > 0)
+        ORE_CUDA(ctx, cudaMemcpy(host_out, src[which], (size_t)n_items * (which == 0 ? sizeof(float) : sizeof(float4)), cudaMemcpyDeviceToHost));
     return ORE_OK;
 }
 
