@@ -164,7 +164,8 @@ int ore_set_planes(ore_context* ctx, const float* pos_normal, int32_t n);
  * copy it (kernel.cu:999-1017, 528-535): the loader and the builder stay on the host, this call replaces the copy.
  *   tris27      : n_tris x 27 floats = `triangle` {points[3], normal, vecNormal[3], vt[3]} (kernel.cu:206-212)
  *   has_normals : mesh::has_normals
- *   box_bounds6 : n_boxes x {bounds[0].xyz, bounds[1].xyz} of each leaf's `bvhbox` cube
+ *   box_bounds6 : n_boxes x {bounds[0].xyz, bounds[1].xyz} of each leaf's `bvhbox` cube.  A box need not contain
+ *                 its triangles: the render then still equals the reference's (DESIGN.md 6c)
  *   box_offsets : n_boxes + 1; leaf j holds box_indices[box_offsets[j] .. box_offsets[j+1])  (Bvhbox::indexes/length)
  * Hit ids continue after spheres, cubes and planes: triangle i -> n_spheres + n_cubes + n_planes + i.
  * Exact tests, linear scan over the leaves per ray like the reference (kernel.cu:1293-1328,1475-1497). */

@@ -193,6 +193,33 @@ int oracle_sphere_intersect(const float org[3], const float dir[3], const float 
     return hit;
 }
 
+int oracle_cube_intersect(const float org[3], const float dir[3], const float c1[3], const float c2[3], float* t) {
+    v3 O = {org[0], org[1], org[2]}, D = {dir[0], dir[1], dir[2]}, b0 = {c1[0], c1[1], c1[2]}, b1 = {c2[0], c2[1], c2[2]};
+    float tt = 0.f;
+    int hit = cube_intersect(O, D, b0, b1, &tt);
+    if (t) *t = tt;
+    return hit;
+}
+
+int oracle_plane_intersect(const float org[3], const float dir[3], const float pos[3], const float normal[3], float* t) {
+    v3 O = {org[0], org[1], org[2]}, D = {dir[0], dir[1], dir[2]}, p = {pos[0], pos[1], pos[2]};
+    v3 n = {normal[0], normal[1], normal[2]};
+    float tt = 0.f;
+    int hit = plane_intersect(O, D, p, n, &tt);
+    if (t) *t = tt;
+    return hit;
+}
+
+int oracle_tri_intersect(const float org[3], const float dir[3], const float tri[9], float* t, float* u, float* v) {
+    v3 O = {org[0], org[1], org[2]}, D = {dir[0], dir[1], dir[2]};
+    float tt = 0.f, uu = 0.f, vv = 0.f;
+    int hit = tri_intersect(O, D, tri, &tt, &uu, &vv);
+    if (t) *t = tt;
+    if (u) *u = uu;
+    if (v) *v = vv;
+    return hit;
+}
+
 const char* oracle_kind(void) { return "port"; }
 
 /* only the _ref library (the reference's own loader) can build a mesh from an OBJ file */

@@ -75,6 +75,18 @@ int oracle_render(const oracle_frame* f, uint32_t* pixels, int32_t* hit_id, floa
 int oracle_sphere_intersect(const float org[3], const float dir[3], const float centre[3],
                             float radius_member, float* t);
 
+/* Single ray-box test exactly as cube::intersect (kernel.cu:460-483), the reference's max/min macros and their NaN
+ * behaviour included; also the leaf-box test of the mesh loops.  c1, c2: the ctor's corners in either order.  Returns
+ * the bool; *t as written (tmin on a hit, tmax otherwise; negative t can be a hit). */
+int oracle_cube_intersect(const float org[3], const float dir[3], const float c1[3], const float c2[3], float* t);
+
+/* Single ray-plane test exactly as plane::intersect (kernel.cu:369-380): one-sided, t >= 0. */
+int oracle_plane_intersect(const float org[3], const float dir[3], const float pos[3], const float normal[3], float* t);
+
+/* Single ray-triangle test exactly as mesh::rayIntersect (kernel.cu:1024-1059).  tri: the 9 vertex floats (points[3]).
+ * Returns the bool; *t, *u, *v as written, 0 where the test returns before writing them. */
+int oracle_tri_intersect(const float org[3], const float dir[3], const float tri[9], float* t, float* u, float* v);
+
 /* rgbToInt (kernel.cu:546-556) */
 uint32_t oracle_rgb_to_int(int r, int g, int b);
 

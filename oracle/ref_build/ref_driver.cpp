@@ -18,6 +18,8 @@
 #include <limits>
 #include <map>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 #include <omp.h>
 
@@ -58,6 +60,83 @@ extern "C" int oracle_sphere_intersect(const float org[3], const float dir[3], c
     bool hit = s.intersect(r, tt);
     if (t) *t = tt;
     return hit ? 1 : 0;
+}
+
+// ---- single-primitive tests: the reference's own cube::intersect, plane::intersect and mesh::rayIntersect ----
+// The call forms are detected at compile time, so this file builds against any revision of kernel.cu; where no form
+// matches, the entry point returns -1 and the pin test (tests/test_primitive_cull_cpu.py) skips.
+template <class T, class = void>
+struct ore_has_intersect : std::false_type {};
+template <class T>
+struct ore_has_intersect<T, std::void_t<decltype(static_cast<bool>(
+                                std::declval<T&>().intersect(std::declval<ray&>(), std::declval<float&>())))>>
+    : std::true_type {};
+template <class T>
+static int ore_ref_intersect(T& obj, const float org[3], const float dir[3], float* t) {
+    if constexpr (ore_has_intersect<T>::value) {
+        ray r({org[0], org[1], org[2]}, {dir[0], dir[1], dir[2]});
+        float tt = 0.f;
+        const bool hit = obj.intersect(r, tt);
+        if (t) *t = tt;
+        return hit ? 1 : 0;
+    } else {
+        return -1;
+    }
+}
+// mesh::rayIntersect as (ray, triangle, t, u, v) or (origin, direction, triangle, t, u, v)
+template <class M, class = void>
+struct ore_tri_by_ray : std::false_type {};
+template <class M>
+struct ore_tri_by_ray<M, std::void_t<decltype(static_cast<bool>(std::declval<M&>().rayIntersect(
+                             std::declval<ray&>(), std::declval<triangle&>(), std::declval<float&>(),
+                             std::declval<float&>(), std::declval<float&>())))>> : std::true_type {};
+template <class M, class = void>
+struct ore_tri_by_vecs : std::false_type {};
+template <class M>
+struct ore_tri_by_vecs<M, std::void_t<decltype(static_cast<bool>(std::declval<M&>().rayIntersect(
+                              std::declval<vec3d&>(), std::declval<vec3d&>(), std::declval<triangle&>(),
+                              std::declval<float&>(), std::declval<float&>(), std::declval<float&>())))>>
+    : std::true_type {};
+template <class M>
+static int ore_ref_tri(M& m, const float org[3], const float dir[3], triangle& tr, float& t, float& u, float& v) {
+    if constexpr (ore_tri_by_ray<M>::value) {
+        ray r({org[0], org[1], org[2]}, {dir[0], dir[1], dir[2]});
+        return m.rayIntersect(r, tr, t, u, v) ? 1 : 0;
+    } else if constexpr (ore_tri_by_vecs<M>::value) {
+        vec3d o({org[0], org[1], org[2]}), d({dir[0], dir[1], dir[2]});
+        return m.rayIntersect(o, d, tr, t, u, v) ? 1 : 0;
+    } else {
+        return -1;
+    }
+}
+
+extern "C" int oracle_cube_intersect(const float org[3], const float dir[3], const float c1[3], const float c2[3],
+                                     float* t) {
+    cube c({c1[0], c1[1], c1[2]}, {c2[0], c2[1], c2[2]});
+    return ore_ref_intersect(c, org, dir, t);
+}
+
+extern "C" int oracle_plane_intersect(const float org[3], const float dir[3], const float pos[3], const float normal[3],
+                                      float* t) {
+    plane p({pos[0], pos[1], pos[2]}, {normal[0], normal[1], normal[2]});
+    return ore_ref_intersect(p, org, dir, t);
+}
+
+extern "C" int oracle_tri_intersect(const float org[3], const float dir[3], const float tri[9], float* t, float* u,
+                                    float* v) {
+    static_assert(sizeof(triangle) == 27 * sizeof(float), "triangle layout");
+    float raw[27] = {};
+    memcpy(raw, tri, 9 * sizeof(float));
+    triangle tr;
+    memcpy(&tr, raw, sizeof tr);
+    mesh* m = new mesh("/nonexistent/ore-none.obj");   // no file: the ctor returns early, as in oracle_render
+    float tt = 0.f, uu = 0.f, vv = 0.f;
+    const int hit = ore_ref_tri(*m, org, dir, tr, tt, uu, vv);
+    delete m;
+    if (t) *t = tt;
+    if (u) *u = uu;
+    if (v) *v = vv;
+    return hit;
 }
 
 // The reference's OWN OBJ loader and BVH builder (mesh::mesh -> createBvhMesh, kernel.cu:577-936), run on a file,

@@ -249,14 +249,49 @@ __device__ __noinline__ void nearest_cube_plane(const float4* __restrict__ cubes
     *best_t = nt;
     *best_id = id;
 }
+// The light-cone culls below skip a box whose bounding sphere the cone cannot touch.  That is sound only for hits that
+// lie in the box, and cube::intersect has one kind that does not (DESIGN.md 6b): a ray with D.k == +-0 that starts on a
+// face plane of the box on axis k gets (b.k - O.k) * (1 / D.k) = 0 * inf = NaN for that slab, and the reference's max/min
+// macros then drop that slab and every slab before it, so the test can report a hit far from the box.  zero_axes gives
+// the axes (bits 0..2) on which some ray of `live` has a component whose reciprocal overflows (+-0, tiny, or NaN);
+// the caller computes it once per light and passes it to both culls as `zaxes`.  on_face_plane says whether O lies on
+// a face plane of box (b0, b1) on one of them.  Such a box is never culled.
+__device__ __forceinline__ uint32_t zero_axes(const float* __restrict__ dirs, int dstride, uint32_t live) {
+    uint32_t z = 0;
+    while (live) {
+        const int r = __ffs(live) - 1;
+        live &= live - 1;
+        const v3 D = dir_at(dirs, dstride, r);
+        z |= (uint32_t)!(fabsf(D.x) >= 0x1p-126f) | (uint32_t)!(fabsf(D.y) >= 0x1p-126f) << 1 |
+             (uint32_t)!(fabsf(D.z) >= 0x1p-126f) << 2;
+    }
+    return z;
+}
+__device__ __forceinline__ bool on_face_plane(uint32_t zaxes, float Ox, float Oy, float Oz, float4 b0, float4 b1) {
+    return ((zaxes & 1u) && (Ox == b0.x || Ox == b1.x)) || ((zaxes & 2u) && (Oy == b0.y || Oy == b1.y)) ||
+           ((zaxes & 4u) && (Oz == b0.z || Oz == b1.z));
+}
+// true when the light's cone (A, ca, sa) cannot touch the ball q (.xyz centre, .w radius incl. margin) seen from O.
+// A NaN anywhere (a non-finite ball, or |O - q|^2 overflowing to inf) answers false: the box stays.
+__device__ __forceinline__ bool cone_misses_ball(float4 q, float Ox, float Oy, float Oz, float Ax, float Ay, float Az, float ca,
+                                                 float sa) {
+    const float lx = Ox - q.x, ly = Oy - q.y, lz = Oz - q.z;
+    const float LL = fmaf(lz, lz, fmaf(ly, ly, lx * lx));
+    const float Cm = fmaf(LL, 1.0f - ORE_KAPPA_SHADOW, -(q.w * q.w));
+    if (!(Cm > 1e-20f)) return false;   // O in or near the ball, or NaN
+    const float sv = Cm * rsqrt_approx(Cm);
+    const float T = fmaf(ca, sv, -(sa * q.w));
+    return fmaf(Ax, lx, fmaf(Ay, ly, fmaf(Az, lz, T))) >= 0.f;
+}
 // castLightRay's plane loop then cube loop (kernel.cu:1512-1536) for the live rays `live` (bits 0..9) of ONE light (ray r =
 // dir_at(dirs, dstride, r)):
 // any hit blocks.  A cube whose bounding sphere (cubes[3*i+2].xyz = orgin, .w = radius incl. margin) the light's cone
-// cannot touch is skipped.  Returns the rays found blocked.
+// cannot touch is skipped, unless O lies on one of its face planes (above).  Returns the rays found blocked.
 __device__ __noinline__ uint32_t cubes_planes_block_light(const float4* __restrict__ cubes, int nc,
                                                           const float4* __restrict__ planes, int np, float Ox, float Oy,
                                                           float Oz, float Ax, float Ay, float Az, float ca, float sa,
-                                                          bool use_cone, const float* __restrict__ dirs, int dstride, uint32_t live) {
+                                                          bool use_cone, uint32_t zaxes, const float* __restrict__ dirs, int dstride,
+                                                          uint32_t live) {
     const v3 O = mk(Ox, Oy, Oz);
     uint32_t hit = 0;
     float t;
@@ -274,17 +309,9 @@ __device__ __noinline__ uint32_t cubes_planes_block_light(const float4* __restri
         }
     }
     for (int i = 0; i < nc && live; i++) {
-        const float4 q = __ldg(&cubes[3 * i + 2]);
-        if (use_cone) {
-            const float lx = Ox - q.x, ly = Oy - q.y, lz = Oz - q.z;
-            const float LL = fmaf(lz, lz, fmaf(ly, ly, lx * lx));
-            const float Cm = fmaf(LL, 1.0f - ORE_KAPPA_SHADOW, -(q.w * q.w));
-            if (Cm > 1e-20f) {
-                const float sv = Cm * rsqrt_approx(Cm);
-                const float T = fmaf(ca, sv, -(sa * q.w));
-                if (!(fmaf(Ax, lx, fmaf(Ay, ly, fmaf(Az, lz, T))) < 0.f)) continue;  // cone misses the cube
-            }
-        }
+        if (use_cone && cone_misses_ball(__ldg(&cubes[3 * i + 2]), Ox, Oy, Oz, Ax, Ay, Az, ca, sa) &&
+            (!zaxes || !on_face_plane(zaxes, Ox, Oy, Oz, __ldg(&cubes[3 * i]), __ldg(&cubes[3 * i + 1]))))
+            continue;
         const float4 b0 = __ldg(&cubes[3 * i]), b1 = __ldg(&cubes[3 * i + 1]);
         uint32_t todo = live;
         while (todo) {
@@ -334,25 +361,18 @@ __device__ __noinline__ void nearest_in_leaf(const MeshArgs m, int j, int id_bas
     *best_id = id;
 }
 // castLightRay's triangle part (kernel.cu:1475-1497) for the live rays `live` (bits 0..9) of ONE light: a leaf is
-// skipped when the light's cone (A, ca, sa; use_cone) cannot touch its bounding sphere; otherwise every live ray
-// runs the exact slab test and the exact triangle tests.  Returns the rays found blocked.
+// skipped when the light's cone (A, ca, sa; use_cone) cannot touch its bounding sphere and O lies on none of its face
+// planes (above: the caller's boxes need not contain their triangles); otherwise every live ray runs the exact slab
+// test and the exact triangle tests.  Returns the rays found blocked.
 __device__ __noinline__ uint32_t mesh_blocks_light(const MeshArgs m, const float4* __restrict__ box_sph, float Ox, float Oy,
                                                    float Oz, float Ax, float Ay, float Az, float ca, float sa, bool use_cone,
-                                                   const float* __restrict__ dirs, int dstride, uint32_t live) {
+                                                   uint32_t zaxes, const float* __restrict__ dirs, int dstride, uint32_t live) {
     const v3 O = mk(Ox, Oy, Oz);
     uint32_t hit = 0;
     for (int j = 0; j < m.n_boxes && live; j++) {
-        if (use_cone) {
-            const float4 q = __ldg(&box_sph[j]);
-            const float lx = Ox - q.x, ly = Oy - q.y, lz = Oz - q.z;
-            const float LL = fmaf(lz, lz, fmaf(ly, ly, lx * lx));
-            const float Cm = fmaf(LL, 1.0f - ORE_KAPPA_SHADOW, -(q.w * q.w));
-            if (Cm > 1e-20f) {
-                const float sv = Cm * rsqrt_approx(Cm);
-                const float T = fmaf(ca, sv, -(sa * q.w));
-                if (!(fmaf(Ax, lx, fmaf(Ay, ly, fmaf(Az, lz, T))) < 0.f)) continue;  // cone misses the leaf
-            }
-        }
+        if (use_cone && cone_misses_ball(__ldg(&box_sph[j]), Ox, Oy, Oz, Ax, Ay, Az, ca, sa) &&
+            (!zaxes || !on_face_plane(zaxes, Ox, Oy, Oz, __ldg(&m.boxes[2 * j]), __ldg(&m.boxes[2 * j + 1]))))
+            continue;
         const float4 b0 = __ldg(&m.boxes[2 * j]), b1 = __ldg(&m.boxes[2 * j + 1]);
         const int k0 = __ldg(&m.offsets[j]), k1 = __ldg(&m.offsets[j + 1]);
         uint32_t todo = live;

@@ -107,10 +107,14 @@ __global__ void prep_frame_kernel(const FrameParams prm) {
             prm.super_cone[(size_t)f * prm.n_supers_pad + i] = cone;
         }
         if (i < prm.n_boxes) {
-            // tile-cone record of leaf box i of the mesh from its bounding sphere (same formula)
+            // tile-cone record of leaf box i of the mesh from its bounding sphere (same formula).  An eye on a face plane
+            // of the box makes it always a candidate: a primary ray with a +-0 component on that axis can pass the slab
+            // test through a NaN slab and then hit a triangle the box does not contain (ore_kernels.cuh, zero_axes)
             const float4 q = prm.box_sph[i];
             float4 rec;
             ball_records(prm, cam, (double)cam.Ox - q.x, (double)cam.Oy - q.y, (double)cam.Oz - q.z, (double)q.w * q.w, nullptr, &rec);
+            if (on_face_plane(7u, cam.Ox, cam.Oy, cam.Oz, prm.boxes[2 * i], prm.boxes[2 * i + 1]))
+                rec = make_float4(0.f, 0.f, 0.f, -ORE_BIG);
             prm.box_cone[(size_t)f * prm.n_boxes + i] = rec;
         }
     }

@@ -403,11 +403,13 @@ __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_ke
             // ---- triangles (kernel.cu:1475-1497; tested first in the reference - the result is an OR, order-free):
             //      leaves outside the light's cone are skipped ----
             const bool use_cone = !EXH && !force && ca > 0.f;
+            // rays blocked later only shrink the live set: this mask covers every box test below
+            const uint32_t zaxes = (use_cone && (prm.n_boxes | prm.n_cubes) && valid) ? zero_axes(dslot, 32, ~blocked & 0x3ffu) : 0u;
             if (prm.n_boxes && valid) {
                 const uint32_t live = ~blocked & 0x3ffu;
                 if (live) {
                     const MeshArgs ma = {prm.tris, prm.boxes, prm.box_offsets, prm.box_indices, prm.n_boxes};
-                    blocked |= mesh_blocks_light(ma, prm.box_sph, start.x, start.y, start.z, Ax, Ay, Az, ca, sa, use_cone, dslot, 32, live);
+                    blocked |= mesh_blocks_light(ma, prm.box_sph, start.x, start.y, start.z, Ax, Ay, Az, ca, sa, use_cone, zaxes, dslot, 32, live);
                 }
             }
             // ---- planes, then cubes (kernel.cu:1512-1536) for the rays nothing blocked yet ----
@@ -415,7 +417,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_ke
                 const uint32_t live = ~blocked & 0x3ffu;
                 if (live)
                     blocked |= cubes_planes_block_light(prm.cubes, prm.n_cubes, prm.planes, prm.n_planes, start.x, start.y, start.z,
-                                                        Ax, Ay, Az, ca, sa, use_cone, dslot, 32, live);
+                                                        Ax, Ay, Az, ca, sa, use_cone, zaxes, dslot, 32, live);
             }
             // ---- light accumulation (kernel.cu:1537-1543, 1673-1675) ----
             if (valid) {

@@ -42,6 +42,17 @@ def _ptr(a: np.ndarray):
     return a.ctypes.data_as(_fp)
 
 
+def _vec(v, n=3):
+    a = np.ascontiguousarray(v, dtype=np.float32).reshape(-1)
+    assert a.size == n
+    return (C.c_float * n).from_buffer_copy(a.tobytes())
+
+
+def _supported(hit):
+    if hit < 0:   # _ref: the reference revision has none of the call forms ref_driver.cpp knows for this test
+        raise NotImplementedError("this reference build does not provide the single-primitive test")
+
+
 def build_port():
     if not os.path.isfile(PORT_SO) or os.path.getmtime(PORT_SO) < os.path.getmtime(os.path.join(ORACLE_DIR, "oracle.c")):
         subprocess.check_call(["make", "-C", ORACLE_DIR, "port"], stdout=subprocess.DEVNULL)
@@ -60,6 +71,15 @@ class Oracle:
         self.lib.oracle_render.argtypes = [C.POINTER(OracleFrame), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         self.lib.oracle_sphere_intersect.restype = C.c_int
         self.lib.oracle_sphere_intersect.argtypes = [_fp, _fp, _fp, C.c_float, _fp]
+        # single-primitive tests: liboracle always has them; a _ref library built before they existed does not
+        self.has_primitive_tests = all(hasattr(self.lib, n) for n in
+                                       ("oracle_cube_intersect", "oracle_plane_intersect", "oracle_tri_intersect"))
+        if self.has_primitive_tests:
+            for name in ("oracle_cube_intersect", "oracle_plane_intersect"):
+                getattr(self.lib, name).restype = C.c_int
+                getattr(self.lib, name).argtypes = [_fp, _fp, _fp, _fp, _fp]
+            self.lib.oracle_tri_intersect.restype = C.c_int
+            self.lib.oracle_tri_intersect.argtypes = [_fp, _fp, _fp, _fp, _fp, _fp]
         self.lib.oracle_rgb_to_int.restype = C.c_uint32
         self.lib.oracle_rgb_to_int.argtypes = [C.c_int, C.c_int, C.c_int]
         self.lib.oracle_kind.restype = C.c_char_p
@@ -133,6 +153,26 @@ class Oracle:
         t = C.c_float(0)
         hit = self.lib.oracle_sphere_intersect(o, d, c, C.c_float(radius_member), C.byref(t))
         return bool(hit), np.float32(t.value)
+
+    def cube_intersect(self, org, direction, c1, c2):
+        """cube::intersect: (hit, t) - t is tmin on a hit, tmax otherwise"""
+        t = C.c_float(0)
+        hit = self.lib.oracle_cube_intersect(_vec(org), _vec(direction), _vec(c1), _vec(c2), C.byref(t))
+        _supported(hit)
+        return bool(hit), np.float32(t.value)
+
+    def plane_intersect(self, org, direction, pos, normal):
+        t = C.c_float(0)
+        hit = self.lib.oracle_plane_intersect(_vec(org), _vec(direction), _vec(pos), _vec(normal), C.byref(t))
+        _supported(hit)
+        return bool(hit), np.float32(t.value)
+
+    def tri_intersect(self, org, direction, tri9):
+        """mesh::rayIntersect on the 9 vertex floats: (hit, t, u, v)"""
+        t, u, v = C.c_float(0), C.c_float(0), C.c_float(0)
+        hit = self.lib.oracle_tri_intersect(_vec(org), _vec(direction), _vec(tri9, 9), C.byref(t), C.byref(u), C.byref(v))
+        _supported(hit)
+        return bool(hit), np.float32(t.value), np.float32(u.value), np.float32(v.value)
 
     def rgb_to_int(self, r, g, b) -> int:
         return int(self.lib.oracle_rgb_to_int(int(r), int(g), int(b)))
