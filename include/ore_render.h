@@ -185,6 +185,22 @@ int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tris, int32_t 
  *   submitted afterwards, on any stream, see the new triangles.  The host never blocks: nothing grows.
  *   Caller's buffer: it must stay allocated and unchanged until the update has run on `stream`. */
 int ore_set_mesh_triangles_device(ore_context* ctx, const float* tris27_dev, int32_t n_tris, void* stream);
+/* Stream-ordered replacement of the whole mesh from DEVICE memory, with the flat BVH built on the GPU (GPU-generated or
+ * strongly deformed geometry, a changing triangle count).  `tris27_dev`: n_tris >= 1 records of ore_set_mesh's tris27
+ * in device memory of the context's GPU, 4-byte aligned; has_normals is taken as != 0.  The leaves are exactly what the
+ * reference's createBvhMesh (kernel.cu:782-936) - and ore_build_flat_bvh in host/ore_mesh.cpp - gives for these
+ * triangles: the same leaf order, the same index order within each leaf and the same bits of every box, so every result
+ * guarantee of ore_set_mesh carries over.  (Removing the mesh stays ore_set_mesh(ctx, NULL, 0, ...).)  n_tris < 1, a
+ * NULL, misaligned or host pointer, or another GPU's memory return ORE_ERR_INVALID and change nothing.
+ *   Leaf count: decided on the device.  The context holds min(1024, n_tris) leaves; those past the live count list no
+ *   triangles and are never visited.  ore_set_mesh_triangles_device afterwards refits this topology.
+ *   Ordering: as ore_set_spheres_device (the same events): enqueued on `stream` (NULL = the context's render stream)
+ *   after every render already submitted and the previous update; renders and setters submitted afterwards, on any
+ *   stream, see the new mesh.
+ *   Host blocking: none while n_tris fits the mesh capacity - the largest mesh either setter uploaded since the mesh was
+ *   last removed.  Growing it first waits on the host for the last render and the last update.
+ *   Caller's buffer: it must stay allocated and unchanged until the update has run on `stream`. */
+int ore_set_mesh_device(ore_context* ctx, const float* tris27_dev, int32_t n_tris, int32_t has_normals, void* stream);
 /* Replaces cudaMalloc+cudaMemcpy of `lights` in update() (kernel.cu:1776-1778):
  * n x {pos.xyz, size, r, g, b} (kernel.cu:1246-1261). */
 int ore_set_lights(ore_context* ctx, const float* lights7, int32_t n);
@@ -292,8 +308,10 @@ int ore_debug_libm(ore_context* ctx, int op, int n, const float* a_host, const f
  * to a multiple of 32, n_supers_pad = ceil(n / 256) rounded up to a multiple of 4.  n_items must be that length. */
 int ore_debug_sphere_tree(ore_context* ctx, int32_t which, void* host_out, int32_t n_items);
 /* Tests only: synchronises the device and copies one array of the mesh to the host.  which: 0 triangles (n_tris * 27
- * floats), 1 leaf boxes lo, hi (2 * n_boxes float4, .w = 0), 2 leaf bounding spheres (n_boxes float4).  n_items must be
- * that length. */
+ * floats), 1 leaf boxes lo, hi (2 * n_boxes float4, .w = 0), 2 leaf bounding spheres (n_boxes float4), 3 leaf offsets
+ * (n_boxes + 1 int32), 4 leaf indices (n_idx int32: box_offsets[n_boxes] of ore_set_mesh, n_tris after
+ * ore_set_mesh_device), 5 the live leaf count (1 int32).  n_boxes is ore_set_mesh's, or min(1024, n_tris) after
+ * ore_set_mesh_device.  n_items must be that length. */
 int ore_debug_mesh(ore_context* ctx, int32_t which, void* host_out, int32_t n_items);
 
 #ifdef __cplusplus

@@ -30,6 +30,7 @@ EXPORTS = [
     "ore_render_async_signal", "ore_host_register", "ore_host_unregister", "ore_flag_write", "ore_flag_wait_geq",
     "ore_flag_write_after", "ore_get_stream", "ore_render_batch_device", "ore_render_batch_async",
     "ore_set_spheres_device", "ore_debug_sphere_tree", "ore_set_mesh_triangles_device", "ore_debug_mesh",
+    "ore_set_mesh_device",
 ]
 
 # ore_debug_sphere_tree: which array of the sphere hierarchy, and its element type
@@ -37,7 +38,10 @@ SPHERE_TREE_ARRAYS = {"sph_exact": 0, "sph_xsort": 1, "sph_sort": 2, "sort_index
 
 
 # ore_debug_mesh: which array of the mesh
-MESH_ARRAYS = {"tris": 0, "boxes": 1, "box_sph": 2}
+MESH_ARRAYS = {"tris": 0, "boxes": 1, "box_sph": 2, "box_offsets": 3, "box_indices": 4, "n_live": 5}
+
+# leaves of a mesh built on the device (ore_set_mesh_device) hold this many at most
+MESH_MAX_LEAVES = 1024
 
 
 def sphere_tree_lengths(n: int) -> dict:
@@ -97,6 +101,7 @@ def load_library(path: str | None = None) -> C.CDLL:
     ip = C.POINTER(C.c_int32)
     lib.ore_set_mesh.argtypes = [vp, fp, i32, i32, fp, ip, ip, i32]
     lib.ore_set_mesh_triangles_device.argtypes = [vp, vp, i32, vp]
+    lib.ore_set_mesh_device.argtypes = [vp, vp, i32, i32, vp]
     lib.ore_debug_mesh.argtypes = [vp, i32, vp, i32]
     lib.ore_set_texture.argtypes = [vp, fp, fp, fp, i32, i32]
     lib.ore_set_sky.argtypes = [vp, fp, fp, fp, i32, i32, C.c_float]
@@ -225,11 +230,35 @@ class Renderer:
         if mesh is None or mesh.n_tris == 0:
             self._check(self.lib.ore_set_mesh(self.ctx, None, 0, 0, None, None, None, 0), "ore_set_mesh")
             self._mesh_counts = (0, 0)
+            self._mesh_n_idx = 0
             return
         self._check(self.lib.ore_set_mesh(self.ctx, _fptr(mesh.tris.reshape(-1)), mesh.n_tris, int(mesh.has_normals),
                                           _fptr(mesh.box_bounds.reshape(-1)), mesh.box_offsets.ctypes.data_as(ip),
                                           mesh.box_indices.ctypes.data_as(ip), mesh.n_boxes), "ore_set_mesh")
         self._mesh_counts = (mesh.n_tris, mesh.n_boxes) if mesh.n_boxes else (0, 0)   # (no leaves: no mesh)
+        self._mesh_n_idx = int(mesh.box_offsets[mesh.n_boxes]) if mesh.n_boxes else 0
+
+    def set_mesh_device(self, t, has_normals: bool, stream: int = 0):
+        """Stream-ordered replacement of the whole mesh from a torch CUDA float32 tensor of shape (n_tris, 27), n_tris >= 1
+        (the records of set_mesh) on this context's GPU, with the reference's flat BVH built on the GPU: the leaves
+        equal the host builder's bit for bit.  `stream`: a raw cudaStream_t (0 = the context's render stream).  Keep `t`
+        alive and unchanged until the update has run on that stream."""
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"set_mesh_device: expected a torch.Tensor, got {type(t).__name__}")
+        if t.dtype != torch.float32:
+            raise TypeError(f"set_mesh_device: expected dtype torch.float32, got {t.dtype}")
+        if t.dim() != 2 or t.shape[1] != 27 or t.shape[0] < 1:
+            raise ValueError(f"set_mesh_device: expected shape (n, 27) with n >= 1, got {tuple(t.shape)}")
+        if t.device.type != "cuda" or t.device.index != self.device:
+            raise ValueError(f"set_mesh_device: the tensor must live on cuda:{self.device}, not {t.device}")
+        if not t.is_contiguous():
+            raise ValueError("set_mesh_device: the tensor must be contiguous")
+        n = int(t.shape[0])
+        self._check(self.lib.ore_set_mesh_device(self.ctx, C.c_void_p(t.data_ptr()), n, int(bool(has_normals)),
+                                                 C.c_void_p(stream) if stream else None), "ore_set_mesh_device")
+        self._mesh_counts = (n, min(MESH_MAX_LEAVES, n))   # (leaf capacity: the live count is on the device)
+        self._mesh_n_idx = n
 
     def set_mesh_triangles_device(self, t, stream: int = 0):
         """Stream-ordered update of the mesh's triangles from a torch CUDA float32 tensor of shape (n_tris, 27) (the
@@ -254,10 +283,14 @@ class Renderer:
 
     def debug_mesh(self, which: str) -> np.ndarray:
         """one array of the current mesh, read back after a device synchronise (tests): tris float32 (n_tris, 27), boxes
-        float32 (2 * n_boxes, 4) (lo, hi per leaf), box_sph float32 (n_boxes, 4)"""
+        float32 (2 * n_boxes, 4) (lo, hi per leaf), box_sph float32 (n_boxes, 4), box_offsets int32 (n_boxes + 1,),
+        box_indices int32 (n_idx,), n_live int32 (1,) (the live leaf count); n_boxes is the leaf capacity after
+        set_mesh_device"""
         n_tris, n_boxes = getattr(self, "_mesh_counts", (0, 0))
+        n_idx = getattr(self, "_mesh_n_idx", 0)
         out = {"tris": lambda: np.zeros((n_tris, 27), np.float32), "boxes": lambda: np.zeros((2 * n_boxes, 4), np.float32),
-               "box_sph": lambda: np.zeros((n_boxes, 4), np.float32)}[which]()
+               "box_sph": lambda: np.zeros((n_boxes, 4), np.float32), "box_offsets": lambda: np.zeros(n_boxes + 1, np.int32),
+               "box_indices": lambda: np.zeros(n_idx, np.int32), "n_live": lambda: np.zeros(1, np.int32)}[which]()
         self._check(self.lib.ore_debug_mesh(self.ctx, MESH_ARRAYS[which], out.ctypes.data if out.size else None,
                                             out.size if which == "tris" else out.shape[0]), "ore_debug_mesh")
         return out

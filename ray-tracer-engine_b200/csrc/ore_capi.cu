@@ -19,6 +19,7 @@
 #include "../../include/ore_render.h"
 #include "ore_clusters.h"
 #include "ore_kernels.cuh"
+#include "ore_mesh_build.h"
 #include "ore_mesh_refit.h"
 #include "ore_scene_build.h"
 
@@ -97,7 +98,20 @@ struct ore_context {
     float4* box_cone = nullptr;  // per-frame tile-cone record per leaf box
     int* box_offsets = nullptr;
     int* box_indices = nullptr;
-    int n_tris = 0, n_boxes = 0, mesh_has_normals = 0;
+    // n_boxes: the leaf capacity (stride of box_cone, grid sizes); the live leaf count is *mesh_live on the device (the
+    // render kernels' leaf loops end there; leaves past it list no triangles)
+    int n_tris = 0, n_boxes = 0, mesh_has_normals = 0, mesh_n_idx = 0;
+    int* mesh_live = nullptr;
+    // capacities of the mesh buffers (triangles, leaves, listed indices) and the device build's work space: the largest
+    // mesh uploaded by either setter since the mesh was last removed
+    size_t mesh_tri_cap = 0, mesh_box_cap = 0, mesh_idx_cap = 0;
+    void* mesh_work = nullptr;
+    size_t mesh_work_bytes = 0;
+    // the device build's launch sequence (about 65 launches, all sized from the capacity; the triangle count is read on
+    // the device) captured once per buffer set and replayed on the caller's stream: enqueuing it launch by launch costs
+    // the host several hundred microseconds
+    cudaGraphExec_t mesh_graph = nullptr;
+    cudaStream_t mesh_capture = nullptr;
 
     // per-frame buffers
     float* dx_tab = nullptr;
@@ -144,7 +158,8 @@ struct ore_context {
     // end of the last render on whichever stream it ran (scene setters wait for it before touching scene buffers)
     cudaEvent_t ev_done = nullptr;
     bool ev_done_set = false;
-    // end of the last stream-ordered scene update (ore_set_spheres_device, ore_set_mesh_triangles_device) on whichever
+    // end of the last stream-ordered scene update (ore_set_spheres_device, ore_set_mesh_device,
+    // ore_set_mesh_triangles_device) on whichever
     // stream it ran: every render and every host setter enqueued later waits for it on the device
     cudaEvent_t ev_scene = nullptr;
     bool ev_scene_set = false;
@@ -301,6 +316,8 @@ extern "C" int ore_destroy(ore_context* ctx) {
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->ev_done) cudaEventDestroy(ctx->ev_done);
     if (ctx->ev_scene) cudaEventDestroy(ctx->ev_scene);
+    if (ctx->mesh_graph) cudaGraphExecDestroy(ctx->mesh_graph);
+    if (ctx->mesh_capture) cudaStreamDestroy(ctx->mesh_capture);
     if (ctx->signal_stream) {
         cudaStreamSynchronize(ctx->signal_stream);
         for (auto& e : ctx->ev_signal)
@@ -318,7 +335,7 @@ extern "C" int ore_destroy(ore_context* ctx) {
                    ctx->prim_sorted, ctx->cone_sorted, ctx->leaf_cone, ctx->super_cone, ctx->tex[0], ctx->tex[1], ctx->tex[2],
                    ctx->sky[0], ctx->sky[1], ctx->sky[2], ctx->dx_tab, ctx->dy_tab, ctx->hit_list, ctx->hit_ids, ctx->hit_ts,
                    ctx->hit_id_map, ctx->hit_t_map, ctx->pixels, ctx->counters, ctx->cubes, ctx->planes, ctx->tris, ctx->boxes,
-                   ctx->box_offsets, ctx->box_indices, ctx->box_sph, ctx->box_cone, ctx->keys_in, ctx->keys_out, ctx->vals_in,
+                   ctx->box_offsets, ctx->box_indices, ctx->box_sph, ctx->box_cone, ctx->mesh_live, ctx->mesh_work, ctx->keys_in, ctx->keys_out, ctx->vals_in,
                    ctx->vals_out, ctx->bbox, ctx->sort_tmp};
     for (void* p : dev)
         if (p) cudaFree(p);
@@ -569,17 +586,13 @@ extern "C" int ore_set_planes(ore_context* ctx, const float* pos_normal, int32_t
     return ORE_OK;
 }
 
-extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tris, int32_t has_normals,
-                            const float* box_bounds6, const int32_t* box_offsets, const int32_t* box_indices,
-                            int32_t n_boxes) {
-    if (!ctx || n_tris < 0 || n_boxes < 0) return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: bad arguments");
-    if (n_tris > 0 && n_boxes > 0 && (!tris27 || !box_bounds6 || !box_offsets || !box_indices))
-        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: null array");
-    ORE_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (int rcw = wait_last_render(ctx)) return rcw;
-    // a pending ore_set_mesh_triangles_device still writes tris, boxes and box_sph
-    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaEventSynchronize(ctx->ev_scene));
-    void* old[] = {ctx->tris, ctx->boxes, ctx->box_offsets, ctx->box_indices, ctx->box_sph, ctx->box_cone};
+// Frees the mesh buffers and, unless tri_cap is 0, allocates them for tri_cap triangles, box_cap leaves and idx_cap
+// listed indices, with the device build's work space for tri_cap triangles.  The caller has waited for every render and
+// update that may use them.
+static int mesh_alloc(ore_context* ctx, size_t tri_cap, size_t box_cap, size_t idx_cap) {
+    if (ctx->mesh_graph) ORE_CUDA(ctx, cudaGraphExecDestroy(ctx->mesh_graph));   // (it holds the old buffers' addresses)
+    ctx->mesh_graph = nullptr;
+    void* old[] = {ctx->tris, ctx->boxes, ctx->box_offsets, ctx->box_indices, ctx->box_sph, ctx->box_cone, ctx->mesh_work};
     for (void* p : old)
         if (p) ORE_CUDA(ctx, cudaFree(p));
     ctx->tris = nullptr;
@@ -588,7 +601,43 @@ extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tri
     ctx->box_indices = nullptr;
     ctx->box_sph = nullptr;
     ctx->box_cone = nullptr;
-    ctx->n_tris = ctx->n_boxes = ctx->mesh_has_normals = 0;
+    ctx->mesh_work = nullptr;
+    ctx->mesh_tri_cap = ctx->mesh_box_cap = ctx->mesh_idx_cap = ctx->mesh_work_bytes = 0;
+    ctx->n_tris = ctx->n_boxes = ctx->mesh_has_normals = ctx->mesh_n_idx = 0;
+    if (tri_cap == 0) return ORE_OK;
+    if (tri_cap > (size_t)INT32_MAX / ore_host::TRI_FLOATS) return fail(ctx, ORE_ERR_INVALID, "mesh: too many triangles");
+    size_t work = 0;
+    ORE_CUDA(ctx, ore_mesh_build_bytes((int)tri_cap, &work));
+    if (!ctx->mesh_live) ORE_CUDA(ctx, cudaMalloc((void**)&ctx->mesh_live, sizeof(int)));
+    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->tris, tri_cap * ore_host::TRI_FLOATS * sizeof(float)));
+    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->boxes, box_cap * 2 * sizeof(float4)));
+    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_offsets, (box_cap + 1) * sizeof(int)));
+    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_indices, std::max(idx_cap, (size_t)1) * sizeof(int)));
+    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_sph, box_cap * sizeof(float4)));
+    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_cone, box_cap * sizeof(float4) * MAX_BATCH));
+    ORE_CUDA(ctx, cudaMalloc(&ctx->mesh_work, work));
+    ctx->mesh_tri_cap = tri_cap;
+    ctx->mesh_box_cap = box_cap;
+    ctx->mesh_idx_cap = idx_cap;
+    ctx->mesh_work_bytes = work;
+    return ORE_OK;
+}
+
+extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tris, int32_t has_normals,
+                            const float* box_bounds6, const int32_t* box_offsets, const int32_t* box_indices,
+                            int32_t n_boxes) {
+    if (!ctx || n_tris < 0 || n_boxes < 0) return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: bad arguments");
+    if (n_tris > 0 && n_boxes > 0 && (!tris27 || !box_bounds6 || !box_offsets || !box_indices))
+        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: null array");
+    ORE_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (int rcw = wait_last_render(ctx)) return rcw;
+    // a pending ore_set_mesh_device or ore_set_mesh_triangles_device still writes the mesh buffers and the build's
+    // work space
+    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaEventSynchronize(ctx->ev_scene));
+    // the buffers are re-allocated at least at the capacity the device setters reached, so that they keep not blocking
+    const size_t tri_cap0 = ctx->mesh_tri_cap, box_cap0 = ctx->mesh_box_cap, idx_cap0 = ctx->mesh_idx_cap;
+    int rc;
+    if ((rc = mesh_alloc(ctx, 0, 0, 0))) return rc;
     if (n_tris == 0 || n_boxes == 0) return ORE_OK;
     const int n_idx = box_offsets[n_boxes];
     if (box_offsets[0] != 0 || n_idx < 0) return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: bad offsets");
@@ -596,14 +645,16 @@ extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tri
         if (box_offsets[j + 1] < box_offsets[j]) return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: offsets must ascend");
     for (int k = 0; k < n_idx; k++)
         if (box_indices[k] < 0 || box_indices[k] >= n_tris) return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh: triangle index out of range");
+    const size_t tri_cap = std::max(tri_cap0, (size_t)n_tris);
+    const size_t box_cap = std::max(std::max(box_cap0, (size_t)n_boxes), (size_t)ore_mesh_leaf_capacity((int)std::min(tri_cap, (size_t)INT32_MAX)));
+    const size_t idx_cap = std::max(std::max(idx_cap0, (size_t)n_idx), tri_cap);
+    if ((rc = mesh_alloc(ctx, tri_cap, box_cap, idx_cap))) return rc;
     const size_t tb = (size_t)n_tris * 27 * sizeof(float), bb = (size_t)n_boxes * 2 * sizeof(float4);
     const size_t ob = (size_t)(n_boxes + 1) * sizeof(int), ib = (size_t)(n_idx > 0 ? n_idx : 1) * sizeof(int);
-    int rc;
-    const size_t sb = (size_t)n_boxes * sizeof(float4);
     // pinned staging layout: the float4 section first (16-byte aligned: bb is a multiple of 16 and the pinned base is
-    // page aligned), then the 4-byte-aligned sections
-    const size_t off_b = 0, off_t = bb, off_o = off_t + tb, off_i = off_o + ob;
-    if ((rc = ensure_pinned(ctx, off_i + ib))) return rc;
+    // page aligned), then the 4-byte-aligned sections, the live leaf count last
+    const size_t off_b = 0, off_t = bb, off_o = off_t + tb, off_i = off_o + ob, off_l = off_i + ib;
+    if ((rc = ensure_pinned(ctx, off_l + sizeof(int)))) return rc;
     char* h = (char*)ctx->pinned;
     float4* hb = (float4*)(h + off_b);
     memcpy(h + off_t, tris27, tb);
@@ -614,22 +665,80 @@ extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tri
     }
     memcpy(h + off_o, box_offsets, ob);
     memcpy(h + off_i, box_indices, (size_t)n_idx * sizeof(int));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->tris, tb));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->boxes, bb));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_offsets, ob));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_indices, ib));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_sph, sb));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_cone, sb * MAX_BATCH));
+    memcpy(h + off_l, &n_boxes, sizeof(int));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->tris, h + off_t, tb, cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->boxes, hb, bb, cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->box_offsets, h + off_o, ob, cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaMemcpyAsync(ctx->box_indices, h + off_i, ib, cudaMemcpyHostToDevice, ctx->stream));
+    ORE_CUDA(ctx, cudaMemcpyAsync(ctx->mesh_live, h + off_l, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     // the leaf balls by the kernel the device update runs too (ore_mesh_refit.cu): one code path for box_sph
     ORE_CUDA(ctx, ore_mesh_balls(ctx->boxes, ctx->box_sph, n_boxes, ctx->stream));
     ORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->n_tris = n_tris;
     ctx->n_boxes = n_boxes;
+    ctx->mesh_n_idx = n_idx;
     ctx->mesh_has_normals = has_normals ? 1 : 0;
+    return ORE_OK;
+}
+
+extern "C" int ore_set_mesh_device(ore_context* ctx, const float* tris27_dev, int32_t n_tris, int32_t has_normals, void* stream) {
+    if (!ctx) return ORE_ERR_INVALID;
+    if (n_tris < 1)
+        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_device: n_tris must be >= 1 (remove the mesh with ore_set_mesh(ctx, NULL, 0, ...))");
+    if ((size_t)n_tris > (size_t)INT32_MAX / ore_host::TRI_FLOATS) return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_device: too many triangles");
+    if (!tris27_dev || ((uintptr_t)tris27_dev & 3))
+        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_device: the triangles must be 4-byte aligned");
+    ORE_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!on_context_gpu(ctx, tris27_dev))
+        return fail(ctx, ORE_ERR_INVALID, "ore_set_mesh_device: the triangles must be device memory of the context's GPU");
+    const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+    const int L = ore_mesh_leaf_capacity(n_tris);
+    int rc;
+    if (!ctx->tris || (size_t)n_tris > ctx->mesh_tri_cap || (size_t)L > ctx->mesh_box_cap || (size_t)n_tris > ctx->mesh_idx_cap) {
+        // growth: the old buffers may still be read by a render or written by an update on another stream
+        if ((rc = wait_last_render(ctx))) return rc;
+        if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaEventSynchronize(ctx->ev_scene));
+        const size_t tri_cap = std::max(ctx->mesh_tri_cap, (size_t)n_tris);
+        if ((rc = mesh_alloc(ctx, tri_cap, std::max(ctx->mesh_box_cap, (size_t)L), std::max(ctx->mesh_idx_cap, tri_cap)))) return rc;
+    }
+    // after every render submitted so far and the previous update, on whatever streams they ran; the host never waits
+    if (ctx->ev_done_set) ORE_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_done, 0));
+    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_scene, 0));
+    ORE_CUDA(ctx, cudaMemcpyAsync(ctx->tris, tris27_dev, (size_t)n_tris * ore_host::TRI_FLOATS * sizeof(float),
+                                  cudaMemcpyDeviceToDevice, st));
+    MeshBuildArgs a;
+    a.tris = ctx->tris;
+    a.cap_tris = (int)ctx->mesh_tri_cap;
+    a.box_offsets = ctx->box_offsets;
+    a.box_indices = ctx->box_indices;
+    a.boxes = ctx->boxes;
+    a.box_sph = ctx->box_sph;
+    a.n_live = ctx->mesh_live;
+    a.work = ctx->mesh_work;
+    a.work_bytes = ctx->mesh_work_bytes;
+    if (!ctx->mesh_graph) {   // (mesh_alloc drops it with the buffers it holds)
+        if (!ctx->mesh_capture) ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->mesh_capture, cudaStreamNonBlocking));
+        cudaGraph_t g = nullptr;
+        ORE_CUDA(ctx, cudaStreamBeginCapture(ctx->mesh_capture, cudaStreamCaptureModeThreadLocal));
+        const cudaError_t eb = ore_mesh_build(a, ctx->mesh_capture);
+        const cudaError_t ec = cudaStreamEndCapture(ctx->mesh_capture, &g);
+        if (eb != cudaSuccess || ec != cudaSuccess) {
+            if (g) cudaGraphDestroy(g);
+            ORE_CUDA(ctx, eb != cudaSuccess ? eb : ec);
+        }
+        const cudaError_t ei = cudaGraphInstantiate(&ctx->mesh_graph, g, 0);
+        cudaGraphDestroy(g);
+        if (ei != cudaSuccess) ctx->mesh_graph = nullptr;
+        ORE_CUDA(ctx, ei);
+    }
+    ORE_CUDA(ctx, ore_mesh_build_count(a, n_tris, st));
+    ORE_CUDA(ctx, cudaGraphLaunch(ctx->mesh_graph, st));
+    ORE_CUDA(ctx, cudaEventRecord(ctx->ev_scene, st));
+    ctx->ev_scene_set = true;
+    ctx->n_tris = n_tris;
+    ctx->n_boxes = L;
+    ctx->mesh_n_idx = n_tris;
+    ctx->mesh_has_normals = has_normals != 0 ? 1 : 0;
     return ORE_OK;
 }
 
@@ -962,6 +1071,7 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
     prm.box_cone = ctx->box_cone;
     prm.n_tris = ctx->n_tris;
     prm.n_boxes = ctx->n_boxes;
+    prm.n_live_boxes = ctx->mesh_live;
     prm.mesh_has_normals = ctx->mesh_has_normals;
     {
         bool skip = ctx->tex_finite && !(fr->flags & ORE_FLAG_EXHAUSTIVE);
@@ -1545,15 +1655,16 @@ extern "C" int ore_debug_sphere_tree(ore_context* ctx, int32_t which, void* host
 }
 
 extern "C" int ore_debug_mesh(ore_context* ctx, int32_t which, void* host_out, int32_t n_items) {
-    if (!ctx || which < 0 || which > 2 || n_items < 0 || (n_items > 0 && !host_out)) return ORE_ERR_INVALID;
+    if (!ctx || which < 0 || which > 5 || n_items < 0 || (n_items > 0 && !host_out)) return ORE_ERR_INVALID;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
     ORE_CUDA(ctx, cudaDeviceSynchronize());
     if (ctx->n_tris == 0) return fail(ctx, ORE_ERR_INVALID, "ore_debug_mesh: no mesh set");
-    const void* src[3] = {ctx->tris, ctx->boxes, ctx->box_sph};
-    const size_t count[3] = {(size_t)ctx->n_tris * ore_host::TRI_FLOATS, 2 * (size_t)ctx->n_boxes, (size_t)ctx->n_boxes};
+    const void* src[6] = {ctx->tris, ctx->boxes, ctx->box_sph, ctx->box_offsets, ctx->box_indices, ctx->mesh_live};
+    const size_t count[6] = {(size_t)ctx->n_tris * ore_host::TRI_FLOATS, 2 * (size_t)ctx->n_boxes, (size_t)ctx->n_boxes,
+                             (size_t)ctx->n_boxes + 1, (size_t)ctx->mesh_n_idx, 1};
+    const size_t item[6] = {sizeof(float), sizeof(float4), sizeof(float4), sizeof(int), sizeof(int), sizeof(int)};
     if ((size_t)n_items != count[which]) return fail(ctx, ORE_ERR_INVALID, "ore_debug_mesh: n_items must be the array's length");
-    if (n_items > 0)
-        ORE_CUDA(ctx, cudaMemcpy(host_out, src[which], (size_t)n_items * (which == 0 ? sizeof(float) : sizeof(float4)), cudaMemcpyDeviceToHost));
+    if (n_items > 0) ORE_CUDA(ctx, cudaMemcpy(host_out, src[which], (size_t)n_items * item[which], cudaMemcpyDeviceToHost));
     return ORE_OK;
 }
 

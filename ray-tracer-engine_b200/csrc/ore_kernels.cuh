@@ -142,7 +142,10 @@ struct FrameParams {
     float4* box_cone;         // tile-cone record of each leaf box (camera frame; frame f at base + f * n_boxes)
     const int* box_offsets;
     const int* box_indices;
+    // n_boxes: the leaf capacity (box_cone's stride); the leaves in use are the first *n_live_boxes (a device build
+    // learns its leaf count on the device; ore_set_mesh: n_boxes), the rest list no triangles and are never read
     int n_tris, n_boxes, mesh_has_normals;
+    const int* n_live_boxes;
     // 1: a light whose castLightRay factor a = normal.toL is not > 0 contributes exactly +0 to the pixel whatever its
     // shadow rays do (kernel.cu:1541-1542, 1673-1675: b *= a > 0 ? a : 0 with b finite, then b * colour * texel with
     // finite colours and texels), so its directions and its sweep are skipped.  0 (exhaustive mode, or a non-finite

@@ -18,20 +18,8 @@ constexpr int REFIT_THREADS = 256;
 constexpr unsigned FULL = 0xffffffffu;
 constexpr int NO_POS = 0x7fffffff;   // with a NaN value: no coordinate taken yet
 
-// (v, p) <- (w, q) when w is beyond v, or equal to it and earlier in the list, or when (v, p) holds nothing yet.  A NaN
-// w never displaces a coordinate (both comparisons are false), and displacing "nothing" by a NaN still holds nothing.
-__device__ __forceinline__ void take_hi(float& v, int& p, float w, int q) {
-    if (w > v || (w == v && q < p) || isnan(v)) {
-        v = w;
-        p = q;
-    }
-}
-__device__ __forceinline__ void take_lo(float& v, int& p, float w, int q) {
-    if (w < v || (w == v && q < p) || isnan(v)) {
-        v = w;
-        p = q;
-    }
-}
+using ore_host::take_hi;
+using ore_host::take_lo;
 
 __global__ void __launch_bounds__(REFIT_THREADS) mesh_refit_kernel(const float* __restrict__ tris, const int* __restrict__ offs,
                                                                    const int* __restrict__ idx, float4* __restrict__ boxes,
@@ -71,16 +59,9 @@ __global__ void __launch_bounds__(REFIT_THREADS) mesh_refit_kernel(const float* 
         }
     if (lane != 0) return;
     // the seeds come first in the rule's order: the reduced coordinate replaces one only when strictly beyond it
-    const float* first = tris + (size_t)idx[o0] * ore_host::TRI_FLOATS;
-    const float* last = tris + (size_t)idx[o0 + m - 1] * ore_host::TRI_FLOATS;
     float blo[3], bhi[3];
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        blo[k] = first[k];
-        bhi[k] = last[k];
-        ore_host::grow_lo(lo[k], blo[k]);
-        ore_host::grow_hi(hi[k], bhi[k]);
-    }
+    ore_host::seed_and_grow(tris + (size_t)idx[o0] * ore_host::TRI_FLOATS, tris + (size_t)idx[o0 + m - 1] * ore_host::TRI_FLOATS,
+                            lo, hi, blo, bhi);
     boxes[2 * j] = make_float4(blo[0], blo[1], blo[2], 0.f);
     boxes[2 * j + 1] = make_float4(bhi[0], bhi[1], bhi[2], 0.f);
 }

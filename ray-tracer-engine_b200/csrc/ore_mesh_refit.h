@@ -24,6 +24,35 @@ ORE_HD inline void grow_lo(float v, float& lo) {
     if (v < lo) lo = v;
 }
 
+// The same rule as a reduction (the device refit and build): (v, p) <- (w, q) when w is beyond v, or equal to it and
+// earlier in the list, or when (v, p) holds nothing yet (v NaN).  A NaN w never displaces a coordinate (both comparisons
+// are false), and displacing "nothing" by a NaN still holds nothing.  "Larger value, or equal value and earlier position"
+// is associative and commutative, so the order of reduction does not matter.
+ORE_HD inline void take_hi(float& v, int& p, float w, int q) {
+    if (w > v || (w == v && q < p) || isnan(v)) {
+        v = w;
+        p = q;
+    }
+}
+ORE_HD inline void take_lo(float& v, int& p, float w, int q) {
+    if (w < v || (w == v && q < p) || isnan(v)) {
+        v = w;
+        p = q;
+    }
+}
+
+// The seed step: the seeds come first in the rule's order (lo from the first listed triangle's first vertex, hi from the
+// last listed triangle's), and the reduced extremes (NaN: none taken) replace them only when strictly beyond.
+ORE_HD inline void seed_and_grow(const float* first, const float* last, const float lo_ext[3], const float hi_ext[3], float lo[3],
+                                 float hi[3]) {
+    for (int k = 0; k < 3; k++) {
+        lo[k] = first[k];
+        hi[k] = last[k];
+        grow_lo(lo_ext[k], lo[k]);
+        grow_hi(hi_ext[k], hi[k]);
+    }
+}
+
 // CPU reference of a leaf box: lo seeded with the first listed triangle's first vertex, hi with the last listed
 // triangle's, then every vertex of every listed triangle grows them in list order.  m == 0: the box is left as it is.
 inline void mesh_leaf_box(const float* tris27, const int32_t* idx, int m, float lo[3], float hi[3]) {

@@ -106,7 +106,7 @@ __global__ void prep_frame_kernel(const FrameParams prm) {
             }
             prm.super_cone[(size_t)f * prm.n_supers_pad + i] = cone;
         }
-        if (i < prm.n_boxes) {
+        if (i < prm.n_boxes && i < __ldg(prm.n_live_boxes)) {
             // tile-cone record of leaf box i of the mesh from its bounding sphere (same formula).  An eye on a face plane
             // of the box makes it always a candidate: a primary ray with a +-0 component on that axis can pass the slab
             // test through a NaN slab and then hit a triangle the box does not contain (ore_kernels.cuh, zero_axes)
@@ -356,12 +356,13 @@ __global__ void __launch_bounds__(PRIMARY_THREADS, ORE_PRIMARY_MIN_CTAS) primary
         //      Lane i tests leaf box s0+i (its bounding sphere) against the tile cone; surviving leaves, in
         //      ascending order, get the exact slab + triangle tests per pixel. ----
         if (prm.n_boxes) {
-            const MeshArgs ma = {prm.tris, prm.boxes, prm.box_offsets, prm.box_indices, prm.n_boxes};
+            const int n_live = __shfl_sync(0xffffffffu, lane == 0 ? __ldg(prm.n_live_boxes) : 0, 0);   // (one load per warp)
+            const MeshArgs ma = {prm.tris, prm.boxes, prm.box_offsets, prm.box_indices, n_live};
             const int id_base = prm.n_spheres + prm.n_cubes + prm.n_planes;
 #pragma unroll 1
-            for (int s0 = 0; s0 < prm.n_boxes; s0 += 32) {
+            for (int s0 = 0; s0 < n_live; s0 += 32) {
                 bool cand = false;
-                if (s0 + lane < prm.n_boxes) cand = EXH || cone_touches(ax, ay, az, __ldg(&prm.box_cone[(size_t)frame * prm.n_boxes + s0 + lane]));
+                if (s0 + lane < n_live) cand = EXH || cone_touches(ax, ay, az, __ldg(&prm.box_cone[(size_t)frame * prm.n_boxes + s0 + lane]));
                 uint32_t mask = __ballot_sync(0xffffffffu, cand && tile_ok);
                 while (mask) {
                     const int i = __ffs(mask) - 1;

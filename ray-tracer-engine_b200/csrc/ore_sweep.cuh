@@ -84,6 +84,8 @@ __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_ke
     const int n_sph = prm.n_spheres, n_leaf = prm.n_leaves, n_sup = prm.n_supers;
     const uint32_t n_items = (uint32_t)prm.counters[CNT_HITS];
     const int NLI = prm.n_lights;
+    // the live leaf count of the mesh (the leaves past it list no triangles), loaded once
+    const int n_live_boxes = prm.n_boxes ? __shfl_sync(0xffffffffu, lane == 0 ? __ldg(prm.n_live_boxes) : 0, 0) : 0;
     unsigned long long n_exact = 0;
     unsigned int n_l1 = 0, n_l2 = 0, n_steps = 0;
 
@@ -408,7 +410,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_ke
             if (prm.n_boxes && valid) {
                 const uint32_t live = ~blocked & 0x3ffu;
                 if (live) {
-                    const MeshArgs ma = {prm.tris, prm.boxes, prm.box_offsets, prm.box_indices, prm.n_boxes};
+                    const MeshArgs ma = {prm.tris, prm.boxes, prm.box_offsets, prm.box_indices, n_live_boxes};
                     blocked |= mesh_blocks_light(ma, prm.box_sph, start.x, start.y, start.z, Ax, Ay, Az, ca, sa, use_cone, zaxes, dslot, 32, live);
                 }
             }
