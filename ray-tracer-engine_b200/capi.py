@@ -146,6 +146,11 @@ def _fptr(a: np.ndarray):
     return a.ctypes.data_as(C.POINTER(C.c_float))
 
 
+def _stream(stream: int):
+    """a raw cudaStream_t for the ABI; 0 = the context's render stream"""
+    return C.c_void_p(stream) if stream else None
+
+
 class Renderer:
     """One render context on one GPU (mirrors the reference's global scene + update())."""
 
@@ -165,6 +170,23 @@ class Renderer:
     def _check(self, rc, what):
         if rc != 0:
             raise OreError(f"{what} failed rc={rc}: {self.lib.ore_last_error(self.ctx).decode()}")
+
+    def _device_tensor(self, t, what: str, cols: int, rows: int | None = None, min_rows: int = 0) -> int:
+        """the argument checks of a stream-ordered setter: a contiguous torch float32 tensor of shape (n, cols) on this
+        context's GPU with n == rows (or n >= min_rows); returns n"""
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{what}: expected a torch.Tensor, got {type(t).__name__}")
+        if t.dtype != torch.float32:
+            raise TypeError(f"{what}: expected dtype torch.float32, got {t.dtype}")
+        if t.dim() != 2 or t.shape[1] != cols or (t.shape[0] != rows if rows is not None else t.shape[0] < min_rows):
+            want = f"({rows}, {cols})" if rows is not None else f"(n, {cols})" + (f" with n >= {min_rows}" if min_rows else "")
+            raise ValueError(f"{what}: expected shape {want}, got {tuple(t.shape)}")
+        if t.device.type != "cuda" or t.device.index != self.device:
+            raise ValueError(f"{what}: the tensor must live on cuda:{self.device}, not {t.device}")
+        if not t.is_contiguous():
+            raise ValueError(f"{what}: the tensor must be contiguous")
+        return int(t.shape[0])
 
     def close(self):
         if self.ctx:
@@ -191,21 +213,9 @@ class Renderer:
         """Stream-ordered sphere update from a torch CUDA float32 tensor of shape (n, 4) (cx, cy, cz, radius member) on
         this context's GPU.  `stream`: a raw cudaStream_t (e.g. torch.cuda.current_stream().cuda_stream; 0 = the
         context's render stream).  Keep `t` alive and unchanged until the update has run on that stream."""
-        import torch
-        if not isinstance(t, torch.Tensor):
-            raise TypeError(f"set_spheres_device: expected a torch.Tensor, got {type(t).__name__}")
-        if t.dtype != torch.float32:
-            raise TypeError(f"set_spheres_device: expected dtype torch.float32, got {t.dtype}")
-        if t.dim() != 2 or t.shape[1] != 4:
-            raise ValueError(f"set_spheres_device: expected shape (n, 4), got {tuple(t.shape)}")
-        if t.device.type != "cuda" or t.device.index != self.device:
-            raise ValueError(f"set_spheres_device: the tensor must live on cuda:{self.device}, not {t.device}")
-        if not t.is_contiguous():
-            raise ValueError("set_spheres_device: the tensor must be contiguous")
-        n = int(t.shape[0])
-        ptr = t.data_ptr() if n else 0
-        self._check(self.lib.ore_set_spheres_device(self.ctx, C.c_void_p(ptr) if ptr else None, n,
-                                                     C.c_void_p(stream) if stream else None), "ore_set_spheres_device")
+        n = self._device_tensor(t, "set_spheres_device", 4)
+        self._check(self.lib.ore_set_spheres_device(self.ctx, C.c_void_p(t.data_ptr()) if n else None, n, _stream(stream)),
+                    "ore_set_spheres_device")
 
     def debug_sphere_tree(self, which: str, n: int) -> np.ndarray:
         """one array of the sphere hierarchy of the current n-sphere scene, read back after a device synchronise
@@ -243,20 +253,9 @@ class Renderer:
         (the records of set_mesh) on this context's GPU, with the reference's flat BVH built on the GPU: the leaves
         equal the host builder's bit for bit.  `stream`: a raw cudaStream_t (0 = the context's render stream).  Keep `t`
         alive and unchanged until the update has run on that stream."""
-        import torch
-        if not isinstance(t, torch.Tensor):
-            raise TypeError(f"set_mesh_device: expected a torch.Tensor, got {type(t).__name__}")
-        if t.dtype != torch.float32:
-            raise TypeError(f"set_mesh_device: expected dtype torch.float32, got {t.dtype}")
-        if t.dim() != 2 or t.shape[1] != 27 or t.shape[0] < 1:
-            raise ValueError(f"set_mesh_device: expected shape (n, 27) with n >= 1, got {tuple(t.shape)}")
-        if t.device.type != "cuda" or t.device.index != self.device:
-            raise ValueError(f"set_mesh_device: the tensor must live on cuda:{self.device}, not {t.device}")
-        if not t.is_contiguous():
-            raise ValueError("set_mesh_device: the tensor must be contiguous")
-        n = int(t.shape[0])
-        self._check(self.lib.ore_set_mesh_device(self.ctx, C.c_void_p(t.data_ptr()), n, int(bool(has_normals)),
-                                                 C.c_void_p(stream) if stream else None), "ore_set_mesh_device")
+        n = self._device_tensor(t, "set_mesh_device", 27, min_rows=1)
+        self._check(self.lib.ore_set_mesh_device(self.ctx, C.c_void_p(t.data_ptr()), n, int(bool(has_normals)), _stream(stream)),
+                    "ore_set_mesh_device")
         self._mesh_counts = (n, min(MESH_MAX_LEAVES, n))   # (leaf capacity: the live count is on the device)
         self._mesh_n_idx = n
 
@@ -265,20 +264,8 @@ class Renderer:
         records of set_mesh) on this context's GPU; the leaf boxes and their spheres are recomputed on the GPU and the
         topology of the last set_mesh stays.  `stream`: a raw cudaStream_t (0 = the context's render stream).  Keep `t`
         alive and unchanged until the update has run on that stream."""
-        import torch
-        if not isinstance(t, torch.Tensor):
-            raise TypeError(f"set_mesh_triangles_device: expected a torch.Tensor, got {type(t).__name__}")
-        if t.dtype != torch.float32:
-            raise TypeError(f"set_mesh_triangles_device: expected dtype torch.float32, got {t.dtype}")
-        n_tris = getattr(self, "_mesh_counts", (0, 0))[0]
-        if t.dim() != 2 or t.shape[1] != 27 or t.shape[0] != n_tris:
-            raise ValueError(f"set_mesh_triangles_device: expected shape ({n_tris}, 27), got {tuple(t.shape)}")
-        if t.device.type != "cuda" or t.device.index != self.device:
-            raise ValueError(f"set_mesh_triangles_device: the tensor must live on cuda:{self.device}, not {t.device}")
-        if not t.is_contiguous():
-            raise ValueError("set_mesh_triangles_device: the tensor must be contiguous")
-        self._check(self.lib.ore_set_mesh_triangles_device(self.ctx, C.c_void_p(t.data_ptr()), n_tris,
-                                                           C.c_void_p(stream) if stream else None),
+        n_tris = self._device_tensor(t, "set_mesh_triangles_device", 27, rows=getattr(self, "_mesh_counts", (0, 0))[0])
+        self._check(self.lib.ore_set_mesh_triangles_device(self.ctx, C.c_void_p(t.data_ptr()), n_tris, _stream(stream)),
                     "ore_set_mesh_triangles_device")
 
     def debug_mesh(self, which: str) -> np.ndarray:
@@ -366,8 +353,8 @@ class Renderer:
         """Render into DEVICE memory at `out_ptr` (asynchronous on `stream`)."""
         f = self._frame(width, height, y0, y1, y_step, aspect, flags, out_pitch, y_block)
         cam = self._cam(camera)
-        self._check(self.lib.ore_render_device(self.ctx, C.byref(cam), C.byref(f), C.c_void_p(out_ptr),
-                                               C.c_void_p(stream) if stream else None), "ore_render_device")
+        self._check(self.lib.ore_render_device(self.ctx, C.byref(cam), C.byref(f), C.c_void_p(out_ptr), _stream(stream)),
+                    "ore_render_device")
 
     # ---- batches of frames (one launch set for several cameras) ----
     def _cams(self, cameras):
@@ -383,7 +370,7 @@ class Renderer:
         f = self._frame(width, height, y0, y1, y_step, aspect, flags, out_pitch, y_block)
         ptrs = (C.c_void_p * len(out_ptrs))(*[int(p) for p in out_ptrs])
         self._check(self.lib.ore_render_batch_device(self.ctx, self._cams(cameras), len(cameras), C.byref(f), ptrs,
-                                                     C.c_void_p(stream) if stream else None), "ore_render_batch_device")
+                                                     _stream(stream)), "ore_render_batch_device")
 
     def render_batch_async(self, cameras, width, height, outs, y0=0, y1=None, y_step=1, aspect=None, flags=0, y_block=1,
                            in_place=False, done_flag: int = 0, first_done_value: int = 0):
@@ -464,17 +451,17 @@ class Renderer:
         return int(self.lib.ore_get_stream(self.ctx, which) or 0)
 
     def flag_write(self, flag_ptr: int, value: int, stream: int = 0):
-        self._check(self.lib.ore_flag_write(self.ctx, C.c_void_p(stream) if stream else None, C.c_void_p(flag_ptr),
-                                            int(value) & 0xffffffff), "ore_flag_write")
+        self._check(self.lib.ore_flag_write(self.ctx, _stream(stream), C.c_void_p(flag_ptr), int(value) & 0xffffffff),
+                    "ore_flag_write")
 
     def flag_write_after(self, flag_ptr: int, value: int, stream: int = 0):
         """ordered variant: issued from this context's signal stream once `stream`'s work so far is complete"""
-        self._check(self.lib.ore_flag_write_after(self.ctx, C.c_void_p(stream) if stream else None, C.c_void_p(flag_ptr),
+        self._check(self.lib.ore_flag_write_after(self.ctx, _stream(stream), C.c_void_p(flag_ptr),
                                                   int(value) & 0xffffffff), "ore_flag_write_after")
 
     def flag_wait_geq(self, flag_ptr: int, value: int, stream: int = 0):
-        self._check(self.lib.ore_flag_wait_geq(self.ctx, C.c_void_p(stream) if stream else None, C.c_void_p(flag_ptr),
-                                               int(value) & 0xffffffff), "ore_flag_wait_geq")
+        self._check(self.lib.ore_flag_wait_geq(self.ctx, _stream(stream), C.c_void_p(flag_ptr), int(value) & 0xffffffff),
+                    "ore_flag_wait_geq")
 
     def wait(self):
         self._check(self.lib.ore_wait(self.ctx), "ore_wait")

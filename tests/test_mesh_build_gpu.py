@@ -8,11 +8,12 @@ import ctypes as C
 import numpy as np
 import pytest
 
+from streamlib import _held_stream, assert_rejected
 from test_host_mesh import host_build, host_lib, write_grid_obj  # noqa: F401  (fixture re-export)
 from test_mesh_build_cpu import AWKWARD_CASES, build_probe, leaves_1024
 from test_mesh_refit_cpu import boxes6, torus_arrays
 from test_mesh_refit_cpu import build_probe as build_refit_probe
-from test_mesh_update_gpu import _held_stream, deformed
+from test_mesh_update_gpu import deformed
 from test_parity_gpu import assert_pixels_close, libm_matches  # noqa: F401  (fixture re-export)
 
 pytestmark = pytest.mark.gpu
@@ -342,10 +343,8 @@ def test_invalid_arguments_are_rejected_and_change_nothing(renderer, build_probe
                (good.data_ptr(), -1)]
         if torch.cuda.device_count() > 1:
             bad.append((torch.from_numpy(moved).to("cuda:1").data_ptr(), n))
-        for ptr, k in bad:
-            rc = lib.ore_set_mesh_device(ctx, C.c_void_p(ptr) if ptr else None, k, 1, None)
-            assert rc == 1, (ptr, k, rc)
-            assert np.array_equal(renderer.render(cam, 160, 120), want), (ptr, k)
+        assert_rejected(lambda ptr, k: lib.ore_set_mesh_device(ctx, ptr or None, k, 1, None), bad,
+                        lambda: renderer.render(cam, 160, 120), want)
         assert np.array_equal(renderer.debug_mesh("tris"), torus)
         assert np.array_equal(renderer.debug_mesh("box_indices"), sc.mesh.box_indices)
         for t, err in ((good.double(), TypeError), (good[:, :26].contiguous(), ValueError), (good[:0], ValueError),
@@ -361,6 +360,44 @@ def test_invalid_arguments_are_rejected_and_change_nothing(renderer, build_probe
         assert np.array_equal(renderer.debug_mesh("tris"), moved)
     finally:
         renderer.host_free(pinned)
+        renderer.set_mesh(None)
+
+
+def test_rejected_set_mesh_keeps_the_mesh_and_its_capacity(renderer, build_probe_lib, host_lib, tmp_path, pkg):
+    """ore_set_mesh checks its host arrays before it frees anything: a rejected call leaves the mesh, and the capacity a
+    larger device build reached, so a device build of that size afterwards still does not block the host"""
+    import torch
+    torus = torus_arrays()[0]
+    sc = _scene(pkg, host_mesh(pkg, build_probe_lib, torus))
+    m = sc.mesh
+    cam = pkg.scene.orbit_camera(sc, 10)
+    big = torch.from_numpy(np.ascontiguousarray(grid_tris(host_lib, tmp_path, 101))).to("cuda:0")   # 20 000 triangles
+    lib, ctx = renderer.lib, renderer.ctx
+    ip = C.POINTER(C.c_int32)
+    descending, shifted, out_of_range = m.box_offsets.copy(), m.box_offsets.copy(), m.box_indices.copy()
+    descending[m.n_boxes // 2] = descending[m.n_boxes // 2 + 1] + 1
+    shifted[0] = 1
+    out_of_range[len(out_of_range) // 2] = m.n_tris
+
+    def set_mesh(offsets, indices):
+        return lib.ore_set_mesh(ctx, m.tris.ctypes.data_as(C.POINTER(C.c_float)), m.n_tris, 1,
+                                m.box_bounds.ctypes.data_as(C.POINTER(C.c_float)), offsets.ctypes.data_as(ip),
+                                indices.ctypes.data_as(ip), m.n_boxes)
+
+    try:
+        renderer.set_scene(sc)
+        renderer.set_mesh_device(big, True)
+        renderer.set_mesh(m)
+        want = renderer.render(cam, 160, 120).copy()
+        assert (renderer.hits(120, 160)[0] >= 64 + 4 + 1).any(), "the mesh must be visible"
+        assert_rejected(set_mesh, [(descending, m.box_indices), (shifted, m.box_indices), (m.box_offsets, out_of_range)],
+                        lambda: renderer.render(cam, 160, 120), want)
+        assert np.array_equal(renderer.debug_mesh("tris"), m.tris)
+        assert np.array_equal(renderer.debug_mesh("box_indices"), m.box_indices)
+        assert renderer.debug_mesh("n_live")[0] == m.n_boxes
+        dt, pending = _held_stream(renderer, lambda s: renderer.set_mesh_device(big, True, s))
+        assert dt < 0.5 and pending, dt
+    finally:
         renderer.set_mesh(None)
 
 

@@ -3,12 +3,12 @@ spheres refit on the GPU (csrc/ore_mesh_refit.cu): the device arrays against the
 csrc/ore_mesh_refit.h byte for byte, animated frames against the oracle, ordering across streams, no host blocking,
 ore_set_mesh behind a pending update, and argument validation."""
 import ctypes as C
-import threading
 import time
 
 import numpy as np
 import pytest
 
+from streamlib import _held_stream, assert_rejected
 from test_host_mesh import host_build, host_lib, write_grid_obj  # noqa: F401  (fixture re-export)
 from test_mesh_refit_cpu import awkward_mesh, boxes6, build_probe, torus_arrays
 from test_parity_gpu import assert_pixels_close, libm_matches  # noqa: F401  (fixture re-export)
@@ -223,35 +223,6 @@ def test_update_on_another_stream_is_ordered_between_renders(renderer, pkg):
 
 # ---- 4. no host blocking; 5. ore_set_mesh behind a pending update ------------------------------------------------------
 
-def _held_stream(renderer, update, after=None):
-    """enqueues `update` on a stream held by a host flag; returns (seconds the call took, still pending at return);
-    `after` runs while the stream is still held"""
-    import torch
-    flag = renderer.host_alloc((16,))
-    flag[:] = 0
-    S = torch.cuda.Stream()
-    timer = threading.Timer(2.0, lambda: flag.__setitem__(0, 1))   # releases the stream in every case
-    try:
-        torch.cuda.synchronize()
-        renderer.flag_wait_geq(flag.ctypes.data, 1, S.cuda_stream)
-        timer.start()
-        t0 = time.perf_counter()
-        update(S.cuda_stream)
-        dt = time.perf_counter() - t0
-        pending = not S.query()
-        if after is not None:
-            after()
-        timer.join()
-        S.synchronize()
-        return dt, pending
-    finally:
-        timer.cancel()
-        flag[0] = 1
-        torch.cuda.synchronize()
-        renderer.synchronize()
-        renderer.host_free(flag)
-
-
 def test_update_does_not_block_the_host(renderer, mesh_probe, pkg):
     import torch
     m = _scene(pkg, None).mesh
@@ -320,10 +291,8 @@ def test_invalid_arguments_are_rejected_and_change_nothing(renderer, pkg):
                (good.data_ptr(), n + 1), (good.data_ptr(), -1), (good.data_ptr(), 0)]
         if torch.cuda.device_count() > 1:
             bad.append((torch.from_numpy(moved).to("cuda:1").data_ptr(), n))
-        for ptr, k in bad:
-            rc = lib.ore_set_mesh_triangles_device(ctx, C.c_void_p(ptr) if ptr else None, k, None)
-            assert rc == 1, (ptr, k, rc)
-            assert np.array_equal(renderer.render(cam, 160, 120), want), (ptr, k)
+        assert_rejected(lambda ptr, k: lib.ore_set_mesh_triangles_device(ctx, ptr or None, k, None), bad,
+                        lambda: renderer.render(cam, 160, 120), want)
         assert np.array_equal(renderer.debug_mesh("tris"), m.tris)
         # the Python binding checks before the call
         for t, err in ((good.double(), TypeError), (good[:, :26].contiguous(), ValueError), (good[:-1], ValueError),

@@ -4,12 +4,11 @@ frames against the oracle, ordering across streams, no host blocking, argument v
 import ctypes as C
 import os
 import subprocess
-import threading
-import time
 
 import numpy as np
 import pytest
 
+from streamlib import _held_stream, assert_rejected
 from test_parity_gpu import assert_pixels_close, libm_matches  # noqa: F401  (fixture re-export)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -257,29 +256,10 @@ def test_update_with_capacity_does_not_block_the_host(renderer, tree_probe, pkg)
     sp2[:, 0] += np.float32(0.5)
     renderer.set_spheres(sp)                   # sizes the buffers for 4096 spheres
     t2 = torch.from_numpy(sp2).to("cuda:0")
-    torch.cuda.synchronize()
-    flag = renderer.host_alloc((16,))
-    flag[:] = 0
-    S = torch.cuda.Stream()
-    timer = threading.Timer(2.0, lambda: flag.__setitem__(0, 1))   # releases the stream in every case
-    try:
-        renderer.flag_wait_geq(flag.ctypes.data, 1, S.cuda_stream)
-        timer.start()
-        t0 = time.perf_counter()
-        renderer.set_spheres_device(t2, S.cuda_stream)
-        dt = time.perf_counter() - t0
-        pending = not S.query()
-        timer.join()
-        S.synchronize()
-        assert dt < 0.5, dt
-        assert pending, "the update must still be waiting behind the held stream"
-        assert_same_tree(read_tree(renderer, len(sp2)), tree_probe(sp2), "after release")
-    finally:
-        timer.cancel()
-        flag[0] = 1
-        torch.cuda.synchronize()
-        renderer.synchronize()
-        renderer.host_free(flag)
+    dt, pending = _held_stream(renderer, lambda s: renderer.set_spheres_device(t2, s))
+    assert dt < 0.5, dt
+    assert pending, "the update must still be waiting behind the held stream"
+    assert_same_tree(read_tree(renderer, len(sp2)), tree_probe(sp2), "after release")
 
 
 # ---- 5. validation ---------------------------------------------------------------------------------------------------
@@ -302,10 +282,8 @@ def test_invalid_pointers_are_rejected_and_change_nothing(renderer, pkg):
                (0, 64)]
         if torch.cuda.device_count() > 1:
             bad.append((torch.from_numpy(host).to("cuda:1").data_ptr(), 64))
-        for ptr, n in bad:
-            rc = lib.ore_set_spheres_device(ctx, C.c_void_p(ptr) if ptr else None, n, None)
-            assert rc == 1, (ptr, n, rc)
-            assert np.array_equal(renderer.render(cam, 160, 120), want), (ptr, n)
+        assert_rejected(lambda ptr, n: lib.ore_set_spheres_device(ctx, ptr or None, n, None), bad,
+                        lambda: renderer.render(cam, 160, 120), want)
         # the Python binding checks before the call
         for t, err in ((other.double(), TypeError), (other[:, :3].contiguous(), ValueError), (other.cpu(), ValueError),
                        (other.t().contiguous().t(), ValueError), (host, TypeError)):
