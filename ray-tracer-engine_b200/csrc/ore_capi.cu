@@ -25,15 +25,6 @@
 
 using namespace ore;
 
-// second instantiation of the default-path kernels with CUDA's libm (ore_fast.cu)
-extern "C" int ore_fast_set_tables(const float* cphi, const float* sphi, const float* bk);
-extern "C" int ore_fast_primary_tile(const void* prm, int sm_count, size_t smem, long long n_batches, int exh,
-                                     cudaStream_t stream);
-// stage: a StageArgs of identical layout; staged = 0 selects the fused form (only first_block is used then)
-extern "C" int ore_fast_shadow_sweep(const void* prm, const void* stage, int staged, int sm_count, size_t smem, int exh,
-                                     cudaStream_t stream);
-extern "C" int ore_fast_shade_setup(const void* prm, const void* stage, int sm_count, cudaStream_t stream);
-
 struct ore_context {
     int device = 0;
     int sm_count = 0;
@@ -328,7 +319,6 @@ extern "C" int ore_create(ore_context** out, int device) {
         }
     }
     ORE_CUDA(ctx, cudaMemcpyToSymbol(c_b_of_k, bk, sizeof bk));
-    if (ore_fast_set_tables(cphi, sphi, bk)) return fail(ctx, ORE_ERR_CUDA, "constant tables of the fast-libm kernels");
     return ORE_OK;
 }
 
@@ -873,26 +863,27 @@ static int frame_rows(const ore_frame* fr) {
     return full * yb + (rem < yb ? rem : yb);
 }
 
+// the instantiation of each render kernel that a frame's flags select, indexed [exhaustive][staged][fast libm] (the
+// indices the kernel has)
+using PrimaryKernel = void (*)(FrameParams);
+using StageKernel = void (*)(FrameParams, StageArgs);
+static constexpr PrimaryKernel primary_kernels[2][2] = {
+    {primary_tile_kernel<TILE_ROWS, false, false>, primary_tile_kernel<TILE_ROWS, false, true>},
+    {primary_tile_kernel<TILE_ROWS, true, false>, primary_tile_kernel<TILE_ROWS, true, true>}};
+static constexpr StageKernel sweep_kernels[2][2][2] = {
+    {{shadow_sweep_kernel<false, false, false>, shadow_sweep_kernel<false, false, true>},
+     {shadow_sweep_kernel<false, true, false>, shadow_sweep_kernel<false, true, true>}},
+    {{shadow_sweep_kernel<true, false, false>, shadow_sweep_kernel<true, false, true>},
+     {shadow_sweep_kernel<true, true, false>, shadow_sweep_kernel<true, true, true>}}};
+static constexpr StageKernel shade_setup_kernels[2] = {shade_setup_kernel<false>, shade_setup_kernel<true>};
+
 // one launch of the sweep kernel (stage B / fused / catch-all)
 static int launch_sweep(ore_context* ctx, const FrameParams& prm, const StageArgs& st, bool staged, bool exh, bool fast_libm,
                         cudaStream_t stream) {
     int rc, grid = 0;
-    const size_t smem = SWEEP_SMEM_BYTES;
-    if (fast_libm) {
-        ORE_CUDA(ctx, (cudaError_t)ore_fast_shadow_sweep(&prm, &st, staged ? 1 : 0, ctx->sm_count, smem, exh ? 1 : 0, stream));
-        return ORE_OK;
-    }
-#define ORE_SWEEP(E, S)                                                                                  \
-    do {                                                                                                 \
-        if ((rc = grid_for(ctx, shadow_sweep_kernel<E, S>, smem, &grid, SWEEP_THREADS))) return rc;      \
-        shadow_sweep_kernel<E, S><<<grid, SWEEP_THREADS, smem, stream>>>(prm, st);                       \
-    } while (0)
-    if (staged) {
-        if (exh) ORE_SWEEP(true, true); else ORE_SWEEP(false, true);
-    } else {
-        if (exh) ORE_SWEEP(true, false); else ORE_SWEEP(false, false);
-    }
-#undef ORE_SWEEP
+    const StageKernel sweep = sweep_kernels[exh][staged][fast_libm];
+    if ((rc = grid_for(ctx, sweep, SWEEP_SMEM_BYTES, &grid, SWEEP_THREADS))) return rc;
+    sweep<<<grid, SWEEP_THREADS, SWEEP_SMEM_BYTES, stream>>>(prm, st);
     ORE_CUDA(ctx, cudaGetLastError());
     return ORE_OK;
 }
@@ -1121,17 +1112,10 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
         int grid = 0;
         const long long tiles = (long long)((W + 31) / 32) * ((n_rows + TILE_ROWS - 1) / TILE_ROWS);
         const long long n_batches = ((tiles + PRIMARY_WARPS - 1) / PRIMARY_WARPS) * n_frames;
-        if (fast_libm) {
-            ORE_CUDA(ctx, (cudaError_t)ore_fast_primary_tile(&prm, ctx->sm_count, psmem, n_batches, exh ? 1 : 0, stream));
-        } else if (exh) {
-            if ((rc = grid_for(ctx, primary_tile_kernel<TILE_ROWS, true>, psmem, &grid, PRIMARY_THREADS))) return rc;
-            if (grid > n_batches) grid = (int)n_batches;
-            primary_tile_kernel<TILE_ROWS, true><<<grid, PRIMARY_THREADS, psmem, stream>>>(prm);
-        } else {
-            if ((rc = grid_for(ctx, primary_tile_kernel<TILE_ROWS, false>, psmem, &grid, PRIMARY_THREADS))) return rc;
-            if (grid > n_batches) grid = (int)n_batches;
-            primary_tile_kernel<TILE_ROWS, false><<<grid, PRIMARY_THREADS, psmem, stream>>>(prm);
-        }
+        const PrimaryKernel primary = primary_kernels[exh][fast_libm];
+        if ((rc = grid_for(ctx, primary, psmem, &grid, PRIMARY_THREADS))) return rc;
+        if (grid > n_batches) grid = (int)n_batches;
+        primary<<<grid, PRIMARY_THREADS, psmem, stream>>>(prm);
         ORE_CUDA(ctx, cudaGetLastError());
         ctx->last_launches++;
     }
@@ -1236,17 +1220,14 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
             st.cap_blocks = (uint32_t)cap_blocks;
             const int n_chunks_max = (int)((n_blocks_px + cap_blocks - 1) / cap_blocks);
             if (n_chunks > n_chunks_max) n_chunks = n_chunks_max;
+            const StageKernel setup = shade_setup_kernels[fast_libm];
             int grid_a = 0;
-            if (!fast_libm && (rc = grid_for(ctx, shade_setup_kernel, 0, &grid_a, STAGE_A_THREADS))) return rc;
+            if ((rc = grid_for(ctx, setup, 0, &grid_a, STAGE_A_THREADS))) return rc;
             for (int c = 0; c < n_chunks; c++) {
                 st.chunk = c;
                 st.first_block = (uint32_t)((size_t)c * cap_blocks);
-                if (fast_libm) {
-                    ORE_CUDA(ctx, (cudaError_t)ore_fast_shade_setup(&prm, &st, ctx->sm_count, stream));
-                } else {
-                    shade_setup_kernel<<<grid_a, STAGE_A_THREADS, 0, stream>>>(prm, st);
-                    ORE_CUDA(ctx, cudaGetLastError());
-                }
+                setup<<<grid_a, STAGE_A_THREADS, 0, stream>>>(prm, st);
+                ORE_CUDA(ctx, cudaGetLastError());
                 if ((rc = join_band())) return rc;   // (band DMA: the first stage A ran beside the copy)
                 if ((rc = launch_sweep(ctx, prm, st, true, exh, fast_libm, stream))) return rc;
                 ctx->last_launches += 2;

@@ -127,6 +127,7 @@ struct SkyArgs {
     float radius;
     float ez;
 };
+template <bool FAST_LIBM>
 __device__ __noinline__ uint32_t sky_pixel(const SkyArgs sk, const CamP cam, float dx, float dy) {
     // primary ray, kernel.cu:1624-1631 + camera::rotateDir :252-255
     const v3 D = primary_dir(cam, sk.ez, dx, dy);
@@ -136,8 +137,8 @@ __device__ __noinline__ uint32_t sky_pixel(const SkyArgs sk, const CamP cam, flo
     v3 hp = ref_add(O, ref_scale(D, t));
     v3 n = ref_sub(hp, mk(0.f, 0.f, 0.f));
     ref_normalise(n);
-    int sx = (int)((1.f + ORE_ATAN2F(n.z, n.x) / 3.1415f) * 0.5f * (float)sk.w);
-    int sy = (int)(ORE_ACOSF(n.y) / 3.1415f * (float)sk.h);
+    int sx = (int)((1.f + libm_atan2f<FAST_LIBM>(n.z, n.x) / 3.1415f) * 0.5f * (float)sk.w);
+    int sy = (int)(libm_acosf<FAST_LIBM>(n.y) / 3.1415f * (float)sk.h);
     int index = clamp_index(sy * sk.w + sx, sk.w * sk.h);
     float r = __ldg(&sk.r[index]), g = __ldg(&sk.g[index]), b = __ldg(&sk.b[index]);
     return ref_rgb_to_int((int)(r * 254.f), (int)(g * 254.f), (int)(b * 254.f));
@@ -156,7 +157,7 @@ __device__ __noinline__ uint32_t sky_pixel(const SkyArgs sk, const CamP cam, flo
 //                    within 1.2 degrees of a pole, always take the exact path);
 //   angle error      4e-6 rad for the polynomial (3.2e-7 evaluated in float, tests/test_sky_filter_cpu.py), the approximate
 //                    reciprocal (1.2e-7), the quadrant fix-ups (2.4e-7) and the 1-ulp error of either libm's atan2f / acosf
-//                    (2.4e-7; 2 ulp for CUDA's in the FAST_LIBM build) - under 1e-6 in total;
+//                    (2.4e-7; 2 ulp for CUDA's in the FAST_LIBM kernels) - under 1e-6 in total;
 //   float roundings  of the u, v expressions on both sides: < 2.7e-7 (w or h) texels, budgeted 1e-6 (w or h) + 1e-4.
 // NaNs fail every comparison and fall through to the exact path.
 // ------------------------------------------------------------------------------------
@@ -249,7 +250,7 @@ __device__ __forceinline__ bool cone_touches(float ax, float ay, float az, const
     return fmaf(ax, rec.x, fmaf(ay, rec.y, fmaf(az, rec.z, rec.w))) <= 0.f;
 }
 
-template <int P, bool EXH>
+template <int P, bool EXH, bool FAST_LIBM>
 __global__ void __launch_bounds__(PRIMARY_THREADS, ORE_PRIMARY_MIN_CTAS) primary_tile_kernel(const FrameParams prm) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t bar;
@@ -512,7 +513,7 @@ __global__ void __launch_bounds__(PRIMARY_THREADS, ORE_PRIMARY_MIN_CTAS) primary
                 if (q0 + lane < n_q) {
                     const int e = tq[q0 + lane];
                     const int kq = min(ty * P + (e >> 5), prm.n_rows - 1);
-                    tp[e] = sky_pixel(sk, cam, prm.dx_tab[tx * 32 + (e & 31)], prm.dy_tab[kq]);
+                    tp[e] = sky_pixel<FAST_LIBM>(sk, cam, prm.dx_tab[tx * 32 + (e & 31)], prm.dy_tab[kq]);
                 }
             }
             __syncwarp();

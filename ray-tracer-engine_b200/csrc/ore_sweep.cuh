@@ -64,7 +64,7 @@ __device__ __forceinline__ bool beam_touches(const Beam& b, const float4 q) {
     return !(q.w < 1e18f) || (u >= 0.f && d2 <= fmaf(thr, thr, slack));
 }
 
-template <bool EXH, bool STAGED>
+template <bool EXH, bool STAGED, bool FAST_LIBM>
 __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_kernel(const FrameParams prm, const StageArgs st) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -161,7 +161,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_ke
                 tb = sp[160];
             }
         } else if (valid) {
-            shade_point(prm, item, out_px, my_id, start, normal, tr, tg, tb);
+            shade_point<FAST_LIBM>(prm, item, out_px, my_id, start, normal, tr, tg, tb);
         }
         float fr = 0.f, fg = 0.f, fb = 0.f;
 
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_ke
                     if (!__any_sync(0xffffffffu, valid && a_dot > 0.f)) continue;   // adds +0 to every pixel of the block
                 }
                 if (valid) {
-                    a_dot = light_directions_reuse(L, start, normal, d);
+                    a_dot = light_directions_reuse<FAST_LIBM>(L, start, normal, d);
                     const float4 cn = cone_of10(d);
                     Ax = cn.x;
                     Ay = cn.y;

@@ -66,14 +66,15 @@ print("TMA bulk copies (`cp.async.bulk`) appear as `UBLKCP`, mbarrier operations
 print("| kernel | regs | stack B | SASS instr | UBLKCP | SYNCS | STL | LDL | STG 32/64/128 | LDG 32/64/128 | LDS | FP64 (DADD+DMUL+DFMA+DSETP) | MUFU | UTC*MMA/HMMA |")
 print("|---|---|---|---|---|---|---|---|---|---|---|---|---|---|")
 for k, c in kern.items():
-    if k.startswith("_ZN8ore_fast") and not any(s in k for s in ("primary_tile_kernelILi8ELb0", "shadow_sweep_kernelILb0ELb1", "shade_setup")):
+    # FAST_LIBM instantiations (last template argument true): only those of the default path are listed
+    if k.startswith("_ZN3ore") and "Lb1EEEv" in k and not any(
+            s in k for s in ("primary_tile_kernelILi8ELb0ELb1", "shadow_sweep_kernelILb0ELb1ELb1", "shade_setup")):
         continue
     r = res.get(k, (0, 0, 0, 0))
-    name = demangle(k).replace("ore::", "").replace("(ore::FrameParams, ore::StageArgs)", "").replace("(ore::FrameParams)", "")
-    name = name.replace("(ore_fast::FrameParams, ore_fast::StageArgs)", "").replace("(ore_fast::FrameParams)", "").replace("void ", "")
+    name = demangle(k).replace("ore::", "").replace("void ", "")
     fp64 = c["DADD"] + c["DMUL"] + c["DFMA"] + c["DSETP"]
     tc = sum(v for kk, v in c.items() if kk.startswith("UTC") or kk in ("HMMA", "LDTM", "STTM"))
     print(f"| `{name}` | {r[0]} | {r[1]} | {c['total']} | {c['UBLKCP']} | {c['SYNCS']} | {c['STL']} | {c['LDL']} | "
           f"{c['STG.32']}/{c['STG.64']}/{c['STG.128']} | {c['LDG.32']}/{c['LDG.64']}/{c['LDG.128']} | {c['LDS']} | {fp64} | {c['MUFU']} | {tc} |")
-print("\n(`ore_fast::*` = the same sources compiled with CUDA's libm for `ORE_FLAG_FAST_LIBM`; only its three render "
-      "kernels are listed.)")
+print("\n(The last template argument of the three render kernels is `FAST_LIBM`: `true` = CUDA's libm for "
+      "`ORE_FLAG_FAST_LIBM`; only the default-path instantiations of it are listed.)")
