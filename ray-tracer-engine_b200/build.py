@@ -16,7 +16,7 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 OBJ_DIR = os.path.join(PKG_DIR, "csrc", "_obj")
 LIB_PATH = os.path.join(PKG_DIR, "libore_b200.so")
 SOURCES = ["ore_capi.cu", "ore_scene_build.cu", "ore_mesh_refit.cu", "ore_mesh_build.cu"]
-HEADERS = ["ore_kernels.cuh", "ore_primary.cuh", "ore_sweep.cuh", "ore_device.cuh", "ore_libm.cuh", "ore_clusters.h", "ore_scene_build.h", "ore_mesh_refit.h", "ore_mesh_build.h", os.path.join("..", "..", "include", "ore_render.h")]
+HEADERS = ["ore_kernels.cuh", "ore_primary.cuh", "ore_sweep.cuh", "ore_device.cuh", "ore_libm.cuh", "ore_clusters.h", "ore_scene_build.h", "ore_mesh_refit.h", "ore_mesh_build.h", "ore_stage_plan.h", os.path.join("..", "..", "include", "ore_render.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

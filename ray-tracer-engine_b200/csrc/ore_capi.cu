@@ -25,7 +25,62 @@
 
 using namespace ore;
 
+namespace {   // (internal linkage: nothing here joins the library's exported symbols)
+
+// Device memory (cudaMalloc) or pinned host memory (cudaMallocHost), as the allocator of a Buf.  slack: the capacity a
+// growing buffer takes for n items, so that reallocations stay rare.
+struct DeviceMem {
+    static cudaError_t alloc(void** p, size_t bytes) { return cudaMalloc(p, bytes); }
+    static cudaError_t free(void* p) { return cudaFree(p); }
+    static size_t slack(size_t n) { return n + n / 8 + 64; }
+};
+struct PinnedMem {
+    static cudaError_t alloc(void** p, size_t bytes) { return cudaMallocHost(p, bytes); }
+    static cudaError_t free(void* p) { return cudaFreeHost(p); }
+    static size_t slack(size_t n) { return n + n / 4 + 4096; }
+};
+
+// A buffer the context owns: the pointer and its capacity in items, freed with the buffer.  Growing never keeps the
+// contents; the caller has waited for whatever may still use the old buffer.
+template <typename T, typename Mem = DeviceMem>
+class Buf {
+public:
+    Buf() = default;
+    Buf(const Buf&) = delete;
+    Buf& operator=(const Buf&) = delete;
+    ~Buf() { release(); }
+    operator T*() const { return p_; }
+    size_t cap() const { return cap_; }
+    bool fits(size_t n) const { return p_ && n <= cap_; }
+    // exactly n items
+    cudaError_t alloc(size_t n) {
+        if (cudaError_t e = release()) return e;
+        const cudaError_t e = Mem::alloc((void**)&p_, n * sizeof(T));
+        if (e == cudaSuccess) cap_ = n;
+        else p_ = nullptr;
+        return e;
+    }
+    // at least n items: unchanged when they fit, else the allocator's slack
+    cudaError_t reserve(size_t n) { return fits(n) ? cudaSuccess : alloc(Mem::slack(n)); }
+    cudaError_t release() {
+        const cudaError_t e = p_ ? Mem::free(p_) : cudaSuccess;
+        p_ = nullptr;
+        cap_ = 0;
+        return e;
+    }
+
+private:
+    T* p_ = nullptr;
+    size_t cap_ = 0;
+};
+template <typename T>
+using DevBuf = Buf<T, DeviceMem>;
+
+}  // namespace
+
 struct ore_context {
+    // (frees every buffer below; not an export of the library)
+    __attribute__((visibility("hidden"))) ~ore_context() = default;
     int device = 0;
     int sm_count = 0;
     cudaStream_t stream = nullptr;
@@ -33,71 +88,62 @@ struct ore_context {
     cudaEvent_t ev_rendered[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
     // device framebuffers of the pipelined presentation: two sets (one being copied out while the other is rendered)
     // of `async_k` frames of `async_px` pixels each, one allocation
-    uint32_t* async_pool = nullptr;
-    size_t async_pool_cap = 0;   // pixels
+    DevBuf<uint32_t> async_pool;
     size_t async_px = 0;
     int async_k = 0;
     unsigned long long async_batches = 0;
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
     bool ev_valid = false;
-    bool ran_count = false;
     std::string err;
 
     // pinned staging (uploads and read-back)
-    void* pinned = nullptr;
-    size_t pinned_cap = 0;
+    Buf<char, PinnedMem> pinned;
 
     // scene (structure of arrays on the device)
     int n_spheres = 0;
-    float4* sph_exact = nullptr;   // cx,cy,cz,radius member in ORIGINAL order (hit attributes by hit id)
+    DevBuf<float4> sph_exact;   // cx,cy,cz,radius member in ORIGINAL order (hit attributes by hit id)
     // the spheres in Morton order with two levels of bounding balls over them (ore_clusters.h)
-    float4* sph_xsort = nullptr;   // exact records, sorted
-    float4* sph_sort = nullptr;    // shadow records cx,cy,cz,R', sorted
-    int* sort_index = nullptr;     // sorted position -> original index
-    float4* leaf_sph = nullptr;    // ball of spheres [8j, 8j+8)
-    float4* super_sph = nullptr;   // ball of leaves [32k, 32k+32)
-    // per-frame (camera-space) records of the primary kernel
-    float4* prim_sorted = nullptr;
-    float4* cone_sorted = nullptr;
-    float4* leaf_cone = nullptr;
-    float4* super_cone = nullptr;
+    DevBuf<float4> sph_xsort;   // exact records, sorted
+    DevBuf<float4> sph_sort;    // shadow records cx,cy,cz,R', sorted
+    DevBuf<int> sort_index;     // sorted position -> original index
+    DevBuf<float4> leaf_sph;    // ball of spheres [8j, 8j+8)
+    DevBuf<float4> super_sph;   // ball of leaves [32k, 32k+32)
+    // per-frame (camera-space) records of the primary kernel, one set per frame of a batch
+    DevBuf<float4> prim_sorted;
+    DevBuf<float4> cone_sorted;
+    DevBuf<float4> leaf_cone;
+    DevBuf<float4> super_cone;
     int n_sort = 0, n_leaves = 0, n_leaves_pad = 0, n_supers = 0, n_supers_pad = 0;
-    size_t sph_cap = 0, sort_cap = 0, leaf_cap = 0, super_cap = 0;
     // work space of the device build of the hierarchy (ore_scene_build.cu), sized with the scene buffers
-    uint32_t* keys_in = nullptr;
-    uint32_t* keys_out = nullptr;
-    int* vals_in = nullptr;
-    int* vals_out = nullptr;
-    size_t key_cap = 0;
-    uint32_t* bbox = nullptr;
-    void* sort_tmp = nullptr;
-    size_t sort_tmp_cap = 0;   // bytes
+    DevBuf<uint32_t> keys_in;
+    DevBuf<uint32_t> keys_out;
+    DevBuf<int> vals_in;
+    DevBuf<int> vals_out;
+    DevBuf<uint32_t> bbox;
+    DevBuf<char> sort_tmp;
     int n_lights = 0;
     LightP lights[MAX_LIGHTS];
-    float* tex[3] = {nullptr, nullptr, nullptr};
+    DevBuf<float> tex[3];
     int tex_w = 0, tex_h = 0;
     bool tex_finite = false;   // every texel of the object texture is finite (checked at upload; FrameParams::skip_dark)
-    float* sky[3] = {nullptr, nullptr, nullptr};
+    DevBuf<float> sky[3];
     int sky_w = 0, sky_h = 0;
     float sky_radius = 0.f;
-    float4* cubes = nullptr;   // 3 float4 per cube: bounds[0], bounds[1], orgin
-    float4* planes = nullptr;  // 2 float4 per plane: orgin, normal
+    DevBuf<float4> cubes;    // 3 float4 per cube: bounds[0], bounds[1], orgin
+    DevBuf<float4> planes;   // 2 float4 per plane: orgin, normal
     int n_cubes = 0, n_planes = 0;
-    float* tris = nullptr;     // 27 floats per triangle
-    float4* boxes = nullptr;   // 2 float4 per leaf box
-    float4* box_sph = nullptr; // bounding sphere per leaf box (cone filters)
-    float4* box_cone = nullptr;  // per-frame tile-cone record per leaf box
-    int* box_offsets = nullptr;
-    int* box_indices = nullptr;
+    // the mesh buffers, sized for the largest mesh uploaded by either setter since the mesh was last removed
+    DevBuf<float> tris;         // 27 floats per triangle
+    DevBuf<float4> boxes;       // 2 float4 per leaf box
+    DevBuf<float4> box_sph;     // bounding sphere per leaf box (cone filters)
+    DevBuf<float4> box_cone;    // per-frame tile-cone record per leaf box
+    DevBuf<int> box_offsets;
+    DevBuf<int> box_indices;
     // n_boxes: the leaf capacity (stride of box_cone, grid sizes); the live leaf count is *mesh_live on the device (the
     // render kernels' leaf loops end there; leaves past it list no triangles)
     int n_tris = 0, n_boxes = 0, mesh_has_normals = 0, mesh_n_idx = 0;
-    int* mesh_live = nullptr;
-    // capacities of the mesh buffers (triangles, leaves, listed indices) and the device build's work space: the largest
-    // mesh uploaded by either setter since the mesh was last removed
-    size_t mesh_tri_cap = 0, mesh_box_cap = 0, mesh_idx_cap = 0;
-    void* mesh_work = nullptr;
-    size_t mesh_work_bytes = 0;
+    DevBuf<int> mesh_live;
+    DevBuf<char> mesh_work;   // the device build's work space
     // the device build's launch sequence (about 65 launches, all sized from the capacity; the triangle count is read on
     // the device) captured once per buffer set and replayed on the caller's stream: enqueuing it launch by launch costs
     // the host several hundred microseconds
@@ -105,36 +151,29 @@ struct ore_context {
     cudaStream_t mesh_capture = nullptr;
 
     // per-frame buffers
-    float* dx_tab = nullptr;
-    size_t dx_cap = 0;
-    float* dy_tab = nullptr;
-    size_t dy_cap = 0;
-    uint32_t* hit_list = nullptr;  // compact hit records (pixel, id, t), one per hit pixel
-    int32_t* hit_ids = nullptr;
-    float* hit_ts = nullptr;
-    uint32_t* pixels = nullptr;    // the context's own framebuffer (ore_render)
-    size_t px_cap = 0, pixels_cap = 0;
-    int32_t* hit_id_map = nullptr;  // per-pixel id / t maps: only built by ore_get_hits
-    float* hit_t_map = nullptr;
-    size_t map_cap = 0;
-    unsigned long long* counters = nullptr;
+    DevBuf<float> dx_tab;
+    DevBuf<float> dy_tab;
+    DevBuf<uint32_t> hit_list;  // compact hit records (pixel, id, t), one per hit pixel
+    DevBuf<int32_t> hit_ids;
+    DevBuf<float> hit_ts;
+    DevBuf<uint32_t> pixels;    // the context's own framebuffer (ore_render)
+    DevBuf<int32_t> hit_id_map;  // per-pixel id / t maps: only built by ore_get_hits
+    DevBuf<float> hit_t_map;
+    DevBuf<unsigned long long> counters;
     // band DMA (ORE_FLAG_BAND_DMA): packed local rows of the primary kernel + the stream / events of their copy
-    uint32_t* band_buf = nullptr;
-    size_t band_cap = 0;   // pixels
+    DevBuf<uint32_t> band_buf;
     cudaStream_t band_stream = nullptr;
     cudaEvent_t ev_band_go = nullptr, ev_band_done = nullptr;
-    float* stage = nullptr;  // staging buffer between the two kernels of the default shadow pass
-    size_t stage_cap = 0;    // floats
+    DevBuf<float> stage;  // staging buffer between the two kernels of the default shadow pass (ore_stage_plan.h)
     size_t stage_blocks_override = 0;  // test hook (env ORE_STAGE_BLOCKS at ore_create): staging capacity in 32-item blocks
     size_t stage_max_items = (size_t)8 << 20;  // env ORE_STAGE_MAX_ITEMS: upper bound of the staging buffer in hit pixels
     bool no_memops = false;            // test hook (env ORE_NO_STREAM_MEMOPS=1): flags through the one-thread kernels
     std::string dbg_cycles_path;       // tools hook (env ORE_DEBUG_BLOCK_CYCLES=file): per-block SM clocks of the shadow pass
-    uint32_t* dbg_cycles = nullptr;
-    size_t dbg_cap = 0;
+    DevBuf<uint32_t> dbg_cycles;       // [2][cap / 2]
     // hit count of this context's previous frame, copied to pinned memory at the end of every frame and read
     // WITHOUT synchronisation by the next one: only a hint for how many staged chunk pairs to launch - whatever
     // lies beyond them is swept by one catch-all fused launch, so any value (stale, zero, mid-copy) is safe
-    unsigned long long* hits_hint = nullptr;
+    Buf<unsigned long long, PinnedMem> hits_hint;
     bool hits_hint_set = false;
     FrameParams last_prm;              // the last frame's parameters (ore_get_hits expands its hit records)
     bool last_prm_valid = false;
@@ -183,40 +222,16 @@ static int fail(ore_context* ctx, int code, const char* msg) {
     return code;
 }
 
-static int ensure_pinned(ore_context* ctx, size_t bytes) {
-    if (bytes <= ctx->pinned_cap) return ORE_OK;
-    if (ctx->pinned) ORE_CUDA(ctx, cudaFreeHost(ctx->pinned));
-    ctx->pinned = nullptr;
-    ctx->pinned_cap = 0;
-    size_t cap = bytes + bytes / 4 + 4096;
-    ORE_CUDA(ctx, cudaMallocHost(&ctx->pinned, cap));
-    ctx->pinned_cap = cap;
-    return ORE_OK;
-}
-
-template <typename T>
-static int ensure_dev(ore_context* ctx, T** p, size_t* cap, size_t n) {
-    if (n <= *cap && *p) return ORE_OK;
-    if (*p) ORE_CUDA(ctx, cudaFree(*p));
-    *p = nullptr;
-    *cap = 0;
-    size_t want = n + n / 8 + 64;
-    ORE_CUDA(ctx, cudaMalloc((void**)p, want * sizeof(T)));
-    *cap = want;
-    return ORE_OK;
-}
-
-// Replaces the device buffer *p by n items that fill(T* staging) writes into the pinned staging buffer, and waits for
+// Replaces the device buffer by n items that fill(T* staging) writes into the pinned staging buffer, and waits for
 // the copy.  n == 0 leaves no buffer and does not synchronise.  The caller has waited for the last render.
 template <typename T, typename Fill>
-static int replace_buffer(ore_context* ctx, T** p, size_t n, Fill fill) {
-    if (*p) ORE_CUDA(ctx, cudaFree(*p));
-    *p = nullptr;
+static int replace_buffer(ore_context* ctx, DevBuf<T>& buf, size_t n, Fill fill) {
+    ORE_CUDA(ctx, buf.release());
     if (n == 0) return ORE_OK;
-    if (int rc = ensure_pinned(ctx, n * sizeof(T))) return rc;
-    fill((T*)ctx->pinned);
-    ORE_CUDA(ctx, cudaMalloc((void**)p, n * sizeof(T)));
-    ORE_CUDA(ctx, cudaMemcpyAsync(*p, ctx->pinned, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+    ORE_CUDA(ctx, ctx->pinned.reserve(n * sizeof(T)));
+    fill((T*)(void*)ctx->pinned);
+    ORE_CUDA(ctx, buf.alloc(n));
+    ORE_CUDA(ctx, cudaMemcpyAsync(buf, ctx->pinned, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
     ORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return ORE_OK;
 }
@@ -238,6 +253,16 @@ static int scene_idle(ore_context* ctx) {
     return ORE_OK;
 }
 
+// Growth of a buffer a frame reads or writes: an earlier frame may still be running on another stream, so the host waits
+// for the last render before the buffer is re-allocated.
+template <typename T>
+static int frame_reserve(ore_context* ctx, DevBuf<T>& buf, size_t n) {
+    if (buf.fits(n)) return ORE_OK;
+    if (int rc = wait_last_render(ctx)) return rc;
+    ORE_CUDA(ctx, buf.reserve(n));
+    return ORE_OK;
+}
+
 // A stream-ordered update runs on `stream` (NULL: the render stream) after every render submitted so far and the
 // previous update, on whatever streams they ran; the host never waits.  update_end marks its end for every render and
 // setter submitted later.
@@ -253,8 +278,6 @@ static int update_end(ore_context* ctx, cudaStream_t st) {
     ctx->ev_scene_set = true;
     return ORE_OK;
 }
-
-static int mesh_alloc(ore_context* ctx, size_t tri_cap, size_t box_cap, size_t idx_cap);
 
 extern "C" int ore_abi_version(void) { return ORE_ABI_VERSION; }
 
@@ -286,7 +309,7 @@ extern "C" int ore_create(ore_context** out, int device) {
     for (int i = 0; i < 5; i++) ORE_CUDA(ctx, cudaEventCreate(&ctx->ev[i]));
     ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_done, cudaEventDisableTiming));
     ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_scene, cudaEventDisableTiming));
-    ORE_CUDA(ctx, cudaMallocHost((void**)&ctx->hits_hint, sizeof(unsigned long long)));
+    ORE_CUDA(ctx, ctx->hits_hint.alloc(1));
     *ctx->hits_hint = 0;
     if (const char* e = getenv("ORE_NO_STREAM_MEMOPS")) ctx->no_memops = atoi(e) != 0;
     if (const char* e = getenv("ORE_STAGE_MAX_ITEMS")) {
@@ -298,7 +321,7 @@ extern "C" int ore_create(ore_context** out, int device) {
         const long v = atol(e);
         if (v > 0) ctx->stage_blocks_override = (size_t)v;
     }
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->counters, CNT_SLOTS * sizeof(unsigned long long)));
+    ORE_CUDA(ctx, ctx->counters.alloc(CNT_SLOTS));
     ORE_CUDA(ctx, cudaMemset(ctx->counters, 0, CNT_SLOTS * sizeof(unsigned long long)));
     // kernel.cu:1454,1462-1463: phi = (float)j/10 * 2.f * 3.1415f; cosf(phi), sinf(phi)
     float cphi[10], sphi[10];
@@ -327,18 +350,17 @@ extern "C" int ore_destroy(ore_context* ctx) {
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     if (ctx->dbg_cycles) {
-        // tools hook: [2][dbg_cap] uint32 of the LAST frame, preceded by dbg_cap as one uint64
+        // tools hook: [2][cap] uint32 of the LAST frame, preceded by cap as one uint64
         cudaDeviceSynchronize();
-        std::vector<uint32_t> h(2 * ctx->dbg_cap);
+        std::vector<uint32_t> h(ctx->dbg_cycles.cap());
         if (cudaMemcpy(h.data(), ctx->dbg_cycles, h.size() * 4, cudaMemcpyDeviceToHost) == cudaSuccess) {
             if (FILE* f = fopen(ctx->dbg_cycles_path.c_str(), "wb")) {
-                const unsigned long long cap = ctx->dbg_cap;
+                const unsigned long long cap = h.size() / 2;
                 fwrite(&cap, 8, 1, f);
                 fwrite(h.data(), 4, h.size(), f);
                 fclose(f);
             }
         }
-        cudaFree(ctx->dbg_cycles);
     }
     if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
     for (int i = 0; i < 2; i++) {
@@ -348,7 +370,7 @@ extern "C" int ore_destroy(ore_context* ctx) {
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->ev_done) cudaEventDestroy(ctx->ev_done);
     if (ctx->ev_scene) cudaEventDestroy(ctx->ev_scene);
-    mesh_alloc(ctx, 0, 0, 0);   // (the mesh buffers and the build's graph)
+    if (ctx->mesh_graph) cudaGraphExecDestroy(ctx->mesh_graph);
     if (ctx->mesh_capture) cudaStreamDestroy(ctx->mesh_capture);
     if (ctx->signal_stream) {
         cudaStreamSynchronize(ctx->signal_stream);
@@ -362,20 +384,10 @@ extern "C" int ore_destroy(ore_context* ctx) {
         cudaEventDestroy(ctx->ev_band_done);
         cudaStreamDestroy(ctx->band_stream);
     }
-    if (ctx->async_pool) cudaFree(ctx->async_pool);
-    void* dev[] = {ctx->band_buf, ctx->stage, ctx->sph_exact, ctx->sph_xsort, ctx->sph_sort, ctx->sort_index, ctx->leaf_sph, ctx->super_sph,
-                   ctx->prim_sorted, ctx->cone_sorted, ctx->leaf_cone, ctx->super_cone, ctx->tex[0], ctx->tex[1], ctx->tex[2],
-                   ctx->sky[0], ctx->sky[1], ctx->sky[2], ctx->dx_tab, ctx->dy_tab, ctx->hit_list, ctx->hit_ids, ctx->hit_ts,
-                   ctx->hit_id_map, ctx->hit_t_map, ctx->pixels, ctx->counters, ctx->cubes, ctx->planes, ctx->mesh_live,
-                   ctx->keys_in, ctx->keys_out, ctx->vals_in, ctx->vals_out, ctx->bbox, ctx->sort_tmp};
-    for (void* p : dev)
-        if (p) cudaFree(p);
-    if (ctx->pinned) cudaFreeHost(ctx->pinned);
-    if (ctx->hits_hint) cudaFreeHost(ctx->hits_hint);
     for (int i = 0; i < 5; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;   // (and with it every buffer the context owns)
     return ORE_OK;
 }
 
@@ -404,52 +416,23 @@ static int scene_reserve(ore_context* ctx, int32_t n) {
     scene_sizes(n, &n_sort, &n_leaf_pad, &n_sup_pad);
     size_t tmp_bytes = 0;
     ORE_CUDA(ctx, ore_scene_sort_bytes(n, &tmp_bytes));
-    const size_t n_ex = (size_t)std::max(n, 1);
-    if (ctx->sph_exact && ctx->keys_in && ctx->bbox && ctx->sort_tmp && n_ex <= ctx->sph_cap && n_sort <= ctx->sort_cap &&
-        n_leaf_pad <= ctx->leaf_cap && n_sup_pad <= ctx->super_cap && (size_t)n <= ctx->key_cap && tmp_bytes <= ctx->sort_tmp_cap)
-        return ORE_OK;
-    int rc;
-    if ((rc = scene_idle(ctx))) return rc;
-    size_t c0 = ctx->sph_cap;
-    if ((rc = ensure_dev(ctx, &ctx->sph_exact, &c0, n_ex))) return rc;
-    ctx->sph_cap = c0;
-    size_t c1 = ctx->sort_cap, c2 = c1, c3 = c1, c4 = c1, c5 = c1;
-    if ((rc = ensure_dev(ctx, &ctx->sph_xsort, &c1, n_sort))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->sph_sort, &c2, n_sort))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->sort_index, &c3, n_sort))) return rc;
-    // camera-space records: one set per frame of a batch
-    c4 *= MAX_BATCH;
-    c5 *= MAX_BATCH;
-    if ((rc = ensure_dev(ctx, &ctx->prim_sorted, &c4, n_sort * MAX_BATCH))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->cone_sorted, &c5, n_sort * MAX_BATCH))) return rc;
-    ctx->sort_cap = std::min(std::min(c1, c2), std::min(std::min(c3, c4 / MAX_BATCH), c5 / MAX_BATCH));
-    size_t l1 = ctx->leaf_cap, l2 = l1;
-    if ((rc = ensure_dev(ctx, &ctx->leaf_sph, &l1, n_leaf_pad))) return rc;
-    l2 *= MAX_BATCH;
-    if ((rc = ensure_dev(ctx, &ctx->leaf_cone, &l2, n_leaf_pad * MAX_BATCH))) return rc;
-    ctx->leaf_cap = std::min(l1, l2 / MAX_BATCH);
-    size_t s1 = ctx->super_cap, s2 = s1;
-    if ((rc = ensure_dev(ctx, &ctx->super_sph, &s1, n_sup_pad))) return rc;
-    s2 *= MAX_BATCH;
-    if ((rc = ensure_dev(ctx, &ctx->super_cone, &s2, n_sup_pad * MAX_BATCH))) return rc;
-    ctx->super_cap = std::min(s1, s2 / MAX_BATCH);
-    size_t k1 = ctx->key_cap, k2 = k1, k3 = k1, k4 = k1;
-    if ((rc = ensure_dev(ctx, &ctx->keys_in, &k1, (size_t)n))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->keys_out, &k2, (size_t)n))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->vals_in, &k3, (size_t)n))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->vals_out, &k4, (size_t)n))) return rc;
-    ctx->key_cap = std::min(std::min(k1, k2), std::min(k3, k4));
-    if (!ctx->bbox) ORE_CUDA(ctx, cudaMalloc((void**)&ctx->bbox, 6 * sizeof(uint32_t)));
+    const size_t n_ex = (size_t)std::max(n, 1), nb = MAX_BATCH;   // (camera-space records: one set per frame of a batch)
+    // op(buffer, items it needs) over every buffer of the scene, until one returns false
+    const auto each = [&](auto&& op) {
+        return op(ctx->sph_exact, n_ex) && op(ctx->sph_xsort, n_sort) && op(ctx->sph_sort, n_sort) && op(ctx->sort_index, n_sort) &&
+               op(ctx->prim_sorted, n_sort * nb) && op(ctx->cone_sorted, n_sort * nb) && op(ctx->leaf_sph, n_leaf_pad) &&
+               op(ctx->leaf_cone, n_leaf_pad * nb) && op(ctx->super_sph, n_sup_pad) && op(ctx->super_cone, n_sup_pad * nb) &&
+               op(ctx->keys_in, (size_t)n) && op(ctx->keys_out, (size_t)n) && op(ctx->vals_in, (size_t)n) &&
+               op(ctx->vals_out, (size_t)n) && op(ctx->bbox, (size_t)6);
+    };
+    if (each([](auto& buf, size_t k) { return buf.fits(k); }) && ctx->sort_tmp.fits(tmp_bytes)) return ORE_OK;
+    if (int rc = scene_idle(ctx)) return rc;
+    cudaError_t e = cudaSuccess;
+    each([&](auto& buf, size_t k) { return (e = buf.reserve(k)) == cudaSuccess; });
+    ORE_CUDA(ctx, e);
     // sort work space for the whole key capacity, so that any n up to it needs no more
-    ORE_CUDA(ctx, ore_scene_sort_bytes((int)std::min(ctx->key_cap, (size_t)INT32_MAX), &tmp_bytes));
-    if (tmp_bytes > ctx->sort_tmp_cap || !ctx->sort_tmp) {
-        if (ctx->sort_tmp) ORE_CUDA(ctx, cudaFree(ctx->sort_tmp));
-        ctx->sort_tmp = nullptr;
-        ctx->sort_tmp_cap = 0;
-        tmp_bytes = std::max(tmp_bytes, (size_t)256);   // (never a null work space: it marks "not sized yet")
-        ORE_CUDA(ctx, cudaMalloc(&ctx->sort_tmp, tmp_bytes));
-        ctx->sort_tmp_cap = tmp_bytes;
-    }
+    ORE_CUDA(ctx, ore_scene_sort_bytes((int)std::min(ctx->keys_in.cap(), (size_t)INT32_MAX), &tmp_bytes));
+    if (!ctx->sort_tmp.fits(tmp_bytes)) ORE_CUDA(ctx, ctx->sort_tmp.alloc(std::max(tmp_bytes, (size_t)256)));
     return ORE_OK;
 }
 
@@ -478,7 +461,7 @@ static int scene_enqueue(ore_context* ctx, const float4* src, int32_t n, cudaStr
     a.vals_out = ctx->vals_out;
     a.bbox = ctx->bbox;
     a.sort_tmp = ctx->sort_tmp;
-    a.sort_tmp_bytes = ctx->sort_tmp_cap;
+    a.sort_tmp_bytes = ctx->sort_tmp.cap();
     ORE_CUDA(ctx, ore_scene_build(a, stream));
     ctx->n_spheres = n;
     ctx->n_sort = a.n_sort;
@@ -498,8 +481,8 @@ static int upload_spheres(ore_context* ctx, const float* src, size_t stride_floa
     if ((rc = scene_idle(ctx))) return rc;
     if ((rc = scene_reserve(ctx, n))) return rc;
     if (n > 0) {
-        if ((rc = ensure_pinned(ctx, (size_t)n * sizeof(float4)))) return rc;
-        float4* h = (float4*)ctx->pinned;
+        ORE_CUDA(ctx, ctx->pinned.reserve((size_t)n * sizeof(float4)));
+        float4* h = (float4*)(void*)ctx->pinned;
         for (int i = 0; i < n; i++) {
             const float* s = src + (size_t)i * stride_floats + first;
             h[i] = make_float4(s[0], s[1], s[2], s[3]);
@@ -572,7 +555,7 @@ extern "C" int ore_set_cubes(ore_context* ctx, const float* c1_c2, int32_t n) {
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
     if (int rcw = wait_last_render(ctx)) return rcw;
     ctx->n_cubes = 0;
-    int rc = replace_buffer(ctx, &ctx->cubes, (size_t)n * 3, [&](float4* h) {
+    int rc = replace_buffer(ctx, ctx->cubes, (size_t)n * 3, [&](float4* h) {
         for (int i = 0; i < n; i++) {
             const float* c = c1_c2 + 6 * (size_t)i;
             h[3 * i + 0] = make_float4(c[0], c[1], c[2], 0.f);  // bounds[0] = c1, kernel.cu:393
@@ -597,7 +580,7 @@ extern "C" int ore_set_planes(ore_context* ctx, const float* pos_normal, int32_t
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
     if (int rcw = wait_last_render(ctx)) return rcw;
     ctx->n_planes = 0;
-    int rc = replace_buffer(ctx, &ctx->planes, (size_t)n * 2, [&](float4* h) {
+    int rc = replace_buffer(ctx, ctx->planes, (size_t)n * 2, [&](float4* h) {
         for (int i = 0; i < n; i++) {
             const float* c = pos_normal + 6 * (size_t)i;
             h[2 * i + 0] = make_float4(c[0], c[1], c[2], 0.f);
@@ -610,36 +593,37 @@ extern "C" int ore_set_planes(ore_context* ctx, const float* pos_normal, int32_t
 }
 
 // Frees the mesh buffers and, unless tri_cap is 0, allocates them for tri_cap triangles, box_cap leaves and idx_cap
-// listed indices, with the device build's work space for tri_cap triangles (tri_cap <= INT32_MAX / TRI_FLOATS: the setters
-// check).  The caller has waited for every render and update that may use them.
+// (>= 1) listed indices, with the device build's work space for tri_cap triangles (tri_cap <= INT32_MAX / TRI_FLOATS: the
+// setters check).  The caller has waited for every render and update that may use them.
 static int mesh_alloc(ore_context* ctx, size_t tri_cap, size_t box_cap, size_t idx_cap) {
     if (ctx->mesh_graph) ORE_CUDA(ctx, cudaGraphExecDestroy(ctx->mesh_graph));   // (it holds the old buffers' addresses)
     ctx->mesh_graph = nullptr;
-    void** bufs[] = {(void**)&ctx->tris, (void**)&ctx->boxes, (void**)&ctx->box_offsets, (void**)&ctx->box_indices,
-                     (void**)&ctx->box_sph, (void**)&ctx->box_cone, &ctx->mesh_work};
-    for (void** p : bufs) {
-        if (*p) ORE_CUDA(ctx, cudaFree(*p));
-        *p = nullptr;
-    }
-    ctx->mesh_tri_cap = ctx->mesh_box_cap = ctx->mesh_idx_cap = ctx->mesh_work_bytes = 0;
+    for (cudaError_t e : {ctx->tris.release(), ctx->boxes.release(), ctx->box_offsets.release(), ctx->box_indices.release(),
+                          ctx->box_sph.release(), ctx->box_cone.release(), ctx->mesh_work.release()})
+        ORE_CUDA(ctx, e);
     ctx->n_tris = ctx->n_boxes = ctx->mesh_has_normals = ctx->mesh_n_idx = 0;
     if (tri_cap == 0) return ORE_OK;
     size_t work = 0;
     ORE_CUDA(ctx, ore_mesh_build_bytes((int)tri_cap, &work));
-    if (!ctx->mesh_live) ORE_CUDA(ctx, cudaMalloc((void**)&ctx->mesh_live, sizeof(int)));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->tris, tri_cap * ore_host::TRI_FLOATS * sizeof(float)));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->boxes, box_cap * 2 * sizeof(float4)));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_offsets, (box_cap + 1) * sizeof(int)));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_indices, std::max(idx_cap, (size_t)1) * sizeof(int)));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_sph, box_cap * sizeof(float4)));
-    ORE_CUDA(ctx, cudaMalloc((void**)&ctx->box_cone, box_cap * sizeof(float4) * MAX_BATCH));
-    ORE_CUDA(ctx, cudaMalloc(&ctx->mesh_work, work));
-    ctx->mesh_tri_cap = tri_cap;
-    ctx->mesh_box_cap = box_cap;
-    ctx->mesh_idx_cap = idx_cap;
-    ctx->mesh_work_bytes = work;
+    if (!ctx->mesh_live) ORE_CUDA(ctx, ctx->mesh_live.alloc(1));
+    ORE_CUDA(ctx, ctx->tris.alloc(tri_cap * ore_host::TRI_FLOATS));
+    ORE_CUDA(ctx, ctx->boxes.alloc(box_cap * 2));
+    ORE_CUDA(ctx, ctx->box_offsets.alloc(box_cap + 1));
+    ORE_CUDA(ctx, ctx->box_indices.alloc(idx_cap));
+    ORE_CUDA(ctx, ctx->box_sph.alloc(box_cap));
+    ORE_CUDA(ctx, ctx->box_cone.alloc(box_cap * MAX_BATCH));
+    ORE_CUDA(ctx, ctx->mesh_work.alloc(work));
     return ORE_OK;
 }
+
+// the mesh buffers hold n_tris triangles, n_boxes leaves and n_idx listed indices
+static bool mesh_fits(const ore_context* ctx, size_t n_tris, size_t n_boxes, size_t n_idx) {
+    return ctx->tris.fits(n_tris * ore_host::TRI_FLOATS) && ctx->boxes.fits(n_boxes * 2) && ctx->box_offsets.fits(n_boxes + 1) &&
+           ctx->box_indices.fits(n_idx) && ctx->box_sph.fits(n_boxes) && ctx->box_cone.fits(n_boxes * MAX_BATCH);
+}
+
+// capacity of the mesh buffers in triangles (0 without a mesh)
+static size_t mesh_tri_cap(const ore_context* ctx) { return ctx->tris.cap() / ore_host::TRI_FLOATS; }
 
 extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tris, int32_t has_normals,
                             const float* box_bounds6, const int32_t* box_offsets, const int32_t* box_indices,
@@ -664,17 +648,17 @@ extern "C" int ore_set_mesh(ore_context* ctx, const float* tris27, int32_t n_tri
     if ((rc = scene_idle(ctx))) return rc;
     if (remove) return mesh_alloc(ctx, 0, 0, 0);
     // the buffers are re-allocated at least at the capacity the device setters reached, so that they keep not blocking
-    const size_t tri_cap = std::max(ctx->mesh_tri_cap, (size_t)n_tris);
-    const size_t box_cap = std::max(std::max(ctx->mesh_box_cap, (size_t)n_boxes), (size_t)ore_mesh_leaf_capacity((int)tri_cap));
-    const size_t idx_cap = std::max(std::max(ctx->mesh_idx_cap, (size_t)n_idx), tri_cap);
+    const size_t tri_cap = std::max(mesh_tri_cap(ctx), (size_t)n_tris);
+    const size_t box_cap = std::max({ctx->box_sph.cap(), (size_t)n_boxes, (size_t)ore_mesh_leaf_capacity((int)tri_cap)});
+    const size_t idx_cap = std::max({ctx->box_indices.cap(), (size_t)n_idx, tri_cap});
     if ((rc = mesh_alloc(ctx, tri_cap, box_cap, idx_cap))) return rc;
     const size_t tb = (size_t)n_tris * 27 * sizeof(float), bb = (size_t)n_boxes * 2 * sizeof(float4);
     const size_t ob = (size_t)(n_boxes + 1) * sizeof(int), ib = (size_t)(n_idx > 0 ? n_idx : 1) * sizeof(int);
     // pinned staging layout: the float4 section first (16-byte aligned: bb is a multiple of 16 and the pinned base is
     // page aligned), then the 4-byte-aligned sections, the live leaf count last
     const size_t off_b = 0, off_t = bb, off_o = off_t + tb, off_i = off_o + ob, off_l = off_i + ib;
-    if ((rc = ensure_pinned(ctx, off_l + sizeof(int)))) return rc;
-    char* h = (char*)ctx->pinned;
+    ORE_CUDA(ctx, ctx->pinned.reserve(off_l + sizeof(int)));
+    char* h = ctx->pinned;
     float4* hb = (float4*)(h + off_b);
     memcpy(h + off_t, tris27, tb);
     for (int j = 0; j < n_boxes; j++) {
@@ -709,11 +693,11 @@ extern "C" int ore_set_mesh_device(ore_context* ctx, const float* tris27_dev, in
     int rc;
     if ((rc = device_records(ctx, tris27_dev, 4, "ore_set_mesh_device: the triangles"))) return rc;
     const int L = ore_mesh_leaf_capacity(n_tris);
-    if (!ctx->tris || (size_t)n_tris > ctx->mesh_tri_cap || (size_t)L > ctx->mesh_box_cap || (size_t)n_tris > ctx->mesh_idx_cap) {
+    if (!mesh_fits(ctx, n_tris, L, n_tris)) {
         // growth: the old buffers may still be read by a render or written by an update on another stream
         if ((rc = scene_idle(ctx))) return rc;
-        const size_t tri_cap = std::max(ctx->mesh_tri_cap, (size_t)n_tris);
-        if ((rc = mesh_alloc(ctx, tri_cap, std::max(ctx->mesh_box_cap, (size_t)L), std::max(ctx->mesh_idx_cap, tri_cap)))) return rc;
+        const size_t tri_cap = std::max(mesh_tri_cap(ctx), (size_t)n_tris);
+        if ((rc = mesh_alloc(ctx, tri_cap, std::max(ctx->box_sph.cap(), (size_t)L), std::max(ctx->box_indices.cap(), tri_cap)))) return rc;
     }
     cudaStream_t st;
     if ((rc = update_begin(ctx, stream, &st))) return rc;
@@ -721,14 +705,14 @@ extern "C" int ore_set_mesh_device(ore_context* ctx, const float* tris27_dev, in
                                   cudaMemcpyDeviceToDevice, st));
     MeshBuildArgs a;
     a.tris = ctx->tris;
-    a.cap_tris = (int)ctx->mesh_tri_cap;
+    a.cap_tris = (int)mesh_tri_cap(ctx);
     a.box_offsets = ctx->box_offsets;
     a.box_indices = ctx->box_indices;
     a.boxes = ctx->boxes;
     a.box_sph = ctx->box_sph;
     a.n_live = ctx->mesh_live;
     a.work = ctx->mesh_work;
-    a.work_bytes = ctx->mesh_work_bytes;
+    a.work_bytes = ctx->mesh_work.cap();
     if (!ctx->mesh_graph) {   // (mesh_alloc drops it with the buffers it holds)
         if (!ctx->mesh_capture) ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->mesh_capture, cudaStreamNonBlocking));
         cudaGraph_t g = nullptr;
@@ -783,7 +767,7 @@ extern "C" int ore_set_lights(ore_context* ctx, const float* lights7, int32_t n)
     return ORE_OK;
 }
 
-static int upload_planes(ore_context* ctx, float* dst[3], const float* r, const float* g, const float* b, int32_t w,
+static int upload_planes(ore_context* ctx, DevBuf<float>* dst, const float* r, const float* g, const float* b, int32_t w,
                          int32_t h) {
     if (!ctx || w <= 0 || h <= 0 || !r || !g || !b) return fail(ctx, ORE_ERR_INVALID, "sprite planes: bad arguments");
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -791,7 +775,7 @@ static int upload_planes(ore_context* ctx, float* dst[3], const float* r, const 
     const size_t n = (size_t)w * h;
     const float* src[3] = {r, g, b};
     for (int c = 0; c < 3; c++)
-        if (int rc = replace_buffer(ctx, &dst[c], n, [&](float* p) { memcpy(p, src[c], n * sizeof(float)); })) return rc;
+        if (int rc = replace_buffer(ctx, dst[c], n, [&](float* p) { memcpy(p, src[c], n * sizeof(float)); })) return rc;
     return ORE_OK;
 }
 
@@ -888,6 +872,266 @@ static int launch_sweep(ore_context* ctx, const FrameParams& prm, const StageArg
     return ORE_OK;
 }
 
+// Copies n_rows rows of W pixels that lie in blocks of B rows, S image rows apart, at dst, from src where they are packed:
+// one strided copy of the full blocks, then one of the ragged tail.
+static int copy_row_blocks(ore_context* ctx, uint32_t* dst, const uint32_t* src, size_t W, int n_rows, int B, int S,
+                           cudaMemcpyKind kind, cudaStream_t stream) {
+    const size_t full = (size_t)(n_rows / B), rem = (size_t)(n_rows % B), row_bytes = W * sizeof(uint32_t);
+    if (full)
+        ORE_CUDA(ctx, cudaMemcpy2DAsync(dst, (size_t)S * row_bytes, src, (size_t)B * row_bytes, (size_t)B * row_bytes, full, kind,
+                                        stream));
+    if (rem) ORE_CUDA(ctx, cudaMemcpyAsync(dst + full * S * W, src + full * B * W, rem * row_bytes, kind, stream));
+    return ORE_OK;
+}
+
+struct TileCone {
+    float px_delta, ca, sa;   // FrameParams::px_delta, tile_ca, tile_sa
+};
+
+// Largest half-angle of a 32 x TILE_ROWS pixel tile seen from the eye (tile cone of the primary kernel), for rendered rows
+// in blocks of y_block, y_step image rows apart: |v_pixel - v_centre| <= halfdiag on the image plane and |v| >= fz, so
+// sin(a) <= halfdiag/fz.
+static TileCone tile_cone(float aspect, int W, int y_block, int y_step, float fz) {
+    const double delta = 2.0 * (double)aspect / (double)W;
+    // tallest image-row span of TILE_ROWS consecutive RENDERED rows
+    int max_span = 0;
+    for (int k0 = 0; k0 < y_block * TILE_ROWS; k0 += TILE_ROWS) {
+        const int k1 = k0 + TILE_ROWS - 1;
+        const int sp = ((k1 / y_block) * y_step + k1 % y_block) - ((k0 / y_block) * y_step + k0 % y_block);
+        if (sp > max_span) max_span = sp;
+    }
+    const double hx = 16.0 * delta, hy = (0.5 * max_span + 0.5) * delta;
+    const double xr = sqrt(hx * hx + hy * hy) / fabs((double)fz);
+    if (!(xr < 0.9)) return {(float)delta, -1e20f, 0.f};   // tiles too wide for a cone: every sphere is a candidate
+    const double a = asin(xr) * 1.001 + 1e-6;
+    return {(float)delta, (float)(cos(a) * (1.0 - 1e-6) - 1e-6), (float)(sin(a) * (1.0 + 1e-6) + 1e-6)};
+}
+
+// The kernel parameters of a launch set: frame geometry and cameras, outputs (outs: the caller's framebuffers, null: the
+// context's own), the context's scene, per-frame buffers (sized by the caller) and lights.  band_dma: the primary kernel
+// writes its rows to band_buf.  *psmem: dynamic shared memory of the primary kernel.
+static FrameParams frame_params(const ore_context* ctx, const ore_camera* cams, int n_frames, const ore_frame* fr,
+                                uint32_t* const* outs, bool band_dma, size_t* psmem) {
+    FrameParams prm;
+    memset(&prm, 0, sizeof prm);
+    const int W = fr->width;
+    const int yb = fr->y_block > 0 ? fr->y_block : 1;
+    prm.W = W;
+    prm.W_pad = (W + 31) & ~31;
+    prm.H = fr->height;
+    prm.y0 = fr->y0;
+    prm.y_step = (yb >= fr->y_step) ? 1 : fr->y_step;
+    prm.n_rows = frame_rows(fr);
+    prm.n_frames = n_frames;
+    prm.n_px_frame = (uint32_t)((size_t)prm.n_rows * W);
+    prm.y_block = (yb >= fr->y_step) ? 1 : yb;
+    prm.out_global = (outs && fr->out_pitch > 0) ? 1 : 0;
+    prm.pitch = prm.out_global ? fr->out_pitch : W;
+    prm.n_spheres = ctx->n_spheres;
+    prm.n_lights = ctx->n_lights;
+    prm.flags = fr->flags;
+    prm.aspect = fr->aspect;
+    prm.ez = (-1 / fr->aspect);  // kernel.cu:1629
+    prm.fz = 0.f - prm.ez;
+    for (int f = 0; f < n_frames; f++) {
+        const ore_camera* cam = &cams[f];
+        CamP& c = prm.cam[f];
+        c.Ox = 0.f + cam->org[0];  // add(eyePos, cam.Org), kernel.cu:1631
+        c.Oy = 0.f + cam->org[1];
+        c.Oz = prm.ez + cam->org[2];
+        // camera::rotateDir, kernel.cu:249-255: frame-uniform, evaluated once on the host
+        float yawRad = cam->yaw * (3.1415 / 180);
+        float pitchRad = cam->pitch * (3.1415 / 180);
+        c.cp = cosf(pitchRad);
+        c.sp = sinf(pitchRad);
+        c.cy = cosf(yawRad);
+        c.sy = sinf(yawRad);
+        prm.pixels[f] = outs ? outs[f] : (uint32_t*)ctx->pixels;
+        prm.sky_pixels[f] = band_dma ? ctx->band_buf + (size_t)f * prm.n_px_frame : prm.pixels[f];
+    }
+    prm.sky_pitch = band_dma ? W : prm.pitch;
+    prm.sky_global = band_dma ? 0 : prm.out_global;
+    const TileCone tc = tile_cone(fr->aspect, W, prm.y_block, prm.y_step, prm.fz);
+    prm.px_delta = tc.px_delta;
+    prm.tile_ca = tc.ca;
+    prm.tile_sa = tc.sa;
+    prm.dx_tab = ctx->dx_tab;
+    prm.dy_tab = ctx->dy_tab;
+    prm.sph_exact = ctx->sph_exact;
+    prm.sph_xsort = ctx->sph_xsort;
+    prm.sph_sort = ctx->sph_sort;
+    prm.sort_index = ctx->sort_index;
+    prm.leaf_sph = ctx->leaf_sph;
+    prm.super_sph = ctx->super_sph;
+    prm.n_sort = ctx->n_sort;
+    prm.n_leaves = ctx->n_leaves;
+    prm.n_leaves_pad = ctx->n_leaves_pad;
+    prm.n_supers = ctx->n_supers;
+    prm.n_supers_pad = ctx->n_supers_pad;
+    prm.prim_sorted = ctx->prim_sorted;
+    prm.cone_sorted = ctx->cone_sorted;
+    prm.leaf_cone = ctx->leaf_cone;
+    prm.super_cone = ctx->super_cone;
+    const size_t tree_bytes = ((size_t)ctx->n_supers_pad + (size_t)ctx->n_leaves_pad) * sizeof(float4);
+    const size_t all_bytes = tree_bytes + (size_t)ctx->n_sort * sizeof(float4);
+    prm.cone_resident = all_bytes <= PRIMARY_RESIDENT_BYTES ? 1 : 0;
+    *psmem = prm.cone_resident ? all_bytes : tree_bytes;
+    prm.tex_r = ctx->tex[0];
+    prm.tex_g = ctx->tex[1];
+    prm.tex_b = ctx->tex[2];
+    prm.tex_w = ctx->tex_w;
+    prm.tex_h = ctx->tex_h;
+    prm.sky_r = ctx->sky[0];
+    prm.sky_g = ctx->sky[1];
+    prm.sky_b = ctx->sky[2];
+    prm.sky_w = ctx->sky_w;
+    prm.sky_h = ctx->sky_h;
+    prm.sky_radius = ctx->sky_radius;
+    prm.cubes = ctx->cubes;
+    prm.planes = ctx->planes;
+    prm.n_cubes = ctx->n_cubes;
+    prm.n_planes = ctx->n_planes;
+    prm.tris = ctx->tris;
+    prm.boxes = ctx->boxes;
+    prm.box_offsets = ctx->box_offsets;
+    prm.box_indices = ctx->box_indices;
+    prm.box_sph = ctx->box_sph;
+    prm.box_cone = ctx->box_cone;
+    prm.n_tris = ctx->n_tris;
+    prm.n_boxes = ctx->n_boxes;
+    prm.n_live_boxes = ctx->mesh_live;
+    prm.mesh_has_normals = ctx->mesh_has_normals;
+    bool skip = ctx->tex_finite && !(fr->flags & ORE_FLAG_EXHAUSTIVE);
+    for (int i = 0; i < ctx->n_lights && skip; i++)
+        skip = std::isfinite(ctx->lights[i].r) && std::isfinite(ctx->lights[i].g) && std::isfinite(ctx->lights[i].b);
+    prm.skip_dark = skip ? 1 : 0;
+    prm.hit_list = ctx->hit_list;
+    prm.hit_ids = ctx->hit_ids;
+    prm.hit_ts = ctx->hit_ts;
+    prm.counters = ctx->counters;
+    for (int i = 0; i < ctx->n_lights; i++) prm.lights[i] = ctx->lights[i];
+    return prm;
+}
+
+// Enqueues a launch set on `stream`, in this order: prep, primary, the band-DMA copy (on band_stream, joined before the
+// first sweep), the shadow pass as ore_stage_plan.h plans it, the hint copy, the count kernel; timing events between them.
+static int launch_frame(ore_context* ctx, const FrameParams& prm, size_t psmem, uint32_t* const* outs, bool band_dma,
+                        cudaStream_t stream) {
+    int rc;
+    const size_t n_px = (size_t)prm.n_px_frame * (size_t)prm.n_frames;
+    const bool timing = !(prm.flags & ORE_FLAG_NO_KERNEL_TIMING);
+    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[0], stream));
+    {
+        int m = prm.W_pad > prm.n_rows ? prm.W_pad : prm.n_rows;
+        m = std::max(m, std::max(ctx->n_sort, std::max(ctx->n_leaves_pad, ctx->n_supers_pad)));
+        m = std::max(m, std::max(ctx->n_boxes, (int)CNT_SLOTS));
+        prep_frame_kernel<<<(m + 255) / 256, 256, 0, stream>>>(prm);
+        ORE_CUDA(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[1], stream));
+    const bool exh = (prm.flags & ORE_FLAG_EXHAUSTIVE) != 0;
+    const bool fast_libm = (prm.flags & ORE_FLAG_FAST_LIBM) != 0;
+    {
+        int grid = 0;
+        const long long tiles = (long long)((prm.W + 31) / 32) * ((prm.n_rows + TILE_ROWS - 1) / TILE_ROWS);
+        const long long n_batches = ((tiles + PRIMARY_WARPS - 1) / PRIMARY_WARPS) * prm.n_frames;
+        const PrimaryKernel primary = primary_kernels[exh][fast_libm];
+        if ((rc = grid_for(ctx, primary, psmem, &grid, PRIMARY_THREADS))) return rc;
+        if (grid > n_batches) grid = (int)n_batches;
+        primary<<<grid, PRIMARY_THREADS, psmem, stream>>>(prm);
+        ORE_CUDA(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[2], stream));
+    bool band_pending = false;
+    if (band_dma) {
+        // the rows the primary kernel has just written (sky pixels, 0 for hit pixels) travel to their place in the
+        // destination frames on a copy engine, behind the primary kernel and concurrently with stage A of the shadow
+        // pass; the sweep, which stores the hit pixels into the same rows, waits for them
+        ORE_CUDA(ctx, cudaEventRecord(ctx->ev_band_go, stream));
+        ORE_CUDA(ctx, cudaStreamWaitEvent(ctx->band_stream, ctx->ev_band_go, 0));
+        for (int f = 0; f < prm.n_frames; f++)   // (y_block and y_step are 1 for a contiguous band)
+            if ((rc = copy_row_blocks(ctx, outs[f], ctx->band_buf + (size_t)f * prm.n_px_frame, prm.W, prm.n_rows, prm.y_block,
+                                      prm.y_step, cudaMemcpyDefault, ctx->band_stream)))
+                return rc;
+        ORE_CUDA(ctx, cudaEventRecord(ctx->ev_band_done, ctx->band_stream));
+        band_pending = true;
+    }
+    auto join_band = [&]() -> int {
+        if (band_pending) {
+            ORE_CUDA(ctx, cudaStreamWaitEvent(stream, ctx->ev_band_done, 0));
+            band_pending = false;
+        }
+        return ORE_OK;
+    };
+    // Two-stage pass (default): shade_setup_kernel -> staging buffer -> staged shadow_sweep_kernel, in the chunk pairs of
+    // plan_stage, from the previous frame's hit count (a hint read without synchronisation), and one catch-all launch
+    // of the fused sweep for whatever lies beyond the staged chunks.  With no lights there is nothing to sweep: the
+    // primary kernel has already written 0 to every hit pixel.
+    const StagePlan plan = plan_stage(n_px, ctx->n_lights, (prm.flags & ORE_FLAG_FUSED_SHADOW) != 0, ctx->hits_hint_set,
+                                      *(volatile unsigned long long*)ctx->hits_hint, ctx->stage.cap(), ctx->stage_blocks_override,
+                                      ctx->stage_max_items);
+    bool staged = plan.staged;
+    if (staged && !ctx->stage.fits(plan.need_floats)) {
+        // (an earlier frame of this context may still be reading the old buffer on another stream)
+        if ((rc = wait_last_render(ctx))) return rc;
+        ORE_CUDA(ctx, ctx->stage.release());
+        if (ctx->stage.alloc(plan.need_floats) != cudaSuccess) {
+            (void)cudaGetLastError();  // no room for the staging buffer: the fused sweep needs none
+            staged = false;
+        }
+    }
+    StageArgs st{};
+    st.nv = STAGE_HEADER + STAGE_PER_LIGHT * ctx->n_lights;
+    if (ctx->n_lights == 0) {
+        // nothing to launch
+    } else if (!staged) {
+        if ((rc = join_band())) return rc;
+        if ((rc = launch_sweep(ctx, prm, st, false, exh, fast_libm, stream))) return rc;
+        ctx->last_launches++;
+    } else {
+        st.buf = ctx->stage;
+        st.cap_blocks = (uint32_t)plan.cap_blocks;
+        const StageKernel setup = shade_setup_kernels[fast_libm];
+        int grid_a = 0;
+        if ((rc = grid_for(ctx, setup, 0, &grid_a, STAGE_A_THREADS))) return rc;
+        for (int c = 0; c < plan.n_chunks; c++) {
+            st.chunk = c;
+            st.first_block = (uint32_t)((size_t)c * plan.cap_blocks);
+            setup<<<grid_a, STAGE_A_THREADS, 0, stream>>>(prm, st);
+            ORE_CUDA(ctx, cudaGetLastError());
+            if ((rc = join_band())) return rc;   // (band DMA: the first stage A ran beside the copy)
+            if ((rc = launch_sweep(ctx, prm, st, true, exh, fast_libm, stream))) return rc;
+            ctx->last_launches += 2;
+        }
+        if (plan.catch_all) {
+            // catch-all: hit-list blocks beyond the staged chunks (normally none: exits at once), one fused launch
+            StageArgs rest{};
+            rest.first_block = (uint32_t)plan.catch_all_block;
+            rest.nv = st.nv;
+            if ((rc = launch_sweep(ctx, prm, rest, false, exh, fast_libm, stream))) return rc;
+            ctx->last_launches++;
+        }
+    }
+    if ((rc = join_band())) return rc;   // (no lights: nothing but the copy writes the frames)
+    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[3], stream));
+    // hint for the next frame of this context (see hits_hint): 8 bytes, no synchronisation
+    ORE_CUDA(ctx, cudaMemcpyAsync(ctx->hits_hint, ctx->counters + CNT_HITS, sizeof(unsigned long long),
+                                  cudaMemcpyDeviceToHost, stream));
+    ctx->hits_hint_set = true;
+    if (prm.flags & ORE_FLAG_COUNT_REFERENCE_TESTS) {
+        count_reference_tests_kernel<<<ctx->sm_count * 8, CTA_THREADS, 0, stream>>>(prm);
+        ORE_CUDA(ctx, cudaGetLastError());
+        ctx->last_launches++;
+    }
+    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[4], stream));
+    ctx->ev_valid = timing;
+    ORE_CUDA(ctx, cudaEventRecord(ctx->ev_done, stream));
+    ctx->ev_done_set = true;
+    return ORE_OK;
+}
+
 // One launch set for a batch of n_frames cameras.  outs: n_frames device framebuffers, or null (n_frames == 1 only): the
 // context's own framebuffer.
 static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, const ore_frame* fr, uint32_t* const* outs,
@@ -921,343 +1165,42 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
     ctx->last_n_spheres = ctx->n_spheres;
     ctx->last_launches = 0;
     ctx->ev_valid = false;
-    ctx->ran_count = false;
     ctx->last_prm_valid = false;
     if (n_px == 0) return ORE_OK;
+    for (int f = 0; outs && f < n_frames; f++)
+        if (!outs[f]) return fail(ctx, ORE_ERR_INVALID, "ore_render: null framebuffer in the batch");
     // the scene of the last stream-ordered update, wherever it ran
     if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaStreamWaitEvent(stream, ctx->ev_scene, 0));
 
     int rc;
-    const int W_pad = (W + 31) & ~31;
-    if ((rc = ensure_dev(ctx, &ctx->dx_tab, &ctx->dx_cap, (size_t)W_pad))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->dy_tab, &ctx->dy_cap, (size_t)n_rows))) return rc;
-    if (n_px > ctx->px_cap || !ctx->hit_list) {
-        if ((rc = wait_last_render(ctx))) return rc;   // (an earlier frame may still be running on another stream)
-        size_t c1 = ctx->hit_list ? ctx->px_cap : 0, c2 = c1, c3 = c1;
-        if ((rc = ensure_dev(ctx, &ctx->hit_list, &c1, n_px))) return rc;
-        if ((rc = ensure_dev(ctx, &ctx->hit_ids, &c2, n_px))) return rc;
-        if ((rc = ensure_dev(ctx, &ctx->hit_ts, &c3, n_px))) return rc;
-        ctx->px_cap = std::min(std::min(c1, c2), c3);
-    }
-    if (!outs && (n_px_frame > ctx->pixels_cap || !ctx->pixels)) {
-        // the context's own framebuffer: only ore_render (one frame, host output) renders into it
-        if ((rc = wait_last_render(ctx))) return rc;
-        if ((rc = ensure_dev(ctx, &ctx->pixels, &ctx->pixels_cap, n_px_frame))) return rc;
-    }
-
-    FrameParams prm;
-    memset(&prm, 0, sizeof prm);
-    prm.W = W;
-    prm.W_pad = W_pad;
-    prm.H = fr->height;
-    prm.y0 = fr->y0;
-    prm.y_step = (yb >= fr->y_step) ? 1 : fr->y_step;
-    prm.n_rows = n_rows;
-    prm.n_frames = n_frames;
-    prm.n_px_frame = (uint32_t)n_px_frame;
-    prm.y_block = (yb >= fr->y_step) ? 1 : yb;
-    prm.out_global = (outs && fr->out_pitch > 0) ? 1 : 0;
-    prm.pitch = prm.out_global ? fr->out_pitch : W;
-    prm.n_spheres = ctx->n_spheres;
-    prm.n_lights = ctx->n_lights;
-    prm.flags = fr->flags;
-    prm.aspect = fr->aspect;
-    prm.ez = (-1 / fr->aspect);  // kernel.cu:1629
-    prm.fz = 0.f - prm.ez;
-    for (int f = 0; f < n_frames; f++) {
-        const ore_camera* cam = &cams[f];
-        CamP& c = prm.cam[f];
-        c.Ox = 0.f + cam->org[0];  // add(eyePos, cam.Org), kernel.cu:1631
-        c.Oy = 0.f + cam->org[1];
-        c.Oz = prm.ez + cam->org[2];
-        // camera::rotateDir, kernel.cu:249-255: frame-uniform, evaluated once on the host
-        float yawRad = cam->yaw * (3.1415 / 180);
-        float pitchRad = cam->pitch * (3.1415 / 180);
-        c.cp = cosf(pitchRad);
-        c.sp = sinf(pitchRad);
-        c.cy = cosf(yawRad);
-        c.sy = sinf(yawRad);
-        prm.pixels[f] = outs ? outs[f] : ctx->pixels;
-        if (!prm.pixels[f]) return fail(ctx, ORE_ERR_INVALID, "ore_render: null framebuffer in the batch");
-        prm.sky_pixels[f] = prm.pixels[f];
-    }
-    prm.sky_pitch = prm.pitch;
-    prm.sky_global = prm.out_global;
+    if ((rc = frame_reserve(ctx, ctx->dx_tab, (size_t)((W + 31) & ~31)))) return rc;
+    if ((rc = frame_reserve(ctx, ctx->dy_tab, (size_t)n_rows))) return rc;
+    if ((rc = frame_reserve(ctx, ctx->hit_list, n_px))) return rc;
+    if ((rc = frame_reserve(ctx, ctx->hit_ids, n_px))) return rc;
+    if ((rc = frame_reserve(ctx, ctx->hit_ts, n_px))) return rc;
+    // the context's own framebuffer: only ore_render (one frame, host output) renders into it
+    if (!outs && (rc = frame_reserve(ctx, ctx->pixels, n_px_frame))) return rc;
     // Band DMA (include/ore_render.h; opt-in): rows whose 8-row blocks are contiguous at the destination (pitch == width)
-    const bool band_dma = prm.out_global && fr->out_pitch == W && (fr->flags & ORE_FLAG_BAND_DMA) != 0;
+    const bool band_dma = outs && fr->out_pitch == W && (fr->flags & ORE_FLAG_BAND_DMA) != 0;
     if (band_dma) {
-        if (n_px > ctx->band_cap || !ctx->band_buf) {
-            if ((rc = wait_last_render(ctx))) return rc;
-            if ((rc = ensure_dev(ctx, &ctx->band_buf, &ctx->band_cap, n_px))) return rc;
-        }
+        if ((rc = frame_reserve(ctx, ctx->band_buf, n_px))) return rc;
         if (!ctx->band_stream) {
             ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->band_stream, cudaStreamNonBlocking));
             ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_band_go, cudaEventDisableTiming));
             ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_band_done, cudaEventDisableTiming));
         }
-        for (int f = 0; f < n_frames; f++) prm.sky_pixels[f] = ctx->band_buf + (size_t)f * n_px_frame;
-        prm.sky_pitch = W;
-        prm.sky_global = 0;
     }
-    {
-        // largest half-angle of a 32 x TILE_ROWS pixel tile seen from the eye (tile cone of the primary
-        // kernel): |v_pixel - v_centre| <= halfdiag on the image plane and |v| >= fz, so sin(a) <= halfdiag/fz
-        const double delta = 2.0 * (double)fr->aspect / (double)W;
-        // tallest image-row span of TILE_ROWS consecutive RENDERED rows (rows come in blocks of y_block)
-        int max_span = 0;
-        {
-            const int B = prm.y_block, S = prm.y_step;
-            for (int k0 = 0; k0 < B * TILE_ROWS; k0 += TILE_ROWS) {
-                const int k1 = k0 + TILE_ROWS - 1;
-                const int sp = ((k1 / B) * S + k1 % B) - ((k0 / B) * S + k0 % B);
-                if (sp > max_span) max_span = sp;
-            }
-        }
-        const double hx = 16.0 * delta, hy = (0.5 * max_span + 0.5) * delta;
-        const double xr = sqrt(hx * hx + hy * hy) / fabs((double)prm.fz);
-        prm.px_delta = (float)delta;
-        if (!(xr < 0.9)) {
-            prm.tile_ca = -1e20f;  // tiles too wide for a cone: every sphere is a candidate
-            prm.tile_sa = 0.f;
-        } else {
-            const double a = asin(xr) * 1.001 + 1e-6;
-            prm.tile_ca = (float)(cos(a) * (1.0 - 1e-6) - 1e-6);
-            prm.tile_sa = (float)(sin(a) * (1.0 + 1e-6) + 1e-6);
-        }
-    }
-    prm.dx_tab = ctx->dx_tab;
-    prm.dy_tab = ctx->dy_tab;
-    prm.sph_exact = ctx->sph_exact;
-    prm.sph_xsort = ctx->sph_xsort;
-    prm.sph_sort = ctx->sph_sort;
-    prm.sort_index = ctx->sort_index;
-    prm.leaf_sph = ctx->leaf_sph;
-    prm.super_sph = ctx->super_sph;
-    prm.n_sort = ctx->n_sort;
-    prm.n_leaves = ctx->n_leaves;
-    prm.n_leaves_pad = ctx->n_leaves_pad;
-    prm.n_supers = ctx->n_supers;
-    prm.n_supers_pad = ctx->n_supers_pad;
-    prm.prim_sorted = ctx->prim_sorted;
-    prm.cone_sorted = ctx->cone_sorted;
-    prm.leaf_cone = ctx->leaf_cone;
-    prm.super_cone = ctx->super_cone;
-    const size_t tree_bytes = ((size_t)ctx->n_supers_pad + (size_t)ctx->n_leaves_pad) * sizeof(float4);
-    const size_t all_bytes = tree_bytes + (size_t)ctx->n_sort * sizeof(float4);
-    prm.cone_resident = all_bytes <= PRIMARY_RESIDENT_BYTES ? 1 : 0;
-    const size_t psmem = prm.cone_resident ? all_bytes : tree_bytes;
+    size_t psmem = 0;
+    FrameParams prm = frame_params(ctx, cams, n_frames, fr, outs, band_dma, &psmem);
     if (psmem > 200 * 1024) return fail(ctx, ORE_ERR_INVALID, "ore_render: more than ~100 000 spheres are not supported");
-    prm.tex_r = ctx->tex[0];
-    prm.tex_g = ctx->tex[1];
-    prm.tex_b = ctx->tex[2];
-    prm.tex_w = ctx->tex_w;
-    prm.tex_h = ctx->tex_h;
-    prm.sky_r = ctx->sky[0];
-    prm.sky_g = ctx->sky[1];
-    prm.sky_b = ctx->sky[2];
-    prm.sky_w = ctx->sky_w;
-    prm.sky_h = ctx->sky_h;
-    prm.sky_radius = ctx->sky_radius;
-    prm.cubes = ctx->cubes;
-    prm.planes = ctx->planes;
-    prm.n_cubes = ctx->n_cubes;
-    prm.n_planes = ctx->n_planes;
-    prm.tris = ctx->tris;
-    prm.boxes = ctx->boxes;
-    prm.box_offsets = ctx->box_offsets;
-    prm.box_indices = ctx->box_indices;
-    prm.box_sph = ctx->box_sph;
-    prm.box_cone = ctx->box_cone;
-    prm.n_tris = ctx->n_tris;
-    prm.n_boxes = ctx->n_boxes;
-    prm.n_live_boxes = ctx->mesh_live;
-    prm.mesh_has_normals = ctx->mesh_has_normals;
-    {
-        bool skip = ctx->tex_finite && !(fr->flags & ORE_FLAG_EXHAUSTIVE);
-        for (int i = 0; i < ctx->n_lights && skip; i++)
-            skip = std::isfinite(ctx->lights[i].r) && std::isfinite(ctx->lights[i].g) && std::isfinite(ctx->lights[i].b);
-        prm.skip_dark = skip ? 1 : 0;
-    }
-    prm.hit_list = ctx->hit_list;
-    prm.hit_ids = ctx->hit_ids;
-    prm.hit_ts = ctx->hit_ts;
-    prm.counters = ctx->counters;
     if (!ctx->dbg_cycles_path.empty()) {
-        const size_t nb = (n_px + 31) / 32;
-        if (nb > ctx->dbg_cap) {
-            if (ctx->dbg_cycles) ORE_CUDA(ctx, cudaFree(ctx->dbg_cycles));
-            ORE_CUDA(ctx, cudaMalloc((void**)&ctx->dbg_cycles, 2 * nb * sizeof(uint32_t)));
-            ctx->dbg_cap = nb;
-        }
-        ORE_CUDA(ctx, cudaMemsetAsync(ctx->dbg_cycles, 0, 2 * ctx->dbg_cap * sizeof(uint32_t), stream));
+        const size_t nb = (n_px + 31) / 32;   // [2][nb]: stage A, stage B
+        if (!ctx->dbg_cycles.fits(2 * nb)) ORE_CUDA(ctx, ctx->dbg_cycles.alloc(2 * nb));
+        ORE_CUDA(ctx, cudaMemsetAsync(ctx->dbg_cycles, 0, ctx->dbg_cycles.cap() * sizeof(uint32_t), stream));
         prm.dbg_cycles = ctx->dbg_cycles;
-        prm.dbg_cap = (uint32_t)ctx->dbg_cap;
+        prm.dbg_cap = (uint32_t)(ctx->dbg_cycles.cap() / 2);
     }
-    for (int i = 0; i < ctx->n_lights; i++) prm.lights[i] = ctx->lights[i];
-
-    const bool timing = !(fr->flags & ORE_FLAG_NO_KERNEL_TIMING);
-    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[0], stream));
-    {
-        int m = W_pad > n_rows ? W_pad : n_rows;
-        m = std::max(m, std::max(ctx->n_sort, std::max(ctx->n_leaves_pad, ctx->n_supers_pad)));
-        m = std::max(m, std::max(ctx->n_boxes, (int)CNT_SLOTS));
-        prep_frame_kernel<<<(m + 255) / 256, 256, 0, stream>>>(prm);
-        ORE_CUDA(ctx, cudaGetLastError());
-        ctx->last_launches++;
-    }
-    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[1], stream));
-    const bool exh = (fr->flags & ORE_FLAG_EXHAUSTIVE) != 0;
-    const bool fast_libm = (fr->flags & ORE_FLAG_FAST_LIBM) != 0;
-    {
-        int grid = 0;
-        const long long tiles = (long long)((W + 31) / 32) * ((n_rows + TILE_ROWS - 1) / TILE_ROWS);
-        const long long n_batches = ((tiles + PRIMARY_WARPS - 1) / PRIMARY_WARPS) * n_frames;
-        const PrimaryKernel primary = primary_kernels[exh][fast_libm];
-        if ((rc = grid_for(ctx, primary, psmem, &grid, PRIMARY_THREADS))) return rc;
-        if (grid > n_batches) grid = (int)n_batches;
-        primary<<<grid, PRIMARY_THREADS, psmem, stream>>>(prm);
-        ORE_CUDA(ctx, cudaGetLastError());
-        ctx->last_launches++;
-    }
-    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[2], stream));
-    bool band_pending = false;
-    if (band_dma) {
-        // the rows the primary kernel has just written (sky pixels, 0 for hit pixels) travel to their place in the
-        // destination frames on a copy engine, behind the primary kernel and concurrently with stage A of the shadow
-        // pass; the sweep, which stores the hit pixels into the same rows, waits for them
-        ORE_CUDA(ctx, cudaEventRecord(ctx->ev_band_go, stream));
-        ORE_CUDA(ctx, cudaStreamWaitEvent(ctx->band_stream, ctx->ev_band_go, 0));
-        const int B = prm.y_block, S = prm.y_step;           // (1, 1 for a contiguous band)
-        const int full = n_rows / B, rem = n_rows % B;
-        for (int f = 0; f < n_frames; f++) {
-            const uint32_t* src = ctx->band_buf + (size_t)f * n_px_frame;
-            uint32_t* dst = outs[f];
-            if (full > 0)
-                ORE_CUDA(ctx, cudaMemcpy2DAsync(dst, (size_t)S * W * sizeof(uint32_t), src, (size_t)B * W * sizeof(uint32_t),
-                                                (size_t)B * W * sizeof(uint32_t), (size_t)full, cudaMemcpyDefault, ctx->band_stream));
-            if (rem > 0)
-                ORE_CUDA(ctx, cudaMemcpyAsync(dst + (size_t)full * S * W, src + (size_t)full * B * W,
-                                              (size_t)rem * W * sizeof(uint32_t), cudaMemcpyDefault, ctx->band_stream));
-        }
-        ORE_CUDA(ctx, cudaEventRecord(ctx->ev_band_done, ctx->band_stream));
-        band_pending = true;
-    }
-    auto join_band = [&]() -> int {
-        if (band_pending) {
-            ORE_CUDA(ctx, cudaStreamWaitEvent(stream, ctx->ev_band_done, 0));
-            band_pending = false;
-        }
-        return ORE_OK;
-    };
-    {
-        // Two-stage pass (default): shade_setup_kernel -> staging buffer -> staged shadow_sweep_kernel.  The host does
-        // not know the hit count (no sync): the first frame of a context sizes the staging buffer from the pixel count,
-        // later frames from the previous frame's hit count (a hint read without synchronisation) - normally ONE chunk
-        // pair per frame -, and one catch-all launch of the fused sweep takes whatever lies beyond the staged chunks.
-        // With no lights there is nothing to sweep: the primary kernel has already written 0 to every hit pixel.
-        StageArgs st{};
-        st.nv = STAGE_HEADER + STAGE_PER_LIGHT * ctx->n_lights;
-        const size_t n_blocks_px = (n_px + 31) / 32;
-        bool staged = !(fr->flags & ORE_FLAG_FUSED_SHADOW);
-        size_t cap_blocks = 0, est_blocks = n_blocks_px;
-        if (ctx->n_lights == 0) {
-            staged = false;
-        } else if (staged) {
-            size_t est_items;
-            if (ctx->hits_hint_set) {
-                // previous frame's hit count + 12.5 % + 32 K items; the catch-all below covers a wrong guess
-                const unsigned long long h = *(volatile unsigned long long*)ctx->hits_hint;
-                est_items = (size_t)(h + h / 8 + 32768ull);
-            } else {
-                // no frame of this context has finished yet: half the pixels (growing the buffer later costs a
-                // device-wide synchronisation; the cap below bounds the memory)
-                est_items = n_px / 2 > ((size_t)1 << 20) ? n_px / 2 : ((size_t)1 << 20);
-            }
-            if (est_items > n_px) est_items = n_px;
-            est_blocks = (est_items + 31) / 32;
-            // the staging buffer never grows past stage_max_items (448 bytes each with three lights: 3.6 GB); a longer hit
-            // list - a batch of several 8K frames - is walked in chunk pairs of that size, each a full-size launch
-            const size_t max_blocks = (ctx->stage_max_items + 31) / 32;
-            const size_t have_blocks = ctx->stage ? ctx->stage_cap / (32 * (size_t)st.nv) : 0;
-            cap_blocks = have_blocks;
-            if (ctx->stage_blocks_override) {
-                cap_blocks = ctx->stage_blocks_override;
-                while ((n_blocks_px + cap_blocks - 1) / cap_blocks > (size_t)MAX_STAGE_CHUNKS) cap_blocks *= 2;
-            } else if (est_blocks > have_blocks && have_blocks < max_blocks) {
-                cap_blocks = est_blocks + est_blocks / 4;   // grow with some slack: reallocations stay rare
-                if (cap_blocks > n_blocks_px) cap_blocks = n_blocks_px;
-                if (cap_blocks > max_blocks) cap_blocks = max_blocks;
-            }
-            while ((est_blocks + cap_blocks - 1) / cap_blocks > (size_t)MAX_STAGE_CHUNKS) cap_blocks *= 2;
-            const size_t need = cap_blocks * 32 * (size_t)st.nv;
-            if (need > ctx->stage_cap || !ctx->stage) {
-                // (an earlier frame of this context may still be reading the old buffer on another stream)
-                if ((rc = wait_last_render(ctx))) return rc;
-                if (ctx->stage) ORE_CUDA(ctx, cudaFree(ctx->stage));
-                ctx->stage = nullptr;
-                ctx->stage_cap = 0;
-                if (cudaMalloc((void**)&ctx->stage, need * sizeof(float)) == cudaSuccess) {
-                    ctx->stage_cap = need;
-                } else {
-                    (void)cudaGetLastError();  // no room for the staging buffer: the fused sweep needs none
-                    ctx->stage = nullptr;
-                    staged = false;
-                }
-            }
-        }
-        if (ctx->n_lights == 0) {
-            // nothing to launch
-        } else if (!staged) {
-            if ((rc = join_band())) return rc;
-            if ((rc = launch_sweep(ctx, prm, st, false, exh, fast_libm, stream))) return rc;
-            ctx->last_launches++;
-        } else {
-            st.buf = ctx->stage;
-            int n_chunks = (int)((est_blocks + cap_blocks - 1) / cap_blocks);
-            if (n_chunks < 1) n_chunks = 1;
-            // equal chunks: the expected hit list is split evenly instead of into full buffers plus a small remainder
-            if (!ctx->stage_blocks_override) cap_blocks = (est_blocks + n_chunks - 1) / n_chunks;
-            st.cap_blocks = (uint32_t)cap_blocks;
-            const int n_chunks_max = (int)((n_blocks_px + cap_blocks - 1) / cap_blocks);
-            if (n_chunks > n_chunks_max) n_chunks = n_chunks_max;
-            const StageKernel setup = shade_setup_kernels[fast_libm];
-            int grid_a = 0;
-            if ((rc = grid_for(ctx, setup, 0, &grid_a, STAGE_A_THREADS))) return rc;
-            for (int c = 0; c < n_chunks; c++) {
-                st.chunk = c;
-                st.first_block = (uint32_t)((size_t)c * cap_blocks);
-                setup<<<grid_a, STAGE_A_THREADS, 0, stream>>>(prm, st);
-                ORE_CUDA(ctx, cudaGetLastError());
-                if ((rc = join_band())) return rc;   // (band DMA: the first stage A ran beside the copy)
-                if ((rc = launch_sweep(ctx, prm, st, true, exh, fast_libm, stream))) return rc;
-                ctx->last_launches += 2;
-            }
-            if (n_chunks < n_chunks_max) {
-                // catch-all: hit-list blocks beyond the staged chunks (normally none: exits at once), one fused launch
-                StageArgs rest{};
-                rest.first_block = (uint32_t)((size_t)n_chunks * cap_blocks);
-                rest.nv = st.nv;
-                if ((rc = launch_sweep(ctx, prm, rest, false, exh, fast_libm, stream))) return rc;
-                ctx->last_launches++;
-            }
-        }
-    }
-    if ((rc = join_band())) return rc;   // (no lights: nothing but the copy writes the frames)
-    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[3], stream));
-    // hint for the next frame of this context (see hits_hint): 8 bytes, no synchronisation
-    ORE_CUDA(ctx, cudaMemcpyAsync(ctx->hits_hint, ctx->counters + CNT_HITS, sizeof(unsigned long long),
-                                  cudaMemcpyDeviceToHost, stream));
-    ctx->hits_hint_set = true;
-    if (fr->flags & ORE_FLAG_COUNT_REFERENCE_TESTS) {
-        count_reference_tests_kernel<<<ctx->sm_count * 8, CTA_THREADS, 0, stream>>>(prm);
-        ORE_CUDA(ctx, cudaGetLastError());
-        ctx->last_launches++;
-        ctx->ran_count = true;
-    }
-    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[4], stream));
-    ctx->ev_valid = timing;
-    ORE_CUDA(ctx, cudaEventRecord(ctx->ev_done, stream));
-    ctx->ev_done_set = true;
+    if ((rc = launch_frame(ctx, prm, psmem, outs, band_dma, stream))) return rc;
     ctx->last_prm = prm;
     ctx->last_prm_valid = true;
     return ORE_OK;
@@ -1426,7 +1369,7 @@ static int render_async_impl(ore_context* ctx, const ore_camera* cams, int n_fra
         // new geometry: the two sets are laid out afresh, so nothing of the old layout may still be in flight
         ORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         ORE_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
-        if ((rc = ensure_dev(ctx, &ctx->async_pool, &ctx->async_pool_cap, 2 * (size_t)n_frames * (n_px ? n_px : 1)))) return rc;
+        ORE_CUDA(ctx, ctx->async_pool.reserve(2 * (size_t)n_frames * (n_px ? n_px : 1)));
         ctx->async_px = n_px;
         ctx->async_k = n_frames;
     }
@@ -1446,15 +1389,10 @@ static int render_async_impl(ore_context* ctx, const ore_camera* cams, int n_fra
                 // packed, or a contiguous band: one linear copy
                 ORE_CUDA(ctx, cudaMemcpyAsync(out_host[f], targets[f], n_px * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->copy_stream));
             } else {
-                // block-interleaved rows: blocks of yb rows, y_step image rows apart -> one strided copy (+ a ragged tail)
-                const size_t blk_bytes = (size_t)yb * W * sizeof(uint32_t);
-                const size_t full = (size_t)n_rows / yb, rem = (size_t)n_rows % yb;
-                if (full)
-                    ORE_CUDA(ctx, cudaMemcpy2DAsync(out_host[f], (size_t)frame->y_step * W * sizeof(uint32_t), targets[f], blk_bytes,
-                                                    blk_bytes, full, cudaMemcpyDeviceToHost, ctx->copy_stream));
-                if (rem)
-                    ORE_CUDA(ctx, cudaMemcpyAsync(out_host[f] + full * (size_t)frame->y_step * W, targets[f] + full * (size_t)yb * W,
-                                                  rem * W * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->copy_stream));
+                // block-interleaved rows: blocks of yb rows, y_step image rows apart
+                if ((rc = copy_row_blocks(ctx, out_host[f], targets[f], W, n_rows, yb, frame->y_step, cudaMemcpyDeviceToHost,
+                                          ctx->copy_stream)))
+                    return rc;
             }
         }
         if (done_flag && (rc = ore_flag_write(ctx, ctx->copy_stream, done_flag, first_value + (uint32_t)f))) return rc;
@@ -1559,11 +1497,8 @@ extern "C" int ore_get_hits(ore_context* ctx, int32_t* hit_id_host, float* hit_t
     if (!ctx->last_prm_valid) return fail(ctx, ORE_ERR_INVALID, "ore_get_hits: no frame rendered");
     if (ctx->last_frames != 1) return fail(ctx, ORE_ERR_INVALID, "ore_get_hits: the last render was a batch (render the frame alone)");
     // the render path keeps compact hit records only; the per-pixel maps are built here, on demand
-    int rc;
-    size_t c1 = ctx->map_cap, c2 = c1;
-    if ((rc = ensure_dev(ctx, &ctx->hit_id_map, &c1, ctx->last_px))) return rc;
-    if ((rc = ensure_dev(ctx, &ctx->hit_t_map, &c2, ctx->last_px))) return rc;
-    ctx->map_cap = std::min(c1, c2);
+    ORE_CUDA(ctx, ctx->hit_id_map.reserve(ctx->last_px));
+    ORE_CUDA(ctx, ctx->hit_t_map.reserve(ctx->last_px));
     fill_hits_kernel<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(ctx->hit_id_map, ctx->hit_t_map, ctx->last_px);
     expand_hits_kernel<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(ctx->last_prm, ctx->hit_id_map, ctx->hit_t_map);
     ORE_CUDA(ctx, cudaGetLastError());
@@ -1612,20 +1547,17 @@ extern "C" int ore_get_kernel_ms(ore_context* ctx, float ms[4]) {
 extern "C" int ore_debug_libm(ore_context* ctx, int op, int n, const float* a_host, const float* b_host, float* out_host) {
     if (!ctx || n <= 0 || !a_host || !out_host || op < 0 || op > 6) return ORE_ERR_INVALID;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
-    float *a = nullptr, *b = nullptr, *o = nullptr;
+    DevBuf<float> a, b, o;
     const size_t bytes = (size_t)n * sizeof(float);
-    ORE_CUDA(ctx, cudaMalloc((void**)&a, bytes));
-    ORE_CUDA(ctx, cudaMalloc((void**)&b, bytes));
-    ORE_CUDA(ctx, cudaMalloc((void**)&o, bytes));
+    ORE_CUDA(ctx, a.alloc(n));
+    ORE_CUDA(ctx, b.alloc(n));
+    ORE_CUDA(ctx, o.alloc(n));
     ORE_CUDA(ctx, cudaMemcpy(a, a_host, bytes, cudaMemcpyHostToDevice));
     ORE_CUDA(ctx, cudaMemcpy(b, b_host ? b_host : a_host, bytes, cudaMemcpyHostToDevice));
     libm_probe_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(op, n, a, b, o);
     ORE_CUDA(ctx, cudaGetLastError());
     ORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     ORE_CUDA(ctx, cudaMemcpy(out_host, o, bytes, cudaMemcpyDeviceToHost));
-    cudaFree(a);
-    cudaFree(b);
-    cudaFree(o);
     return ORE_OK;
 }
 
@@ -1660,28 +1592,31 @@ extern "C" int ore_debug_mesh(ore_context* ctx, int32_t which, void* host_out, i
 extern "C" int ore_measure_fp32_peak(ore_context* ctx, double* tflops, double* sm_clock_mhz_nominal) {
     if (!ctx || !tflops) return ORE_ERR_INVALID;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
-    float* d = nullptr;
-    ORE_CUDA(ctx, cudaMalloc((void**)&d, sizeof(float)));
+    DevBuf<float> d;
+    ORE_CUDA(ctx, d.alloc(1));
     const int iters = 4096, grid = ctx->sm_count * 8;
-    cudaEvent_t a, b;
-    ORE_CUDA(ctx, cudaEventCreate(&a));
-    ORE_CUDA(ctx, cudaEventCreate(&b));
+    struct Events {   // (destroyed on every path out)
+        cudaEvent_t a = nullptr, b = nullptr;
+        ~Events() {
+            if (a) cudaEventDestroy(a);
+            if (b) cudaEventDestroy(b);
+        }
+    } ev;
+    ORE_CUDA(ctx, cudaEventCreate(&ev.a));
+    ORE_CUDA(ctx, cudaEventCreate(&ev.b));
     double best = 0.0;
     for (int rep = 0; rep < 6; rep++) {
-        ORE_CUDA(ctx, cudaEventRecord(a, ctx->stream));
+        ORE_CUDA(ctx, cudaEventRecord(ev.a, ctx->stream));
         fp32_burn_kernel<<<grid, CTA_THREADS, 0, ctx->stream>>>(d, iters, 1.0000001f, 1e-9f);
         ORE_CUDA(ctx, cudaGetLastError());
-        ORE_CUDA(ctx, cudaEventRecord(b, ctx->stream));
-        ORE_CUDA(ctx, cudaEventSynchronize(b));
+        ORE_CUDA(ctx, cudaEventRecord(ev.b, ctx->stream));
+        ORE_CUDA(ctx, cudaEventSynchronize(ev.b));
         float ms = 0.f;
-        ORE_CUDA(ctx, cudaEventElapsedTime(&ms, a, b));
+        ORE_CUDA(ctx, cudaEventElapsedTime(&ms, ev.a, ev.b));
         const double flop = 2.0 * 16 * 8 * (double)iters * CTA_THREADS * (double)grid;
         const double tf = flop / (ms * 1e-3) / 1e12;
         if (rep >= 1 && tf > best) best = tf;
     }
-    cudaEventDestroy(a);
-    cudaEventDestroy(b);
-    cudaFree(d);
     *tflops = best;
     if (sm_clock_mhz_nominal) {
         int khz = 0;

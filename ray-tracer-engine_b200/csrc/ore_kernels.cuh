@@ -11,6 +11,7 @@
 #pragma once
 #include "ore_clusters.h"   // ORE_KAPPA_SHADOW (the margin R' is rounded up for)
 #include "ore_device.cuh"
+#include "ore_stage_plan.h"   // the staging buffer's layout constants
 
 namespace ore {
 
@@ -48,15 +49,8 @@ enum CounterSlot {
     CNT_STAGE_B0 = CNT_STAGE_A0 + 32,          // per-chunk block cursors of the staged shadow_sweep_kernel
     CNT_SLOTS = CNT_STAGE_B0 + 32
 };
-constexpr int MAX_STAGE_CHUNKS = 32;
 
-// Staging buffer between shade_setup_kernel and the staged shadow_sweep_kernel: blocks of 32 hit-list items,
-// value-major inside a block (value v of lane i at (block * nv + v) * 32 + i, so every access is one coalesced
-// 128-byte line and a light's 30 direction components are one contiguous 3840-byte piece for a TMA bulk copy).
-// Values: 0-2 start, 3-5 texel r,g,b, then 35 per light: cone axis (3), cone min-dot (-1: degenerate bundle),
-// a = dot(normal, toL), 30 direction components.
-constexpr int STAGE_HEADER = 6;
-constexpr int STAGE_PER_LIGHT = 35;
+// staging buffer layout (MAX_STAGE_CHUNKS, STAGE_HEADER, STAGE_PER_LIGHT): ore_stage_plan.h
 constexpr int STAGE_DIRS_AT = 5;
 struct StageArgs {
     float* buf;
