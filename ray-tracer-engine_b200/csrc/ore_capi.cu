@@ -76,24 +76,74 @@ private:
 template <typename T>
 using DevBuf = Buf<T, DeviceMem>;
 
+// A stream, event or graph the context (or a scope) owns, destroyed with it.  A caller's stream is never owned.
+template <typename H, cudaError_t (*Destroy)(H)>
+class Handle {
+public:
+    Handle() = default;
+    Handle(const Handle&) = delete;
+    Handle& operator=(const Handle&) = delete;
+    ~Handle() { reset(); }
+    operator H() const { return h_; }
+    cudaError_t reset() {
+        const cudaError_t e = h_ ? Destroy(h_) : cudaSuccess;
+        h_ = nullptr;
+        return e;
+    }
+    // where a create call writes the new handle (the one held before is destroyed)
+    H* put() {
+        reset();
+        return &h_;
+    }
+
+private:
+    H h_ = nullptr;
+};
+using Stream = Handle<cudaStream_t, cudaStreamDestroy>;
+using Event = Handle<cudaEvent_t, cudaEventDestroy>;
+using Graph = Handle<cudaGraph_t, cudaGraphDestroy>;
+using GraphExec = Handle<cudaGraphExec_t, cudaGraphExecDestroy>;
+
+// The last X, if any: an event and whether it has been recorded.  Waiting for a marker never recorded (or forgotten)
+// does nothing.
+class Marker {
+public:
+    cudaEvent_t* put() { return ev_.put(); }
+    cudaError_t record(cudaStream_t s) {
+        const cudaError_t e = cudaEventRecord(ev_, s);
+        if (e == cudaSuccess) recorded_ = true;
+        return e;
+    }
+    cudaError_t stream_wait(cudaStream_t s) const { return recorded_ ? cudaStreamWaitEvent(s, ev_, 0) : cudaSuccess; }
+    cudaError_t host_wait() const { return recorded_ ? cudaEventSynchronize(ev_) : cudaSuccess; }
+    void forget() { recorded_ = false; }
+    bool recorded() const { return recorded_; }
+    cudaEvent_t event() const { return ev_; }
+
+private:
+    Event ev_;
+    bool recorded_ = false;
+};
+
 }  // namespace
 
 struct ore_context {
-    // (frees every buffer below; not an export of the library)
+    // (frees every buffer, stream, event and graph below; not an export of the library)
     __attribute__((visibility("hidden"))) ~ore_context() = default;
     int device = 0;
     int sm_count = 0;
-    cudaStream_t stream = nullptr;
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_rendered[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
+    Stream stream;
+    Stream copy_stream;
+    Event ev_rendered[2], ev_copied[2];
     // device framebuffers of the pipelined presentation: two sets (one being copied out while the other is rendered)
     // of `async_k` frames of `async_px` pixels each, one allocation
     DevBuf<uint32_t> async_pool;
     size_t async_px = 0;
     int async_k = 0;
     unsigned long long async_batches = 0;
-    cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    bool ev_valid = false;
+    // kernel timing (ore_get_kernel_ms): ev[0..3] before each step of launch_frame, ev_end after the last (timed frames)
+    Event ev[4];
+    Marker ev_end;
     std::string err;
 
     // pinned staging (uploads and read-back)
@@ -147,8 +197,8 @@ struct ore_context {
     // the device build's launch sequence (about 65 launches, all sized from the capacity; the triangle count is read on
     // the device) captured once per buffer set and replayed on the caller's stream: enqueuing it launch by launch costs
     // the host several hundred microseconds
-    cudaGraphExec_t mesh_graph = nullptr;
-    cudaStream_t mesh_capture = nullptr;
+    GraphExec mesh_graph;
+    Stream mesh_capture;
 
     // per-frame buffers
     DevBuf<float> dx_tab;
@@ -162,8 +212,9 @@ struct ore_context {
     DevBuf<unsigned long long> counters;
     // band DMA (ORE_FLAG_BAND_DMA): packed local rows of the primary kernel + the stream / events of their copy
     DevBuf<uint32_t> band_buf;
-    cudaStream_t band_stream = nullptr;
-    cudaEvent_t ev_band_go = nullptr, ev_band_done = nullptr;
+    Stream band_stream;
+    Event ev_band_go;
+    Marker ev_band_done;
     DevBuf<float> stage;  // staging buffer between the two kernels of the default shadow pass (ore_stage_plan.h)
     size_t stage_blocks_override = 0;  // test hook (env ORE_STAGE_BLOCKS at ore_create): staging capacity in 32-item blocks
     size_t stage_max_items = (size_t)8 << 20;  // env ORE_STAGE_MAX_ITEMS: upper bound of the staging buffer in hit pixels
@@ -186,16 +237,14 @@ struct ore_context {
     };
     std::vector<GridEntry> grid_cache;
     // end of the last render on whichever stream it ran (scene setters wait for it before touching scene buffers)
-    cudaEvent_t ev_done = nullptr;
-    bool ev_done_set = false;
+    Marker ev_done;
     // end of the last stream-ordered scene update (ore_set_spheres_device, ore_set_mesh_device,
     // ore_set_mesh_triangles_device) on whichever
     // stream it ran: every render and every host setter enqueued later waits for it on the device
-    cudaEvent_t ev_scene = nullptr;
-    bool ev_scene_set = false;
+    Marker ev_scene;
     // ordered flag writes (ore_flag_write_after)
-    cudaStream_t signal_stream = nullptr;
-    cudaEvent_t ev_signal[8] = {};
+    Stream signal_stream;
+    Event ev_signal[8];
     unsigned n_signals = 0;
 
     // last frame
@@ -239,8 +288,8 @@ static int replace_buffer(ore_context* ctx, DevBuf<T>& buf, size_t n, Fill fill)
 // scene setters: the previous render may still be running on a caller-supplied stream, and a scene update on another
 // stream may still be pending (what the setter enqueues next on the render stream follows it)
 static int wait_last_render(ore_context* ctx) {
-    if (ctx->ev_done_set) ORE_CUDA(ctx, cudaEventSynchronize(ctx->ev_done));
-    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_scene, 0));
+    ORE_CUDA(ctx, ctx->ev_done.host_wait());
+    ORE_CUDA(ctx, ctx->ev_scene.stream_wait(ctx->stream));
     return ORE_OK;
 }
 
@@ -248,8 +297,8 @@ static int wait_last_render(ore_context* ctx) {
 // waits for the last render and the last update to complete.
 static int scene_idle(ore_context* ctx) {
     if (int rc = wait_last_render(ctx)) return rc;
-    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaEventSynchronize(ctx->ev_scene));
-    ctx->ev_scene_set = false;
+    ORE_CUDA(ctx, ctx->ev_scene.host_wait());
+    ctx->ev_scene.forget();
     return ORE_OK;
 }
 
@@ -268,14 +317,13 @@ static int frame_reserve(ore_context* ctx, DevBuf<T>& buf, size_t n) {
 // setter submitted later.
 static int update_begin(ore_context* ctx, void* stream, cudaStream_t* st) {
     *st = stream ? (cudaStream_t)stream : ctx->stream;
-    if (ctx->ev_done_set) ORE_CUDA(ctx, cudaStreamWaitEvent(*st, ctx->ev_done, 0));
-    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaStreamWaitEvent(*st, ctx->ev_scene, 0));
+    ORE_CUDA(ctx, ctx->ev_done.stream_wait(*st));
+    ORE_CUDA(ctx, ctx->ev_scene.stream_wait(*st));
     return ORE_OK;
 }
 
 static int update_end(ore_context* ctx, cudaStream_t st) {
-    ORE_CUDA(ctx, cudaEventRecord(ctx->ev_scene, st));
-    ctx->ev_scene_set = true;
+    ORE_CUDA(ctx, ctx->ev_scene.record(st));
     return ORE_OK;
 }
 
@@ -300,15 +348,16 @@ extern "C" int ore_create(ore_context** out, int device) {
         return fail(ctx, ORE_ERR_CUDA, b);
     }
     ctx->sm_count = prop.multiProcessorCount;
-    ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
-    ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    ORE_CUDA(ctx, cudaStreamCreateWithFlags(ctx->stream.put(), cudaStreamNonBlocking));
+    ORE_CUDA(ctx, cudaStreamCreateWithFlags(ctx->copy_stream.put(), cudaStreamNonBlocking));
     for (int i = 0; i < 2; i++) {
-        ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_rendered[i], cudaEventDisableTiming));
-        ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_copied[i], cudaEventDisableTiming));
+        ORE_CUDA(ctx, cudaEventCreateWithFlags(ctx->ev_rendered[i].put(), cudaEventDisableTiming));
+        ORE_CUDA(ctx, cudaEventCreateWithFlags(ctx->ev_copied[i].put(), cudaEventDisableTiming));
     }
-    for (int i = 0; i < 5; i++) ORE_CUDA(ctx, cudaEventCreate(&ctx->ev[i]));
-    ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_done, cudaEventDisableTiming));
-    ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_scene, cudaEventDisableTiming));
+    for (Event& e : ctx->ev) ORE_CUDA(ctx, cudaEventCreate(e.put()));
+    ORE_CUDA(ctx, cudaEventCreate(ctx->ev_end.put()));
+    ORE_CUDA(ctx, cudaEventCreateWithFlags(ctx->ev_done.put(), cudaEventDisableTiming));
+    ORE_CUDA(ctx, cudaEventCreateWithFlags(ctx->ev_scene.put(), cudaEventDisableTiming));
     ORE_CUDA(ctx, ctx->hits_hint.alloc(1));
     *ctx->hits_hint = 0;
     if (const char* e = getenv("ORE_NO_STREAM_MEMOPS")) ctx->no_memops = atoi(e) != 0;
@@ -363,31 +412,9 @@ extern "C" int ore_destroy(ore_context* ctx) {
         }
     }
     if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
-    for (int i = 0; i < 2; i++) {
-        if (ctx->ev_rendered[i]) cudaEventDestroy(ctx->ev_rendered[i]);
-        if (ctx->ev_copied[i]) cudaEventDestroy(ctx->ev_copied[i]);
-    }
-    if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-    if (ctx->ev_done) cudaEventDestroy(ctx->ev_done);
-    if (ctx->ev_scene) cudaEventDestroy(ctx->ev_scene);
-    if (ctx->mesh_graph) cudaGraphExecDestroy(ctx->mesh_graph);
-    if (ctx->mesh_capture) cudaStreamDestroy(ctx->mesh_capture);
-    if (ctx->signal_stream) {
-        cudaStreamSynchronize(ctx->signal_stream);
-        for (auto& e : ctx->ev_signal)
-            if (e) cudaEventDestroy(e);
-        cudaStreamDestroy(ctx->signal_stream);
-    }
-    if (ctx->band_stream) {
-        cudaStreamSynchronize(ctx->band_stream);
-        cudaEventDestroy(ctx->ev_band_go);
-        cudaEventDestroy(ctx->ev_band_done);
-        cudaStreamDestroy(ctx->band_stream);
-    }
-    for (int i = 0; i < 5; i++)
-        if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
-    if (ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;   // (and with it every buffer the context owns)
+    if (ctx->signal_stream) cudaStreamSynchronize(ctx->signal_stream);
+    if (ctx->band_stream) cudaStreamSynchronize(ctx->band_stream);
+    delete ctx;   // (and with it every buffer, stream, event and graph the context owns)
     return ORE_OK;
 }
 
@@ -596,8 +623,7 @@ extern "C" int ore_set_planes(ore_context* ctx, const float* pos_normal, int32_t
 // (>= 1) listed indices, with the device build's work space for tri_cap triangles (tri_cap <= INT32_MAX / TRI_FLOATS: the
 // setters check).  The caller has waited for every render and update that may use them.
 static int mesh_alloc(ore_context* ctx, size_t tri_cap, size_t box_cap, size_t idx_cap) {
-    if (ctx->mesh_graph) ORE_CUDA(ctx, cudaGraphExecDestroy(ctx->mesh_graph));   // (it holds the old buffers' addresses)
-    ctx->mesh_graph = nullptr;
+    ORE_CUDA(ctx, ctx->mesh_graph.reset());   // (it holds the old buffers' addresses)
     for (cudaError_t e : {ctx->tris.release(), ctx->boxes.release(), ctx->box_offsets.release(), ctx->box_indices.release(),
                           ctx->box_sph.release(), ctx->box_cone.release(), ctx->mesh_work.release()})
         ORE_CUDA(ctx, e);
@@ -714,19 +740,13 @@ extern "C" int ore_set_mesh_device(ore_context* ctx, const float* tris27_dev, in
     a.work = ctx->mesh_work;
     a.work_bytes = ctx->mesh_work.cap();
     if (!ctx->mesh_graph) {   // (mesh_alloc drops it with the buffers it holds)
-        if (!ctx->mesh_capture) ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->mesh_capture, cudaStreamNonBlocking));
-        cudaGraph_t g = nullptr;
+        if (!ctx->mesh_capture) ORE_CUDA(ctx, cudaStreamCreateWithFlags(ctx->mesh_capture.put(), cudaStreamNonBlocking));
+        Graph g;
         ORE_CUDA(ctx, cudaStreamBeginCapture(ctx->mesh_capture, cudaStreamCaptureModeThreadLocal));
         const cudaError_t eb = ore_mesh_build(a, ctx->mesh_capture);
-        const cudaError_t ec = cudaStreamEndCapture(ctx->mesh_capture, &g);
-        if (eb != cudaSuccess || ec != cudaSuccess) {
-            if (g) cudaGraphDestroy(g);
-            ORE_CUDA(ctx, eb != cudaSuccess ? eb : ec);
-        }
-        const cudaError_t ei = cudaGraphInstantiate(&ctx->mesh_graph, g, 0);
-        cudaGraphDestroy(g);
-        if (ei != cudaSuccess) ctx->mesh_graph = nullptr;
-        ORE_CUDA(ctx, ei);
+        const cudaError_t ec = cudaStreamEndCapture(ctx->mesh_capture, g.put());
+        ORE_CUDA(ctx, eb != cudaSuccess ? eb : ec);
+        ORE_CUDA(ctx, cudaGraphInstantiate(ctx->mesh_graph.put(), g, 0));
     }
     ORE_CUDA(ctx, ore_mesh_build_count(a, n_tris, st));
     ORE_CUDA(ctx, cudaGraphLaunch(ctx->mesh_graph, st));
@@ -1044,7 +1064,7 @@ static int launch_frame(ore_context* ctx, const FrameParams& prm, size_t psmem, 
         ctx->last_launches++;
     }
     if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[2], stream));
-    bool band_pending = false;
+    ctx->ev_band_done.forget();   // (recorded below when this frame copies its rows)
     if (band_dma) {
         // the rows the primary kernel has just written (sky pixels, 0 for hit pixels) travel to their place in the
         // destination frames on a copy engine, behind the primary kernel and concurrently with stage A of the shadow
@@ -1055,14 +1075,11 @@ static int launch_frame(ore_context* ctx, const FrameParams& prm, size_t psmem, 
             if ((rc = copy_row_blocks(ctx, outs[f], ctx->band_buf + (size_t)f * prm.n_px_frame, prm.W, prm.n_rows, prm.y_block,
                                       prm.y_step, cudaMemcpyDefault, ctx->band_stream)))
                 return rc;
-        ORE_CUDA(ctx, cudaEventRecord(ctx->ev_band_done, ctx->band_stream));
-        band_pending = true;
+        ORE_CUDA(ctx, ctx->ev_band_done.record(ctx->band_stream));
     }
-    auto join_band = [&]() -> int {
-        if (band_pending) {
-            ORE_CUDA(ctx, cudaStreamWaitEvent(stream, ctx->ev_band_done, 0));
-            band_pending = false;
-        }
+    auto join_band = [&]() -> int {   // (the first call waits for the copy, later ones do nothing)
+        ORE_CUDA(ctx, ctx->ev_band_done.stream_wait(stream));
+        ctx->ev_band_done.forget();
         return ORE_OK;
     };
     // Two-stage pass (default): shade_setup_kernel -> staging buffer -> staged shadow_sweep_kernel, in the chunk pairs of
@@ -1125,10 +1142,8 @@ static int launch_frame(ore_context* ctx, const FrameParams& prm, size_t psmem, 
         ORE_CUDA(ctx, cudaGetLastError());
         ctx->last_launches++;
     }
-    if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[4], stream));
-    ctx->ev_valid = timing;
-    ORE_CUDA(ctx, cudaEventRecord(ctx->ev_done, stream));
-    ctx->ev_done_set = true;
+    if (timing) ORE_CUDA(ctx, ctx->ev_end.record(stream));
+    ORE_CUDA(ctx, ctx->ev_done.record(stream));
     return ORE_OK;
 }
 
@@ -1164,13 +1179,13 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
     ctx->last_frames = n_frames;
     ctx->last_n_spheres = ctx->n_spheres;
     ctx->last_launches = 0;
-    ctx->ev_valid = false;
+    ctx->ev_end.forget();
     ctx->last_prm_valid = false;
     if (n_px == 0) return ORE_OK;
     for (int f = 0; outs && f < n_frames; f++)
         if (!outs[f]) return fail(ctx, ORE_ERR_INVALID, "ore_render: null framebuffer in the batch");
     // the scene of the last stream-ordered update, wherever it ran
-    if (ctx->ev_scene_set) ORE_CUDA(ctx, cudaStreamWaitEvent(stream, ctx->ev_scene, 0));
+    ORE_CUDA(ctx, ctx->ev_scene.stream_wait(stream));
 
     int rc;
     if ((rc = frame_reserve(ctx, ctx->dx_tab, (size_t)((W + 31) & ~31)))) return rc;
@@ -1184,10 +1199,10 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
     const bool band_dma = outs && fr->out_pitch == W && (fr->flags & ORE_FLAG_BAND_DMA) != 0;
     if (band_dma) {
         if ((rc = frame_reserve(ctx, ctx->band_buf, n_px))) return rc;
-        if (!ctx->band_stream) {
-            ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->band_stream, cudaStreamNonBlocking));
-            ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_band_go, cudaEventDisableTiming));
-            ORE_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_band_done, cudaEventDisableTiming));
+        if (!ctx->band_stream) {   // (the stream last: it marks the group as made)
+            ORE_CUDA(ctx, cudaEventCreateWithFlags(ctx->ev_band_go.put(), cudaEventDisableTiming));
+            ORE_CUDA(ctx, cudaEventCreateWithFlags(ctx->ev_band_done.put(), cudaEventDisableTiming));
+            ORE_CUDA(ctx, cudaStreamCreateWithFlags(ctx->band_stream.put(), cudaStreamNonBlocking));
         }
     }
     size_t psmem = 0;
@@ -1238,19 +1253,20 @@ extern "C" int ore_render(ore_context* ctx, const ore_camera* cam, const ore_fra
 // ---- stream-ordered 32-bit flags (cuStreamWriteValue32 / cuStreamWaitValue32, no SM involved) ----------------
 // The driver entry points are resolved at run time (the library links against cudart only).
 typedef int (*ore_cu_memop32)(cudaStream_t, unsigned long long /*CUdeviceptr*/, unsigned int, unsigned int);
-static ore_cu_memop32 cu_write32 = nullptr, cu_wait32 = nullptr;
-static bool memops_resolved = false;
-static void resolve_memops() {
-    if (memops_resolved) return;
-    memops_resolved = true;
+static ore_cu_memop32 driver_memop(const char* name) {   // null when the driver does not offer it
     void* f = nullptr;
     cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuStreamWriteValue32", &f, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-        cu_write32 = (ore_cu_memop32)f;
-    f = nullptr;
-    if (cudaGetDriverEntryPoint("cuStreamWaitValue32", &f, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-        cu_wait32 = (ore_cu_memop32)f;
+    const bool ok = cudaGetDriverEntryPoint(name, &f, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess;
     (void)cudaGetLastError();
+    return ok ? (ore_cu_memop32)f : nullptr;
+}
+struct MemOps {
+    ore_cu_memop32 write32, wait32;
+};
+// resolved by the first flag call of the process (a function-local static: initialised once, thread-safely)
+static const MemOps& memops() {
+    static const MemOps m{driver_memop("cuStreamWriteValue32"), driver_memop("cuStreamWaitValue32")};
+    return m;
 }
 
 // fallbacks on an SM: one thread.  The wait kernel is only ever used when the driver offers no stream wait; it
@@ -1272,14 +1288,14 @@ static cudaStream_t pick_stream(ore_context* ctx, void* stream) { return stream 
 
 extern "C" void* ore_get_stream(ore_context* ctx, int which) {
     if (!ctx) return nullptr;
-    if (which == 2) return (void*)ctx->signal_stream;  // null until the first ore_flag_write_after
-    return which == 1 ? (void*)ctx->copy_stream : (void*)ctx->stream;
+    if (which == 2) return (cudaStream_t)ctx->signal_stream;  // null until the first ore_flag_write_after
+    return which == 1 ? (cudaStream_t)ctx->copy_stream : (cudaStream_t)ctx->stream;
 }
 
 extern "C" int ore_flag_write(ore_context* ctx, void* stream, uint32_t* flag, uint32_t value) {
     if (!ctx || !flag) return ORE_ERR_INVALID;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
-    resolve_memops();
+    const ore_cu_memop32 cu_write32 = memops().write32;
     cudaStream_t st = pick_stream(ctx, stream);
     // peer-mapped device memory (another GPU's flag, imported with ore_ipc_import) is written by a one-thread
     // kernel (st.release.sys over NVLink); local device memory and registered host memory by the stream itself
@@ -1304,11 +1320,11 @@ extern "C" int ore_flag_write(ore_context* ctx, void* stream, uint32_t* flag, ui
 extern "C" int ore_flag_write_after(ore_context* ctx, void* stream, uint32_t* flag, uint32_t value) {
     if (!ctx || !flag) return ORE_ERR_INVALID;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (!ctx->signal_stream) {
-        ORE_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->signal_stream, cudaStreamNonBlocking));
-        for (auto& e : ctx->ev_signal) ORE_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    if (!ctx->signal_stream) {   // (the stream last: it marks the group as made)
+        for (Event& e : ctx->ev_signal) ORE_CUDA(ctx, cudaEventCreateWithFlags(e.put(), cudaEventDisableTiming));
+        ORE_CUDA(ctx, cudaStreamCreateWithFlags(ctx->signal_stream.put(), cudaStreamNonBlocking));
     }
-    cudaEvent_t e = ctx->ev_signal[ctx->n_signals++ % 8];
+    const Event& e = ctx->ev_signal[ctx->n_signals++ % 8];
     ORE_CUDA(ctx, cudaEventRecord(e, pick_stream(ctx, stream)));
     ORE_CUDA(ctx, cudaStreamWaitEvent(ctx->signal_stream, e, 0));
     return ore_flag_write(ctx, ctx->signal_stream, flag, value);
@@ -1317,7 +1333,7 @@ extern "C" int ore_flag_write_after(ore_context* ctx, void* stream, uint32_t* fl
 extern "C" int ore_flag_wait_geq(ore_context* ctx, void* stream, const uint32_t* flag, uint32_t value) {
     if (!ctx || !flag) return ORE_ERR_INVALID;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
-    resolve_memops();
+    const ore_cu_memop32 cu_wait32 = memops().wait32;
     cudaStream_t st = pick_stream(ctx, stream);
     cudaPointerAttributes at;
     void* dptr = (void*)flag;
@@ -1537,10 +1553,11 @@ extern "C" int ore_get_counters(ore_context* ctx, ore_counters* out) {
 extern "C" int ore_get_kernel_ms(ore_context* ctx, float ms[4]) {
     if (!ctx || !ms) return ORE_ERR_INVALID;
     ms[0] = ms[1] = ms[2] = ms[3] = 0.f;
-    if (!ctx->ev_valid) return ORE_OK;
+    if (!ctx->ev_end.recorded()) return ORE_OK;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
-    ORE_CUDA(ctx, cudaEventSynchronize(ctx->ev[4]));
-    for (int i = 0; i < 4; i++) ORE_CUDA(ctx, cudaEventElapsedTime(&ms[i], ctx->ev[i], ctx->ev[i + 1]));
+    ORE_CUDA(ctx, ctx->ev_end.host_wait());
+    for (int i = 0; i < 4; i++)
+        ORE_CUDA(ctx, cudaEventElapsedTime(&ms[i], ctx->ev[i], i < 3 ? (cudaEvent_t)ctx->ev[i + 1] : ctx->ev_end.event()));
     return ORE_OK;
 }
 
@@ -1595,24 +1612,18 @@ extern "C" int ore_measure_fp32_peak(ore_context* ctx, double* tflops, double* s
     DevBuf<float> d;
     ORE_CUDA(ctx, d.alloc(1));
     const int iters = 4096, grid = ctx->sm_count * 8;
-    struct Events {   // (destroyed on every path out)
-        cudaEvent_t a = nullptr, b = nullptr;
-        ~Events() {
-            if (a) cudaEventDestroy(a);
-            if (b) cudaEventDestroy(b);
-        }
-    } ev;
-    ORE_CUDA(ctx, cudaEventCreate(&ev.a));
-    ORE_CUDA(ctx, cudaEventCreate(&ev.b));
+    Event a, b;
+    ORE_CUDA(ctx, cudaEventCreate(a.put()));
+    ORE_CUDA(ctx, cudaEventCreate(b.put()));
     double best = 0.0;
     for (int rep = 0; rep < 6; rep++) {
-        ORE_CUDA(ctx, cudaEventRecord(ev.a, ctx->stream));
+        ORE_CUDA(ctx, cudaEventRecord(a, ctx->stream));
         fp32_burn_kernel<<<grid, CTA_THREADS, 0, ctx->stream>>>(d, iters, 1.0000001f, 1e-9f);
         ORE_CUDA(ctx, cudaGetLastError());
-        ORE_CUDA(ctx, cudaEventRecord(ev.b, ctx->stream));
-        ORE_CUDA(ctx, cudaEventSynchronize(ev.b));
+        ORE_CUDA(ctx, cudaEventRecord(b, ctx->stream));
+        ORE_CUDA(ctx, cudaEventSynchronize(b));
         float ms = 0.f;
-        ORE_CUDA(ctx, cudaEventElapsedTime(&ms, ev.a, ev.b));
+        ORE_CUDA(ctx, cudaEventElapsedTime(&ms, a, b));
         const double flop = 2.0 * 16 * 8 * (double)iters * CTA_THREADS * (double)grid;
         const double tf = flop / (ms * 1e-3) / 1e12;
         if (rep >= 1 && tf > best) best = tf;
