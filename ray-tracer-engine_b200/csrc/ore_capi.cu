@@ -1569,12 +1569,15 @@ extern "C" int ore_debug_libm(ore_context* ctx, int op, int n, const float* a_ho
     ORE_CUDA(ctx, a.alloc(n));
     ORE_CUDA(ctx, b.alloc(n));
     ORE_CUDA(ctx, o.alloc(n));
-    ORE_CUDA(ctx, cudaMemcpy(a, a_host, bytes, cudaMemcpyHostToDevice));
-    ORE_CUDA(ctx, cudaMemcpy(b, b_host ? b_host : a_host, bytes, cudaMemcpyHostToDevice));
+    // every copy on the kernel's stream: a plain cudaMemcpy from pageable memory may return before its DMA has landed,
+    // and ctx->stream (non-blocking) does not wait for the legacy stream - the kernel could read part of the inputs
+    // before they arrive
+    ORE_CUDA(ctx, cudaMemcpyAsync(a, a_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    ORE_CUDA(ctx, cudaMemcpyAsync(b, b_host ? b_host : a_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
     libm_probe_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(op, n, a, b, o);
     ORE_CUDA(ctx, cudaGetLastError());
+    ORE_CUDA(ctx, cudaMemcpyAsync(out_host, o, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     ORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    ORE_CUDA(ctx, cudaMemcpy(out_host, o, bytes, cudaMemcpyDeviceToHost));
     return ORE_OK;
 }
 

@@ -13,7 +13,9 @@
 //   atan2f : 2*10^9 random pairs (half unit-vector components) - 0 mismatches
 //   sinf, cosf : all floats with |x| < 120, both signs       - 0 mismatches (glibc's FMA ifunc variant)
 // |x| >= 120 (never produced by the path: arguments are 2*dot(unit,unit) and acosf results) falls back to CUDA's.
-// tests/test_parity_gpu.py re-checks a random sample against the host libm on the GPU box.
+// (abstop12 compares sign, exponent and 3 mantissa bits: the sinf/cosf branches actually split at 0x1p-12, 0x1.9p-1
+// and 120.)  tests/golden/libm_kat.npz keeps glibc's answers at every threshold and special case of the four functions;
+// tests/test_parity_gpu.py holds the device to them.
 //
 // Algorithms:
 //  * acosf, atanf, atan2f: FreeBSD/Sun fdlibm float versions (e_acosf.c, s_atanf.c, e_atan2f.c):
