@@ -1159,6 +1159,10 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
     if (fr->width <= 0 || fr->height <= 0 || fr->y_step <= 0 || fr->y0 < 0 || fr->y1 < 0 || fr->y1 > fr->height ||
         (fr->out_pitch != 0 && fr->out_pitch < fr->width))
         return fail(ctx, ORE_ERR_INVALID, "ore_render: bad frame geometry");
+    // the eye sits 1/aspect behind the image plane (kernel.cu:1629): 0, +-inf, NaN and aspects whose reciprocal
+    // overflows give no finite eye and are rejected before anything renders
+    if (!std::isfinite(fr->aspect) || !std::isfinite(1.f / fr->aspect))
+        return fail(ctx, ORE_ERR_INVALID, "ore_render: aspect must be finite and non-zero, with a finite 1/aspect");
     if (fr->flags & ~(uint32_t)(ORE_FLAG_EXHAUSTIVE | ORE_FLAG_COUNT_REFERENCE_TESTS | ORE_FLAG_FAST_LIBM | ORE_FLAG_FUSED_SHADOW |
                                 ORE_FLAG_NO_KERNEL_TIMING | ORE_FLAG_BAND_DMA))
         return fail(ctx, ORE_ERR_INVALID, "ore_render: unknown flag");

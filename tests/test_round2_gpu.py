@@ -437,26 +437,27 @@ def _index_sky(pkg, w, h):
     return pkg.scene.Sprite(width=w, height=h, r=chan(i // 65025), g=chan((i // 255) % 255), b=chan(i % 255))
 
 
+RA = float(np.float32(math.tan((90 * 0.5 * 3.1415) / 180)))   # scene.REFERENCE_ASPECT
 SKY_CASES = [
-    # (sky w, h, sky size, camera org, yaw, pitch)
-    (1024, 512, 10000.0, (4.0, 3.0, 10.0), 180.0, -20.0),       # the reference's camera
-    (1024, 512, 10000.0, (4.0, 3.0, 10.0), 37.0, 88.5),         # a pole in view
-    (1024, 512, 10000.0, (4.0, 3.0, 10.0), 200.0, -89.0),       # the other pole
-    (300, 200, 10000.0, (-3.0, 12.0, 2.0), 301.0, 10.0),        # odd texture size
-    (4096, 2048, 10000.0, (4.0, 3.0, 10.0), 90.0, 0.0),         # texels smaller than pixels
-    (1024, 512, 10000.0, (3.0e7, 1.0e7, -2.0e7), 10.0, 5.0),    # camera a third of the way to the sky sphere
-    (1024, 512, 10000.0, (6.0e7, 0.0, 0.0), 10.0, 5.0),         # |O| > R/2: the shortcut must stand down
-    (512, 256, 3.0, (4.0, 3.0, 10.0), 180.0, -20.0),            # tiny sky sphere: camera outside it (NaN roots)
-    (512, 256, 0.5, (0.1, 0.0, 0.05), 45.0, 30.0),              # R^2 < 1
+    # (sky w, h, sky size, camera org, yaw, pitch, aspect); other fields of view: tests/test_view_geometry_gpu.py
+    (1024, 512, 10000.0, (4.0, 3.0, 10.0), 180.0, -20.0, RA),       # the reference's camera
+    (1024, 512, 10000.0, (4.0, 3.0, 10.0), 37.0, 88.5, RA),         # a pole in view
+    (1024, 512, 10000.0, (4.0, 3.0, 10.0), 200.0, -89.0, RA),       # the other pole
+    (300, 200, 10000.0, (-3.0, 12.0, 2.0), 301.0, 10.0, RA),        # odd texture size
+    (4096, 2048, 10000.0, (4.0, 3.0, 10.0), 90.0, 0.0, RA),         # texels smaller than pixels
+    (1024, 512, 10000.0, (3.0e7, 1.0e7, -2.0e7), 10.0, 5.0, RA),    # camera a third of the way to the sky sphere
+    (1024, 512, 10000.0, (6.0e7, 0.0, 0.0), 10.0, 5.0, RA),         # |O| > R/2: the shortcut must stand down
+    (512, 256, 3.0, (4.0, 3.0, 10.0), 180.0, -20.0, RA),            # tiny sky sphere: camera outside it (NaN roots)
+    (512, 256, 0.5, (0.1, 0.0, 0.05), 45.0, 30.0, RA),              # R^2 < 1
 ]
 
 
 @pytest.mark.parametrize("case", range(len(SKY_CASES)))
 def test_sky_texel_shortcut_equals_the_oracle_with_an_index_encoding_sky(case, renderer, oracle_best, pkg, libm_matches):
-    w, h, size, org, yaw, pitch = SKY_CASES[case]
+    w, h, size, org, yaw, pitch, aspect = SKY_CASES[case]
     base = pkg.scene.reference_scene(64, 1)
     sc = pkg.scene.Scene(spheres=base.spheres, lights=base.lights, texture=base.texture, sky=_index_sky(pkg, w, h),
-                         sky_size=size, extent=base.extent, name=f"index_sky_{case}")
+                         sky_size=size, aspect=np.float32(aspect), extent=base.extent, name=f"index_sky_{case}")
     cam = pkg.scene.Camera(org=org, yaw=yaw, pitch=pitch)
     W, H = 333, 187
     F = pkg.capi

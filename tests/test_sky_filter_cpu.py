@@ -7,6 +7,7 @@ import os
 import re
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = open(os.path.join(ROOT, "ray-tracer-engine_b200", "csrc", "ore_primary.cuh")).read()
@@ -144,3 +145,33 @@ def test_sky_fast_never_accepts_a_wrong_texel():
         total += n
         accepted += int(ok.sum())
     assert accepted > 0.5 * total, (accepted, total)     # and it is useful: most pixels are decided by the shortcut
+
+
+REF_ASPECT = float(f32(np.tan(90 * 0.5 * 3.1415 / 180)))
+ASPECTS = [1e-3, 0.02, 0.35, REF_ASPECT, 1.7, 4.0, 25.0, 1e3, -REF_ASPECT]
+
+
+@pytest.mark.parametrize("aspect", ASPECTS, ids=[f"{a:g}" for a in ASPECTS])
+def test_sky_fast_never_accepts_a_wrong_texel_at_other_fields_of_view(aspect):
+    """the image-plane coordinates the reference really produces at this field of view (kernel.cu:1624-1625):
+    dx in [-1, 2 aspect - 1], dy in [-1, 2 aspect H/W - 1], fz = 1/aspect (negative: the view looks backwards)"""
+    rng = np.random.default_rng(int(1000 + 7 * ASPECTS.index(aspect)))
+    a = f32(aspect)
+    fz = f32(0) - (f32(-1) / a)
+    hw = 0.5625                                                    # a 16:9 frame
+    total = accepted = 0
+    for it in range(24):
+        w, h = [(1024, 512), (300, 200), (4096, 2048)][it % 3]
+        size = [10000.0, 10000.0, 30.0, 1e3][it % 4]
+        extent = [30.0, 2000.0, 5.0, 100.0][it % 4]
+        cam, O = _camera(rng, extent)
+        n = 20000
+        dx = (np.float64(a) * rng.uniform(0, 2, n) - 1).astype(f32)
+        dy = (np.float64(a) * rng.uniform(0, 2, n) * hw - 1).astype(f32)
+        ok, idx = sky_fast(dx, dy, fz, cam, O, size * size, w, h)
+        ref = exact_index(dx, dy, fz, cam, O, size * size, w, h)
+        bad = ok & (idx != ref)
+        assert not bad.any(), (aspect, it, int(bad.sum()), w, h, size, O)
+        total += n
+        accepted += int(ok.sum())
+    assert accepted > 0.5 * total, (accepted, total)
