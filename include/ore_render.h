@@ -135,7 +135,11 @@ const char* ore_last_error(const ore_context* ctx); /* "" if none */
  * into structure-of-arrays device buffers; the caller's memory is not retained. */
 
 /* Replaces object::sphereAllocMem (kernel.cu:1208-1212): n records of cx,cy,cz and the
- * stored `radius` MEMBER (= ctor r*r, kernel.cu:287; squared again in the test :334). */
+ * stored `radius` MEMBER (= ctor r*r, kernel.cu:287; squared again in the test :334).
+ * Sphere counts: the setters accept any n >= 0; a render accepts scenes of up to 2^24 = 16 777 216 spheres and returns
+ * ORE_ERR_INVALID, writing nothing, above that.  Scenes of 99 073 spheres and more get a fourth level of the sphere
+ * hierarchy (hyper-clusters of 8192 spheres) and the large-scene kernels; the results are the same either way.  The
+ * environment variable ORE_LARGE_SCENE_MIN_SPHERES, read by ore_create, lowers that threshold (tests). */
 int ore_set_spheres(ore_context* ctx, const float* xyz_radius, int32_t n);
 /* Same, from the reference's own 32-byte AoS records (vptr@0, orgin@8, reflective@20,
  * radius@24; `sizeof(float)*8` per sphere, kernel.cu:1218-1220). */
@@ -312,8 +316,10 @@ int ore_debug_libm(ore_context* ctx, int op, int n, const float* a_host, const f
 /* Tests only: synchronises the device and copies one array of the sphere hierarchy to the host.  which: 0 records in
  * original order (max(n, 1) float4), 1 exact records sorted (n_sort float4), 2 shadow records cx,cy,cz,R' sorted
  * (n_sort float4), 3 sorted position -> original index (n_sort int32), 4 leaf balls (n_leaves_pad float4), 5 super-
- * cluster balls (n_supers_pad float4); n_sort = 32 ceil(n / 32) (32 when n = 0), n_leaves_pad = ceil(n / 8) rounded up
- * to a multiple of 32, n_supers_pad = ceil(n / 256) rounded up to a multiple of 4.  n_items must be that length. */
+ * cluster balls (n_supers_pad float4), 6 hyper-cluster balls (n_hypers_pad float4; ORE_ERR_INVALID when the scene
+ * has no hyper level, i.e. is not a large scene: see ore_set_spheres); n_sort = 32 ceil(n / 32) (32 when n = 0),
+ * n_leaves_pad = ceil(n / 8) rounded up to a multiple of 32, n_supers_pad = ceil(n / 256) rounded up to a multiple of 4,
+ * n_hypers_pad = ceil(n / 8192) rounded up to a multiple of 4.  n_items must be that length. */
 int ore_debug_sphere_tree(ore_context* ctx, int32_t which, void* host_out, int32_t n_items);
 /* Tests only: synchronises the device and copies one array of the mesh to the host.  which: 0 triangles (n_tris * 27
  * floats), 1 leaf boxes lo, hi (2 * n_boxes float4, .w = 0), 2 leaf bounding spheres (n_boxes float4), 3 leaf offsets

@@ -34,7 +34,8 @@ EXPORTS = [
 ]
 
 # ore_debug_sphere_tree: which array of the sphere hierarchy, and its element type
-SPHERE_TREE_ARRAYS = {"sph_exact": 0, "sph_xsort": 1, "sph_sort": 2, "sort_index": 3, "leaf_sph": 4, "super_sph": 5}
+SPHERE_TREE_ARRAYS = {"sph_exact": 0, "sph_xsort": 1, "sph_sort": 2, "sort_index": 3, "leaf_sph": 4, "super_sph": 5,
+                      "hyper": 6}   # (hyper: large scenes only)
 
 
 # ore_debug_mesh: which array of the mesh
@@ -45,12 +46,14 @@ MESH_MAX_LEAVES = 1024
 
 
 def sphere_tree_lengths(n: int) -> dict:
-    """item counts of the six hierarchy arrays for n spheres (include/ore_render.h, ore_debug_sphere_tree)"""
+    """item counts of the hierarchy arrays for n spheres (include/ore_render.h, ore_debug_sphere_tree); "hyper" exists
+    only in a large scene"""
     n_sort = max(1, (n + 31) // 32) * 32
     n_leaf = (n + 7) // 8
     n_sup = (n_leaf + 31) // 32
+    n_hyp = (n_sup + 31) // 32
     return {"sph_exact": max(n, 1), "sph_xsort": n_sort, "sph_sort": n_sort, "sort_index": n_sort,
-            "leaf_sph": (n_leaf + 31) // 32 * 32, "super_sph": (n_sup + 3) // 4 * 4}
+            "leaf_sph": (n_leaf + 31) // 32 * 32, "super_sph": (n_sup + 3) // 4 * 4, "hyper": (n_hyp + 3) // 4 * 4}
 
 
 class OreCamera(C.Structure):

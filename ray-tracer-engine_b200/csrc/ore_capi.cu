@@ -11,6 +11,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <string>
 #include <algorithm>
 #include <utility>
@@ -127,6 +128,13 @@ private:
 
 }  // namespace
 
+// Scenes from this many spheres on take the large-scene path: the primary kernel's shared-memory copy of the leaf and
+// super-cluster records, (n_leaves_pad + n_supers_pad) x 16 bytes, would pass 200 KB at 99 073 spheres.
+static constexpr int LARGE_SCENE_MIN_SPHERES = 99073;
+// The largest scene a render accepts: the per-frame sphere records (prim_sorted, cone_sorted: MAX_BATCH frames of 16 bytes
+// per sphere each) come to 4 GiB there, and the hyper-cluster records of a frame to 32 KB of shared memory.
+static constexpr int MAX_RENDER_SPHERES = 1 << 24;
+
 struct ore_context {
     // (frees every buffer, stream, event and graph below; not an export of the library)
     __attribute__((visibility("hidden"))) ~ore_context() = default;
@@ -164,6 +172,12 @@ struct ore_context {
     DevBuf<float4> leaf_cone;
     DevBuf<float4> super_cone;
     int n_sort = 0, n_leaves = 0, n_leaves_pad = 0, n_supers = 0, n_supers_pad = 0;
+    // large scenes (n >= large_min) only: a fourth level of hyper-cluster balls over 32 supers each, and their per-frame
+    // records; the render then runs the LARGE kernel instantiations.  n_hypers_pad = 0: the scene has no hyper level.
+    DevBuf<float4> hyper_sph;
+    DevBuf<float4> hyper_cone;
+    int n_hypers = 0, n_hypers_pad = 0;
+    int large_min = LARGE_SCENE_MIN_SPHERES;   // env ORE_LARGE_SCENE_MIN_SPHERES (tests: the large path on small scenes)
     // work space of the device build of the hierarchy (ore_scene_build.cu), sized with the scene buffers
     DevBuf<uint32_t> keys_in;
     DevBuf<uint32_t> keys_out;
@@ -370,6 +384,10 @@ extern "C" int ore_create(ore_context** out, int device) {
         const long v = atol(e);
         if (v > 0) ctx->stage_blocks_override = (size_t)v;
     }
+    if (const char* e = getenv("ORE_LARGE_SCENE_MIN_SPHERES")) {   // (only ever lowers the threshold)
+        const long v = atol(e);
+        if (v >= 1 && v < LARGE_SCENE_MIN_SPHERES) ctx->large_min = (int)v;
+    }
     ORE_CUDA(ctx, ctx->counters.alloc(CNT_SLOTS));
     ORE_CUDA(ctx, cudaMemset(ctx->counters, 0, CNT_SLOTS * sizeof(unsigned long long)));
     // kernel.cu:1454,1462-1463: phi = (float)j/10 * 2.f * 3.1415f; cosf(phi), sinf(phi)
@@ -427,20 +445,26 @@ extern "C" int ore_destroy(ore_context* ctx) {
 // (t, original index)).  The hierarchy is built on the device (ore_scene_build.cu) for both setters; the host builder
 // of ore_clusters.h is its CPU reference (tests/test_clusters_cpu.py, tests/test_scene_update_gpu.py).
 
-static void scene_sizes(int32_t n, size_t* n_sort, size_t* n_leaf_pad, size_t* n_sup_pad) {
+static void scene_sizes(int32_t n, size_t* n_sort, size_t* n_leaf_pad, size_t* n_sup_pad, size_t* n_hyp_pad) {
     const size_t n_clu = ((size_t)n + 31) / 32;
     *n_sort = n > 0 ? n_clu * 32 : 32;   // empty scene: one block of padding records
     const size_t n_leaf = ((size_t)n + ore_host::LEAF_SPHERES - 1) / ore_host::LEAF_SPHERES;
     const size_t n_sup = (n_leaf + ore_host::SUPER_LEAVES - 1) / ore_host::SUPER_LEAVES;
+    const size_t n_hyp = (n_sup + ore_host::HYPER_SUPERS - 1) / ore_host::HYPER_SUPERS;
     *n_leaf_pad = (n_leaf + 31) & ~(size_t)31;
     *n_sup_pad = (n_sup + 3) & ~(size_t)3;
+    *n_hyp_pad = (n_hyp + 3) & ~(size_t)3;
 }
+
+// the scene takes the large-scene path (hyper level, LARGE kernels); decided once per scene by the setters
+static bool large_scene(const ore_context* ctx, int32_t n) { return n > 0 && n >= ctx->large_min; }
 
 // Capacity of the scene buffers and of the build's work space for n spheres.  Only growth blocks the host: the old
 // buffers may still be read by a render or written by an update on another stream, so both are waited for first.
 static int scene_reserve(ore_context* ctx, int32_t n) {
-    size_t n_sort, n_leaf_pad, n_sup_pad;
-    scene_sizes(n, &n_sort, &n_leaf_pad, &n_sup_pad);
+    size_t n_sort, n_leaf_pad, n_sup_pad, n_hyp_pad;
+    scene_sizes(n, &n_sort, &n_leaf_pad, &n_sup_pad, &n_hyp_pad);
+    const bool large = large_scene(ctx, n);
     size_t tmp_bytes = 0;
     ORE_CUDA(ctx, ore_scene_sort_bytes(n, &tmp_bytes));
     const size_t n_ex = (size_t)std::max(n, 1), nb = MAX_BATCH;   // (camera-space records: one set per frame of a batch)
@@ -450,7 +474,8 @@ static int scene_reserve(ore_context* ctx, int32_t n) {
                op(ctx->prim_sorted, n_sort * nb) && op(ctx->cone_sorted, n_sort * nb) && op(ctx->leaf_sph, n_leaf_pad) &&
                op(ctx->leaf_cone, n_leaf_pad * nb) && op(ctx->super_sph, n_sup_pad) && op(ctx->super_cone, n_sup_pad * nb) &&
                op(ctx->keys_in, (size_t)n) && op(ctx->keys_out, (size_t)n) && op(ctx->vals_in, (size_t)n) &&
-               op(ctx->vals_out, (size_t)n) && op(ctx->bbox, (size_t)6);
+               op(ctx->vals_out, (size_t)n) && op(ctx->bbox, (size_t)6) &&
+               (!large || (op(ctx->hyper_sph, n_hyp_pad) && op(ctx->hyper_cone, n_hyp_pad * nb)));
     };
     if (each([](auto& buf, size_t k) { return buf.fits(k); }) && ctx->sort_tmp.fits(tmp_bytes)) return ORE_OK;
     if (int rc = scene_idle(ctx)) return rc;
@@ -466,8 +491,9 @@ static int scene_reserve(ore_context* ctx, int32_t n) {
 // Enqueues the device build of the hierarchy over the n records at src (device memory; may be sph_exact itself) on
 // `stream` and sets the scene's counts.  Capacity comes from scene_reserve.
 static int scene_enqueue(ore_context* ctx, const float4* src, int32_t n, cudaStream_t stream) {
-    size_t n_sort, n_leaf_pad, n_sup_pad;
-    scene_sizes(n, &n_sort, &n_leaf_pad, &n_sup_pad);
+    size_t n_sort, n_leaf_pad, n_sup_pad, n_hyp_pad;
+    scene_sizes(n, &n_sort, &n_leaf_pad, &n_sup_pad, &n_hyp_pad);
+    const bool large = large_scene(ctx, n);
     SceneBuildArgs a;
     a.src = src;
     a.n = n;
@@ -482,6 +508,9 @@ static int scene_enqueue(ore_context* ctx, const float4* src, int32_t n, cudaStr
     a.n_leaves_pad = (int)n_leaf_pad;
     a.n_supers = (a.n_leaves + ore_host::SUPER_LEAVES - 1) / ore_host::SUPER_LEAVES;
     a.n_supers_pad = (int)n_sup_pad;
+    a.hyper_sph = large ? (float4*)ctx->hyper_sph : nullptr;
+    a.n_hypers = large ? (a.n_supers + ore_host::HYPER_SUPERS - 1) / ore_host::HYPER_SUPERS : 0;
+    a.n_hypers_pad = large ? (int)n_hyp_pad : 0;
     a.keys_in = ctx->keys_in;
     a.keys_out = ctx->keys_out;
     a.vals_in = ctx->vals_in;
@@ -496,6 +525,8 @@ static int scene_enqueue(ore_context* ctx, const float4* src, int32_t n, cudaStr
     ctx->n_leaves_pad = a.n_leaves_pad;
     ctx->n_supers = a.n_supers;
     ctx->n_supers_pad = a.n_supers_pad;
+    ctx->n_hypers = a.n_hypers;
+    ctx->n_hypers_pad = a.n_hypers_pad;
     return ORE_OK;
 }
 
@@ -836,6 +867,31 @@ static constexpr int TILE_ROWS = TILE_P;   // rows per tile of the primary kerne
 // everything stays within this budget (6 CTAs of 128 threads per SM)
 static constexpr size_t PRIMARY_RESIDENT_BYTES = 30 * 1024;
 
+// The opt-in dynamic shared-memory limit of a kernel (cudaFuncAttributeMaxDynamicSharedMemorySize) belongs to the kernel
+// on a device, not to a context: every context of the process shares it.  It therefore only ever grows, per (device,
+// kernel) and process-wide, so that a configuration any context has cached stays launchable whatever another context
+// asks for later.
+static cudaError_t raise_smem_limit(int device, const void* fn, size_t smem) {
+    struct Limit {
+        int device;
+        const void* fn;
+        size_t smem;
+    };
+    static std::mutex mu;
+    static std::vector<Limit> limits;
+    std::lock_guard<std::mutex> lock(mu);
+    for (Limit& l : limits)
+        if (l.device == device && l.fn == fn) {
+            if (l.smem >= smem) return cudaSuccess;
+            const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e == cudaSuccess) l.smem = smem;
+            return e;
+        }
+    const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) limits.push_back({device, fn, smem});
+    return e;
+}
+
 template <typename K>
 static int grid_for(ore_context* ctx, K kernel, size_t smem, int* grid, int threads = CTA_THREADS) {
     const void* fn = reinterpret_cast<const void*>(kernel);
@@ -845,11 +901,7 @@ static int grid_for(ore_context* ctx, K kernel, size_t smem, int* grid, int thre
             return ORE_OK;
         }
     int occ = 0;
-    // the opt-in limit only ever grows, so that earlier (cached) configurations of this kernel stay launchable
-    size_t limit = smem;
-    for (const auto& e : ctx->grid_cache)
-        if (e.fn == fn && e.smem > limit) limit = e.smem;
-    ORE_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    ORE_CUDA(ctx, raise_smem_limit(ctx->device, fn, smem));
     ORE_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem));
     if (occ < 1) return fail(ctx, ORE_ERR_CUDA, "kernel does not fit on an SM");
     *grid = occ * ctx->sm_count;
@@ -867,25 +919,32 @@ static int frame_rows(const ore_frame* fr) {
     return full * yb + (rem < yb ? rem : yb);
 }
 
-// the instantiation of each render kernel that a frame's flags select, indexed [exhaustive][staged][fast libm] (the
-// indices the kernel has)
+// the instantiation of each render kernel that a frame's scene and flags select, indexed [large scene][exhaustive]
+// [staged][fast libm] (the indices the kernel has)
 using PrimaryKernel = void (*)(FrameParams);
 using StageKernel = void (*)(FrameParams, StageArgs);
-static constexpr PrimaryKernel primary_kernels[2][2] = {
-    {primary_tile_kernel<TILE_ROWS, false, false>, primary_tile_kernel<TILE_ROWS, false, true>},
-    {primary_tile_kernel<TILE_ROWS, true, false>, primary_tile_kernel<TILE_ROWS, true, true>}};
-static constexpr StageKernel sweep_kernels[2][2][2] = {
-    {{shadow_sweep_kernel<false, false, false>, shadow_sweep_kernel<false, false, true>},
-     {shadow_sweep_kernel<false, true, false>, shadow_sweep_kernel<false, true, true>}},
-    {{shadow_sweep_kernel<true, false, false>, shadow_sweep_kernel<true, false, true>},
-     {shadow_sweep_kernel<true, true, false>, shadow_sweep_kernel<true, true, true>}}};
+static constexpr PrimaryKernel prep_kernels[2] = {prep_frame_kernel<false>, prep_frame_kernel<true>};
+static constexpr PrimaryKernel primary_kernels[2][2][2] = {
+    {{primary_tile_kernel<TILE_ROWS, false, false, false>, primary_tile_kernel<TILE_ROWS, false, true, false>},
+     {primary_tile_kernel<TILE_ROWS, true, false, false>, primary_tile_kernel<TILE_ROWS, true, true, false>}},
+    {{primary_tile_kernel<TILE_ROWS, false, false, true>, primary_tile_kernel<TILE_ROWS, false, true, true>},
+     {primary_tile_kernel<TILE_ROWS, true, false, true>, primary_tile_kernel<TILE_ROWS, true, true, true>}}};
+static constexpr StageKernel sweep_kernels[2][2][2][2] = {
+    {{{shadow_sweep_kernel<false, false, false, false>, shadow_sweep_kernel<false, false, true, false>},
+      {shadow_sweep_kernel<false, true, false, false>, shadow_sweep_kernel<false, true, true, false>}},
+     {{shadow_sweep_kernel<true, false, false, false>, shadow_sweep_kernel<true, false, true, false>},
+      {shadow_sweep_kernel<true, true, false, false>, shadow_sweep_kernel<true, true, true, false>}}},
+    {{{shadow_sweep_kernel<false, false, false, true>, shadow_sweep_kernel<false, false, true, true>},
+      {shadow_sweep_kernel<false, true, false, true>, shadow_sweep_kernel<false, true, true, true>}},
+     {{shadow_sweep_kernel<true, false, false, true>, shadow_sweep_kernel<true, false, true, true>},
+      {shadow_sweep_kernel<true, true, false, true>, shadow_sweep_kernel<true, true, true, true>}}}};
 static constexpr StageKernel shade_setup_kernels[2] = {shade_setup_kernel<false>, shade_setup_kernel<true>};
 
 // one launch of the sweep kernel (stage B / fused / catch-all)
 static int launch_sweep(ore_context* ctx, const FrameParams& prm, const StageArgs& st, bool staged, bool exh, bool fast_libm,
                         cudaStream_t stream) {
     int rc, grid = 0;
-    const StageKernel sweep = sweep_kernels[exh][staged][fast_libm];
+    const StageKernel sweep = sweep_kernels[prm.n_hypers_pad > 0][exh][staged][fast_libm];
     if ((rc = grid_for(ctx, sweep, SWEEP_SMEM_BYTES, &grid, SWEEP_THREADS))) return rc;
     sweep<<<grid, SWEEP_THREADS, SWEEP_SMEM_BYTES, stream>>>(prm, st);
     ORE_CUDA(ctx, cudaGetLastError());
@@ -992,10 +1051,20 @@ static FrameParams frame_params(const ore_context* ctx, const ore_camera* cams, 
     prm.cone_sorted = ctx->cone_sorted;
     prm.leaf_cone = ctx->leaf_cone;
     prm.super_cone = ctx->super_cone;
-    const size_t tree_bytes = ((size_t)ctx->n_supers_pad + (size_t)ctx->n_leaves_pad) * sizeof(float4);
-    const size_t all_bytes = tree_bytes + (size_t)ctx->n_sort * sizeof(float4);
-    prm.cone_resident = all_bytes <= PRIMARY_RESIDENT_BYTES ? 1 : 0;
-    *psmem = prm.cone_resident ? all_bytes : tree_bytes;
+    if (ctx->n_hypers_pad) {
+        // large scene: only the hyper-cluster records are staged
+        prm.hyper_sph = ctx->hyper_sph;
+        prm.hyper_cone = ctx->hyper_cone;
+        prm.n_hypers = ctx->n_hypers;
+        prm.n_hypers_pad = ctx->n_hypers_pad;
+        prm.cone_resident = 0;
+        *psmem = (size_t)ctx->n_hypers_pad * sizeof(float4);
+    } else {
+        const size_t tree_bytes = ((size_t)ctx->n_supers_pad + (size_t)ctx->n_leaves_pad) * sizeof(float4);
+        const size_t all_bytes = tree_bytes + (size_t)ctx->n_sort * sizeof(float4);
+        prm.cone_resident = all_bytes <= PRIMARY_RESIDENT_BYTES ? 1 : 0;
+        *psmem = prm.cone_resident ? all_bytes : tree_bytes;
+    }
     prm.tex_r = ctx->tex[0];
     prm.tex_g = ctx->tex[1];
     prm.tex_b = ctx->tex[2];
@@ -1040,12 +1109,14 @@ static int launch_frame(ore_context* ctx, const FrameParams& prm, size_t psmem, 
     int rc;
     const size_t n_px = (size_t)prm.n_px_frame * (size_t)prm.n_frames;
     const bool timing = !(prm.flags & ORE_FLAG_NO_KERNEL_TIMING);
+    const bool large = prm.n_hypers_pad > 0;
     if (timing) ORE_CUDA(ctx, cudaEventRecord(ctx->ev[0], stream));
     {
+        // (n_hypers_pad <= n_supers_pad)
         int m = prm.W_pad > prm.n_rows ? prm.W_pad : prm.n_rows;
         m = std::max(m, std::max(ctx->n_sort, std::max(ctx->n_leaves_pad, ctx->n_supers_pad)));
         m = std::max(m, std::max(ctx->n_boxes, (int)CNT_SLOTS));
-        prep_frame_kernel<<<(m + 255) / 256, 256, 0, stream>>>(prm);
+        prep_kernels[large]<<<(m + 255) / 256, 256, 0, stream>>>(prm);
         ORE_CUDA(ctx, cudaGetLastError());
         ctx->last_launches++;
     }
@@ -1056,7 +1127,7 @@ static int launch_frame(ore_context* ctx, const FrameParams& prm, size_t psmem, 
         int grid = 0;
         const long long tiles = (long long)((prm.W + 31) / 32) * ((prm.n_rows + TILE_ROWS - 1) / TILE_ROWS);
         const long long n_batches = ((tiles + PRIMARY_WARPS - 1) / PRIMARY_WARPS) * prm.n_frames;
-        const PrimaryKernel primary = primary_kernels[exh][fast_libm];
+        const PrimaryKernel primary = primary_kernels[large][exh][fast_libm];
         if ((rc = grid_for(ctx, primary, psmem, &grid, PRIMARY_THREADS))) return rc;
         if (grid > n_batches) grid = (int)n_batches;
         primary<<<grid, PRIMARY_THREADS, psmem, stream>>>(prm);
@@ -1167,6 +1238,8 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
                                 ORE_FLAG_NO_KERNEL_TIMING | ORE_FLAG_BAND_DMA))
         return fail(ctx, ORE_ERR_INVALID, "ore_render: unknown flag");
     if (!ctx->tex[0] || !ctx->sky[0]) return fail(ctx, ORE_ERR_INVALID, "ore_render: texture and sky must be set first");
+    if (ctx->n_spheres > MAX_RENDER_SPHERES)
+        return fail(ctx, ORE_ERR_INVALID, "ore_render: a scene of more than 2^24 = 16 777 216 spheres is not supported");
     if (!ctx->sph_exact) {
         int rc = upload_spheres(ctx, nullptr, 4, 0, 0);
         if (rc) return rc;
@@ -1211,7 +1284,6 @@ static int render_impl(ore_context* ctx, const ore_camera* cams, int n_frames, c
     }
     size_t psmem = 0;
     FrameParams prm = frame_params(ctx, cams, n_frames, fr, outs, band_dma, &psmem);
-    if (psmem > 200 * 1024) return fail(ctx, ORE_ERR_INVALID, "ore_render: more than ~100 000 spheres are not supported");
     if (!ctx->dbg_cycles_path.empty()) {
         const size_t nb = (n_px + 31) / 32;   // [2][nb]: stage A, stage B
         if (!ctx->dbg_cycles.fits(2 * nb)) ORE_CUDA(ctx, ctx->dbg_cycles.alloc(2 * nb));
@@ -1586,13 +1658,14 @@ extern "C" int ore_debug_libm(ore_context* ctx, int op, int n, const float* a_ho
 }
 
 extern "C" int ore_debug_sphere_tree(ore_context* ctx, int32_t which, void* host_out, int32_t n_items) {
-    if (!ctx || which < 0 || which > 5 || n_items < 0 || (n_items > 0 && !host_out)) return ORE_ERR_INVALID;
+    if (!ctx || which < 0 || which > 6 || n_items < 0 || (n_items > 0 && !host_out)) return ORE_ERR_INVALID;
     ORE_CUDA(ctx, cudaSetDevice(ctx->device));
     ORE_CUDA(ctx, cudaDeviceSynchronize());
     if (!ctx->sph_exact) return fail(ctx, ORE_ERR_INVALID, "ore_debug_sphere_tree: no spheres set");
-    const void* src[6] = {ctx->sph_exact, ctx->sph_xsort, ctx->sph_sort, ctx->sort_index, ctx->leaf_sph, ctx->super_sph};
-    const size_t count[6] = {(size_t)std::max(ctx->n_spheres, 1), (size_t)ctx->n_sort, (size_t)ctx->n_sort, (size_t)ctx->n_sort,
-                             (size_t)ctx->n_leaves_pad, (size_t)ctx->n_supers_pad};
+    if (which == 6 && !ctx->n_hypers_pad) return fail(ctx, ORE_ERR_INVALID, "ore_debug_sphere_tree: the scene has no hyper level");
+    const void* src[7] = {ctx->sph_exact, ctx->sph_xsort, ctx->sph_sort, ctx->sort_index, ctx->leaf_sph, ctx->super_sph, ctx->hyper_sph};
+    const size_t count[7] = {(size_t)std::max(ctx->n_spheres, 1), (size_t)ctx->n_sort, (size_t)ctx->n_sort, (size_t)ctx->n_sort,
+                             (size_t)ctx->n_leaves_pad, (size_t)ctx->n_supers_pad, (size_t)ctx->n_hypers_pad};
     if ((size_t)n_items != count[which]) return fail(ctx, ORE_ERR_INVALID, "ore_debug_sphere_tree: n_items must be the array's length");
     if (n_items > 0)
         ORE_CUDA(ctx, cudaMemcpy(host_out, src[which], (size_t)n_items * (which == 3 ? sizeof(int) : sizeof(float4)), cudaMemcpyDeviceToHost));

@@ -9,7 +9,8 @@
 // so the shadow sweep and the primary kernel test supers first, open the leaves of the survivors and only then single
 // spheres (DESIGN.md 2.4).  Soundness rests on one property, which tests/test_clusters_cpu.py checks: every member ball
 // (centre, R') lies inside the ball of its leaf AND inside the ball of its super-cluster, or that radius is +inf
-// ("always open": a member with non-finite or >= 1e15 coordinates / radius).
+// ("always open": a member with non-finite or >= 1e15 coordinates / radius).  Large scenes get a fourth level of
+// HYPER-clusters over the supers (build_hypers below; tests/test_hyper_clusters_cpu.py checks the same property).
 //
 // Every ORE_HD helper is compiled for both sides.  The library is built with --fmad=false and the host side with g++
 // without FMA, so the same double / float expressions give the same bits on the host and on the device.
@@ -212,6 +213,20 @@ inline void build_hierarchy(const std::vector<Rec4>& sorted_shadow, int n, std::
         leaves[j] = bounding_ball(sorted_shadow, j * LEAF_SPHERES, std::min((j + 1) * LEAF_SPHERES, (size_t)n));
     const size_t per = (size_t)LEAF_SPHERES * SUPER_LEAVES;
     for (size_t k = 0; k < n_sup; k++) supers[k] = bounding_ball(sorted_shadow, k * per, std::min((k + 1) * per, (size_t)n));
+}
+
+// A fourth level for large scenes (ore_capi.cu: n >= the large-scene threshold): HYPER-clusters of 32 consecutive
+// super-clusters (8192 spheres), each the bounding ball of its super balls taken as member balls.  Every sphere ball
+// lies inside its super ball and every super ball inside its hyper ball, so containment holds by transitivity; an
+// unboundable super (radius +inf) makes its hyper +inf too.  hypers: ceil(n_supers / 32) entries rounded up to a
+// multiple of 4 (padding = radius -1: never touched).
+constexpr int HYPER_SUPERS = 32;
+inline void build_hypers(const std::vector<Rec4>& supers, int n_supers, std::vector<Rec4>& hypers) {
+    const size_t n_sup = (size_t)std::max(n_supers, 0);
+    const size_t n_hyp = (n_sup + HYPER_SUPERS - 1) / HYPER_SUPERS;
+    hypers.assign((n_hyp + 3) & ~(size_t)3, Rec4{0.f, 0.f, 0.f, -1.f});
+    for (size_t h = 0; h < n_hyp; h++)
+        hypers[h] = bounding_ball(supers, h * HYPER_SUPERS, std::min((h + 1) * HYPER_SUPERS, n_sup));
 }
 
 }  // namespace ore_host

@@ -150,6 +150,12 @@ struct FrameParams {
     uint32_t* dbg_cycles;
     uint32_t dbg_cap;
     LightP lights[MAX_LIGHTS];
+    // large scenes only (the LARGE kernel instantiations; n_hypers_pad = 0 otherwise): hyper-cluster h = super-clusters
+    // [32h, 32h+32) with its bounding ball, and its tile-cone record per frame (frame f at hyper_cone + f * n_hypers_pad).
+    // (Last in the struct: the offsets of the fields above, and with them the code of the other instantiations, stay as they are.)
+    const float4* hyper_sph;
+    float4* hyper_cone;
+    int n_hypers, n_hypers_pad;
 };
 
 // cosf/sinf((float)j/10*2.f*3.1415f), kernel.cu:1454,1462-1463 - ten frame-independent

@@ -2,8 +2,8 @@
 //
 //   prep_frame_kernel   : per-frame tables (dx per column, dy per rendered row, in the reference's double arithmetic)
 //                         and the camera-space filter records of every sphere (in the Morton order of the upload), of
-//                         every LEAF (8 consecutive spheres) and of every SUPER-cluster (32 leaves); same for the leaf
-//                         boxes of a mesh.
+//                         every LEAF (8 consecutive spheres), of every SUPER-cluster (32 leaves) and, in a large scene,
+//                         of every HYPER-cluster (32 supers); same for the leaf boxes of a mesh.
 //   primary_tile_kernel : nearest hit (castRay, kernel.cu:1288-1431) for tiles of 32 x 8 pixels, one warp per tile:
 //                           1. the tile's bounding cone against the super-clusters, then the leaves, then - four
 //                              surviving leaves per step - the spheres (records staged in shared memory by TMA bulk
@@ -21,6 +21,7 @@
 //                              more than its own error bound; the few pixels near a boundary (and those near the
 //                              poles) are queued in shared memory and run the exact sequence 32 at a time.
 //                         Warps fetch tiles dynamically (tile cost varies ~8x between sky and sphere tiles).
+//                         Large scenes (LARGE) start the walk of step 1 one level higher, at the hyper-clusters.
 #pragma once
 
 namespace ore {
@@ -35,6 +36,7 @@ constexpr int PRIMARY_THREADS = ORE_PRIMARY_THREADS;
 constexpr int PRIMARY_WARPS = PRIMARY_THREADS / 32;
 constexpr int LEAF_SPHERES = 8;    // = ore_host::LEAF_SPHERES (ore_clusters.h)
 constexpr int SUPER_LEAVES = 32;   // = ore_host::SUPER_LEAVES
+constexpr int HYPER_SUPERS = 32;   // = ore_host::HYPER_SUPERS
 
 // Tile-cone record of a ball (centre c, radius R) seen from the eye O (DESIGN.md 2.4): a pixel tile whose directions
 // lie within `a` of its axis A can only contain a hit if  A.M + cos(a) sv - sin(a) sqrt(LL - sv^2) <= 0  with
@@ -60,6 +62,7 @@ __device__ __forceinline__ void ball_records(const FrameParams& prm, const CamP&
     *cone = make_float4((float)Mx, (float)My, (float)Mz, (float)(Wd - 4e-6 * sqrt(LL) - 1e-30));
 }
 
+template <bool LARGE>
 __global__ void prep_frame_kernel(const FrameParams prm) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < CNT_SLOTS) prm.counters[i] = 0ull;
@@ -105,6 +108,14 @@ __global__ void prep_frame_kernel(const FrameParams prm) {
                 ball_records(prm, cam, (double)cam.Ox - q.x, (double)cam.Oy - q.y, (double)cam.Oz - q.z, (double)q.w * q.w, nullptr, &cone);
             }
             prm.super_cone[(size_t)f * prm.n_supers_pad + i] = cone;
+        }
+        if (LARGE && i < prm.n_hypers_pad) {
+            float4 cone = make_float4(0.f, 0.f, 0.f, ORE_BIG);
+            if (i < prm.n_hypers) {
+                const float4 q = prm.hyper_sph[i];
+                ball_records(prm, cam, (double)cam.Ox - q.x, (double)cam.Oy - q.y, (double)cam.Oz - q.z, (double)q.w * q.w, nullptr, &cone);
+            }
+            prm.hyper_cone[(size_t)f * prm.n_hypers_pad + i] = cone;
         }
         if (i < prm.n_boxes && i < __ldg(prm.n_live_boxes)) {
             // tile-cone record of leaf box i of the mesh from its bounding sphere (same formula).  An eye on a face plane
@@ -250,7 +261,11 @@ __device__ __forceinline__ bool cone_touches(float ax, float ay, float az, const
     return fmaf(ax, rec.x, fmaf(ay, rec.y, fmaf(az, rec.z, rec.w))) <= 0.f;
 }
 
-template <int P, bool EXH, bool FAST_LIBM>
+// LARGE: the large-scene variant (FrameParams::hyper_cone).  Only the hyper-cluster records are staged in shared memory
+// (<= 32 KB up to 2^24 spheres); the walk is hyper -> super -> leaf -> sphere, with the super, leaf and sphere records
+// read through the read-only path (L2-resident: about 18 MB per frame at 1M spheres).  Everything past the leaf level
+// is the same code as in the other instantiations.
+template <int P, bool EXH, bool FAST_LIBM, bool LARGE>
 __global__ void __launch_bounds__(PRIMARY_THREADS, ORE_PRIMARY_MIN_CTAS) primary_tile_kernel(const FrameParams prm) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t bar;
@@ -266,9 +281,13 @@ __global__ void __launch_bounds__(PRIMARY_THREADS, ORE_PRIMARY_MIN_CTAS) primary
     // ---- the cone records of ONE frame at a time are staged in shared memory: [supers][leaves][spheres, when they fit]
     //      - one TMA bulk copy each, shared by the CTA's warps for all their tiles of that frame.  Batches are fetched
     //      in ascending order, so a CTA restages at most once per frame of the batch. ----
+    //      (LARGE: [hypers] only.) ----
     float4* const s_super = reinterpret_cast<float4*>(smem_raw);
     float4* const s_leaf = s_super + prm.n_supers_pad;
     float4* const s_sph = s_leaf + prm.n_leaves_pad;
+    const float4* const s_hyper = reinterpret_cast<const float4*>(smem_raw);
+    const float4* __restrict__ g_super = nullptr;   // LARGE: this frame's super and leaf records in global memory
+    const float4* __restrict__ g_leaf = nullptr;
     if (tid == 0) {
         mbar_init(&bar, 1);
         mbar_fence_init();
@@ -301,19 +320,31 @@ __global__ void __launch_bounds__(PRIMARY_THREADS, ORE_PRIMARY_MIN_CTAS) primary
             // (every warp is past its reads of the previous frame's records: it has gone through the barriers of the
             // previous batch since)
             __syncthreads();
-            if (tid == 0) {
-                const uint32_t b_sup = (uint32_t)prm.n_supers_pad * 16u, b_leaf = (uint32_t)prm.n_leaves_pad * 16u;
-                const uint32_t b_sph = prm.cone_resident ? (uint32_t)prm.n_sort * 16u : 0u;
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                mbar_expect_tx(&bar, b_sup + b_leaf + b_sph);
-                if (b_sup) tma_bulk_g2s(s_super, prm.super_cone + (size_t)frame * prm.n_supers_pad, b_sup, &bar);
-                if (b_leaf) tma_bulk_g2s(s_leaf, prm.leaf_cone + (size_t)frame * prm.n_leaves_pad, b_leaf, &bar);
-                if (b_sph) tma_bulk_g2s(s_sph, prm.cone_sorted + (size_t)frame * prm.n_sort, b_sph, &bar);
+            if constexpr (LARGE) {
+                if (tid == 0) {
+                    const uint32_t b_hyp = (uint32_t)prm.n_hypers_pad * 16u;
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    mbar_expect_tx(&bar, b_hyp);
+                    if (b_hyp) tma_bulk_g2s(smem_raw, prm.hyper_cone + (size_t)frame * prm.n_hypers_pad, b_hyp, &bar);
+                }
+                g_super = prm.super_cone + (size_t)frame * prm.n_supers_pad;
+                g_leaf = prm.leaf_cone + (size_t)frame * prm.n_leaves_pad;
+                sph_cone = prm.cone_sorted + (size_t)frame * prm.n_sort;
+            } else {
+                if (tid == 0) {
+                    const uint32_t b_sup = (uint32_t)prm.n_supers_pad * 16u, b_leaf = (uint32_t)prm.n_leaves_pad * 16u;
+                    const uint32_t b_sph = prm.cone_resident ? (uint32_t)prm.n_sort * 16u : 0u;
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    mbar_expect_tx(&bar, b_sup + b_leaf + b_sph);
+                    if (b_sup) tma_bulk_g2s(s_super, prm.super_cone + (size_t)frame * prm.n_supers_pad, b_sup, &bar);
+                    if (b_leaf) tma_bulk_g2s(s_leaf, prm.leaf_cone + (size_t)frame * prm.n_leaves_pad, b_leaf, &bar);
+                    if (b_sph) tma_bulk_g2s(s_sph, prm.cone_sorted + (size_t)frame * prm.n_sort, b_sph, &bar);
+                }
             }
             mbar_wait(&bar, bar_phase);
             bar_phase ^= 1u;
             staged_frame = frame;
-            sph_cone = prm.cone_resident ? s_sph : prm.cone_sorted + (size_t)frame * prm.n_sort;
+            if constexpr (!LARGE) sph_cone = prm.cone_resident ? s_sph : prm.cone_sorted + (size_t)frame * prm.n_sort;
         }
         const CamP cam = prm.cam[frame];
         const v3 O = mk(cam.Ox, cam.Oy, cam.Oz);
@@ -379,65 +410,95 @@ __global__ void __launch_bounds__(PRIMARY_THREADS, ORE_PRIMARY_MIN_CTAS) primary
             }
         }
 
-        // ---- spheres: super-clusters -> leaves -> (four leaves per step) spheres -> per-pixel filter -> exact ----
-#pragma unroll 1
-        for (int s0 = 0; s0 < n_sup; s0 += 32) {
-            uint32_t smask = __ballot_sync(0xffffffffu, tile_ok && s0 + lane < n_sup &&
-                                                            (EXH || cone_touches(ax, ay, az, s_super[min(s0 + lane, n_sup - 1)])));
+        // ---- spheres: (LARGE: hyper-clusters ->) super-clusters -> leaves -> (four leaves per step) spheres ->
+        //      per-pixel filter -> exact.  open_super is everything below the super level. ----
+        auto open_super = [&](const int sup) {
+            const int leaf = sup * SUPER_LEAVES + lane;
+            const int lc = min(leaf, n_leaf - 1);
+            uint32_t cmask = __ballot_sync(0xffffffffu, leaf < n_leaf && (EXH || cone_touches(ax, ay, az, LARGE ? __ldg(&g_leaf[lc]) : s_leaf[lc])));
             n_steps++;
 #pragma unroll 1
-            while (smask) {
-                const int sup = s0 + __ffs(smask) - 1;
-                smask &= smask - 1;
-                const int leaf = sup * SUPER_LEAVES + lane;
-                uint32_t cmask = __ballot_sync(0xffffffffu, leaf < n_leaf && (EXH || cone_touches(ax, ay, az, s_leaf[min(leaf, n_leaf - 1)])));
+            while (cmask) {
+                int mine = -1;
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    const int c = cmask ? __ffs(cmask) - 1 : -1;
+                    cmask &= cmask - 1;
+                    if ((lane >> 3) == k) mine = c;
+                }
+                const int s_mine = mine >= 0 ? (sup * SUPER_LEAVES + mine) * LEAF_SPHERES + (lane & 7) : n_sph;
+                const bool in = s_mine < n_sph;
+                const int sc = in ? s_mine : 0;
+                uint32_t wmask = __ballot_sync(0xffffffffu, in && (EXH || cone_touches(ax, ay, az, LARGE ? __ldg(&sph_cone[sc]) : sph_cone[sc])));
                 n_steps++;
-#pragma unroll 1
-                while (cmask) {
-                    int mine = -1;
+                while (wmask) {
+                    const int i = __ffs(wmask) - 1;
+                    wmask &= wmask - 1;
+                    const int s = __shfl_sync(0xffffffffu, s_mine, i);
+                    const float4 q = __ldg(&prim_rec[s]);
+                    const float e = fmaf(dx, q.x, q.z);
+                    uint32_t pass = 0;
 #pragma unroll
-                    for (int k = 0; k < 4; k++) {
-                        const int c = cmask ? __ffs(cmask) - 1 : -1;
-                        cmask &= cmask - 1;
-                        if ((lane >> 3) == k) mine = c;
-                    }
-                    const int s_mine = mine >= 0 ? (sup * SUPER_LEAVES + mine) * LEAF_SPHERES + (lane & 7) : n_sph;
-                    const bool in = s_mine < n_sph;
-                    uint32_t wmask = __ballot_sync(0xffffffffu, in && (EXH || cone_touches(ax, ay, az, sph_cone[in ? s_mine : 0])));
-                    n_steps++;
-                    while (wmask) {
-                        const int i = __ffs(wmask) - 1;
-                        wmask &= wmask - 1;
-                        const int s = __shfl_sync(0xffffffffu, s_mine, i);
-                        const float4 q = __ldg(&prim_rec[s]);
-                        const float e = fmaf(dx, q.x, q.z);
-                        uint32_t pass = 0;
+                    for (int p = 0; p < P; p++) pass |= (fmaf(dyp[p], q.y, e) <= negn[p]) ? (1u << p) : 0u;
+                    if (pass) {
+                        const float4 ex = __ldg(&prm.sph_xsort[s]);
+                        const int id = __ldg(&prm.sort_index[s]);
 #pragma unroll
-                        for (int p = 0; p < P; p++) pass |= (fmaf(dyp[p], q.y, e) <= negn[p]) ? (1u << p) : 0u;
-                        if (pass) {
-                            const float4 ex = __ldg(&prm.sph_xsort[s]);
-                            const int id = __ldg(&prm.sort_index[s]);
-#pragma unroll
-                            for (int p = 0; p < P; p++) {
-                                if ((pass >> p) & 1u) {
-                                    const v3 D = primary_dir_call(da, dx, dyp[p]);
-                                    float t;
-                                    n_exact++;
-                                    if (ref_intersect(O, D, ex.x, ex.y, ex.z, ex.w, t)) {
-                                        // kernel.cu:1335 visits the spheres in ascending index with a strict '<': the
-                                        // winner is the smallest t and, among equal t, the lowest sphere index - but
-                                        // never a sphere against a triangle found before it with the same t
-                                        const bool better = t < best_t[p] ||
-                                                            (t == best_t[p] && best_id[p] >= 0 && best_id[p] < n_sph && id < best_id[p]);
-                                        if (better) {
-                                            best_t[p] = t;
-                                            best_id[p] = id;
-                                        }
+                        for (int p = 0; p < P; p++) {
+                            if ((pass >> p) & 1u) {
+                                const v3 D = primary_dir_call(da, dx, dyp[p]);
+                                float t;
+                                n_exact++;
+                                if (ref_intersect(O, D, ex.x, ex.y, ex.z, ex.w, t)) {
+                                    // kernel.cu:1335 visits the spheres in ascending index with a strict '<': the
+                                    // winner is the smallest t and, among equal t, the lowest sphere index - but
+                                    // never a sphere against a triangle found before it with the same t
+                                    const bool better = t < best_t[p] ||
+                                                        (t == best_t[p] && best_id[p] >= 0 && best_id[p] < n_sph && id < best_id[p]);
+                                    if (better) {
+                                        best_t[p] = t;
+                                        best_id[p] = id;
                                     }
                                 }
                             }
                         }
                     }
+                }
+            }
+        };
+        if constexpr (LARGE) {
+            const int n_hyp = prm.n_hypers;
+#pragma unroll 1
+            for (int h0 = 0; h0 < n_hyp; h0 += 32) {
+                uint32_t hmask = __ballot_sync(0xffffffffu, tile_ok && h0 + lane < n_hyp &&
+                                                                (EXH || cone_touches(ax, ay, az, s_hyper[min(h0 + lane, n_hyp - 1)])));
+                n_steps++;
+#pragma unroll 1
+                while (hmask) {
+                    const int hyp = h0 + __ffs(hmask) - 1;
+                    hmask &= hmask - 1;
+                    const int sl = hyp * HYPER_SUPERS + lane;
+                    uint32_t smask = __ballot_sync(0xffffffffu, sl < n_sup && (EXH || cone_touches(ax, ay, az, __ldg(&g_super[min(sl, n_sup - 1)]))));
+                    n_steps++;
+#pragma unroll 1
+                    while (smask) {
+                        const int sup = hyp * HYPER_SUPERS + __ffs(smask) - 1;
+                        smask &= smask - 1;
+                        open_super(sup);
+                    }
+                }
+            }
+        } else {
+#pragma unroll 1
+            for (int s0 = 0; s0 < n_sup; s0 += 32) {
+                uint32_t smask = __ballot_sync(0xffffffffu, tile_ok && s0 + lane < n_sup &&
+                                                                (EXH || cone_touches(ax, ay, az, s_super[min(s0 + lane, n_sup - 1)])));
+                n_steps++;
+#pragma unroll 1
+                while (smask) {
+                    const int sup = s0 + __ffs(smask) - 1;
+                    smask &= smask - 1;
+                    open_super(sup);
                 }
             }
         }

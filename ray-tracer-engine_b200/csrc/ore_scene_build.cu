@@ -7,6 +7,7 @@
 //   scene_gather_kernel  sorted exact + shadow records (R' = shadow_radius), sort_index, padding to 32
 //   scene_balls_kernel   leaf balls (one thread per leaf: bounding_ball itself) and super balls (one warp per super:
 //                        box and max radius reduced across lanes, the mean summed by one lane in member order)
+//   scene_hypers_kernel  large scenes only: hyper balls over the super balls (one thread per hyper: bounding_ball)
 //
 // Every value is computed by the ORE_HD helpers the host builder uses, with the same double expressions; only the
 // order of min / max reductions differs, and min / max of finite values do not depend on it.  So the arrays are
@@ -189,6 +190,19 @@ __global__ void __launch_bounds__(BUILD_THREADS) scene_balls_kernel(const float4
     if ((threadIdx.x & 31) == 0) super_sph[k] = as_f4(b);
 }
 
+// large scenes only: one thread per hyper-cluster, bounding_ball itself over its <= 32 super balls (padding: radius -1)
+__global__ void __launch_bounds__(BUILD_THREADS) scene_hypers_kernel(const float4* super_sph, int n_supers, float4* hyper_sph,
+                                                                     int n_hypers, int n_hypers_pad) {
+    const int h = blockIdx.x * blockDim.x + threadIdx.x;
+    if (h >= n_hypers_pad) return;
+    if (h >= n_hypers) {
+        hyper_sph[h] = make_float4(0.f, 0.f, 0.f, -1.f);
+        return;
+    }
+    const int k0 = h * ore_host::HYPER_SUPERS, m = min(ore_host::HYPER_SUPERS, n_supers - k0);
+    hyper_sph[h] = as_f4(ore_host::bounding_ball(reinterpret_cast<const Rec4*>(super_sph + k0), (size_t)m));
+}
+
 }  // namespace
 
 cudaError_t ore_scene_sort_bytes(int n, size_t* bytes) {
@@ -222,5 +236,8 @@ cudaError_t ore_scene_build(const SceneBuildArgs& a, cudaStream_t stream) {
                                                                                       a.n_leaves_pad, a.super_sph, a.n_supers,
                                                                                       a.n_supers_pad, leaf_blocks);
     }
+    if (a.n_hypers_pad > 0)
+        scene_hypers_kernel<<<(a.n_hypers_pad + BUILD_THREADS - 1) / BUILD_THREADS, BUILD_THREADS, 0, stream>>>(
+            a.super_sph, a.n_supers, a.hyper_sph, a.n_hypers, a.n_hypers_pad);
     return cudaGetLastError();
 }

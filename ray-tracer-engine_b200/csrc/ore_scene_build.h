@@ -1,7 +1,8 @@
 // ore_scene_build.h - the sphere hierarchy built on the device (ore_scene_build.cu), enqueued on a stream.
 //
 // Input: n records (cx, cy, cz, radius member) in device memory.  Output: the scene arrays of ore_capi.cu - the
-// records in original order, both sorted arrays, the permutation and the leaf / super-cluster balls - bit-identical to
+// records in original order, both sorted arrays, the permutation, the leaf / super-cluster balls and, for a large scene,
+// the hyper-cluster balls - bit-identical to
 // what the host builder of ore_clusters.h gives for the same values (DESIGN.md "Device build of the sphere hierarchy").
 #pragma once
 #include <cuda_runtime.h>
@@ -18,6 +19,8 @@ struct SceneBuildArgs {
     float4* leaf_sph;      // n_leaves_pad balls (padding: radius -1)
     float4* super_sph;     // n_supers_pad balls (padding: radius -1)
     int n_sort, n_leaves, n_leaves_pad, n_supers, n_supers_pad;
+    float4* hyper_sph;     // n_hypers_pad balls over 32 supers each (padding: radius -1); n_hypers_pad = 0: not built
+    int n_hypers, n_hypers_pad;
     // work space, all sized by the caller for at least n items
     uint32_t* keys_in;
     uint32_t* keys_out;

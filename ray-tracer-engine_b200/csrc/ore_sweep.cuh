@@ -64,7 +64,9 @@ __device__ __forceinline__ bool beam_touches(const Beam& b, const float4 q) {
     return !(q.w < 1e18f) || (u >= 0.f && d2 <= fmaf(thr, thr, slack));
 }
 
-template <bool EXH, bool STAGED, bool FAST_LIBM>
+// LARGE: the large-scene variant, with a level-H pass over the hyper-cluster balls (FrameParams::hyper_sph) before the
+// super level; everything from the super level down is the same code as in the other instantiations.
+template <bool EXH, bool STAGED, bool FAST_LIBM, bool LARGE>
 __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_kernel(const FrameParams prm, const StageArgs st) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -319,84 +321,114 @@ __global__ void __launch_bounds__(SWEEP_THREADS, SWEEP_MIN_CTAS) shadow_sweep_ke
                 if (EXH) wforce = true;
 
                 bool warp_done = false;
-#pragma unroll 1
-                for (int s0 = 0; s0 < n_sup && !warp_done; s0 += 32) {
-                    // ---- level S: lane i tests super-cluster s0 + i (256 spheres) ----
-                    uint32_t smask = __ballot_sync(0xffffffffu, s0 + lane < n_sup && (wforce || beam_touches(bm, __ldg(&supers[min(s0 + lane, n_sup - 1)]))));
+                // everything below the super level, for super-cluster `sup`
+                auto open_super = [&](const int sup) {
+                    // ---- level 0: lane i tests leaf sup * 32 + i (8 spheres) ----
+                    const int leaf = sup * 32 + lane;
+                    uint32_t cmask = __ballot_sync(0xffffffffu, leaf < n_leaf && (wforce || beam_touches(bm, __ldg(&leaves[min(leaf, n_leaf - 1)]))));
                     n_steps++;
 #pragma unroll 1
-                    while (smask && !warp_done) {
-                        const int sup = s0 + __ffs(smask) - 1;
-                        smask &= smask - 1;
-                        // ---- level 0: lane i tests leaf sup * 32 + i (8 spheres) ----
-                        const int leaf = sup * 32 + lane;
-                        uint32_t cmask = __ballot_sync(0xffffffffu, leaf < n_leaf && (wforce || beam_touches(bm, __ldg(&leaves[min(leaf, n_leaf - 1)]))));
+                    while (cmask && !warp_done) {
+                        // ---- level 1, dense: the four lowest surviving leaves, lane i tests sphere i % 8 of leaf i / 8 ----
+                        int mine = -1;
+#pragma unroll
+                        for (int k = 0; k < 4; k++) {
+                            const int c = cmask ? __ffs(cmask) - 1 : -1;
+                            cmask &= cmask - 1;   // (0 & -1 = 0)
+                            if ((lane >> 3) == k) mine = c;
+                        }
+                        const int s_mine = mine >= 0 ? (sup * 32 + mine) * 8 + (lane & 7) : n_sph;
+                        const bool in = s_mine < n_sph;
+                        uint32_t wmask = __ballot_sync(0xffffffffu, in && (wforce || beam_touches(bm, __ldg(&spheres[in ? s_mine : 0]))));
+                        n_steps++;
+                        n_l1 += __popc(wmask);
+                        // ---- level 2: every lane of the group runs its own cone test on the surviving spheres ----
+                        while (wmask) {
+                            const int i = __ffs(wmask) - 1;
+                            wmask &= wmask - 1;
+                            const int s = __shfl_sync(0xffffffffu, s_mine, i);
+                            const float4 q = __ldg(&spheres[s]);
+                            const float lx = start.x - q.x, ly = start.y - q.y, lz = start.z - q.z;
+                            const float LL = fmaf(lz, lz, fmaf(ly, ly, lx * lx));
+                            const float Cm = fmaf(LL, 1.0f - ORE_KAPPA_SHADOW, -(q.w * q.w));
+                            const float sq = Cm * rsqrt_approx(Cm);
+                            const float svu = (EXH || !(Cm > 1e-20f)) ? -ORE_BIG : sq;
+                            uint32_t live = ing ? (~blocked & 0x3ffu) : 0u;
+                            if (!force) {
+                                const float T = fmaf(ca, svu, -(sa * q.w));
+                                if (!(fmaf(Ax, lx, fmaf(Ay, ly, fmaf(Az, lz, T))) < 0.f)) live = 0u;
+                            }
+                            if (live) {
+                                n_l2++;
+                                const float4 ex4 = __ldg(&prm.sph_xsort[s]);
+                                // per-ray filter h = D.L + s' < 0 on the 10 rays (shared-memory directions), the "sure
+                                // hit" shortcut (DESIGN.md 2.5), then the exact sequence on what lies in between
+                                const float sure_thr = (EXH || force)
+                                                           ? INFINITY
+                                                           : fmaxf(fmaf(LL, 1e-6f, 1e-6f), fmaf(LL, 2e-5f, fmaf(-ex4.w, ex4.w, LL)));
+                                uint32_t m = 0, sure = 0;
+#pragma unroll
+                                for (int j = 0; j < 10; j++) {
+                                    const float b = fmaf(dslot[(3 * j) * 32], lx, fmaf(dslot[(3 * j + 1) * 32], ly, dslot[(3 * j + 2) * 32] * lz));
+                                    if (b + svu < 0.f) m |= 1u << j;
+                                    if (b < 0.f && b * b > sure_thr) sure |= 1u << j;
+                                }
+                                sure &= m & live;  // only rays the filter lets through, that are still unblocked
+                                blocked |= sure;
+                                uint32_t cand = m & live & ~sure;
+                                while (cand) {
+                                    const int j = __ffs(cand) - 1;
+                                    cand &= cand - 1;
+                                    float t;
+                                    n_exact++;
+                                    if (ref_intersect(start, dir_at(dslot, 32, j), ex4.x, ex4.y, ex4.z, ex4.w, t)) blocked |= 1u << j;
+                                }
+                                if (blocked == 0x3ffu) {   // all 10 rays of this light are blocked: the lane drops out
+                                    Ax = Ay = Az = 0.f;
+                                    ca = 0.f;
+                                    sa = 0.f;
+                                    force = false;
+                                }
+                            }
+                        }
+                        if (__all_sync(0xffffffffu, !ing || blocked == 0x3ffu)) warp_done = true;
+                    }
+                };
+                if constexpr (LARGE) {
+                    const float4* __restrict__ hypers = prm.hyper_sph;   // bounding ball of supers [32h, 32h+32)
+                    const int n_hyp = prm.n_hypers;
+#pragma unroll 1
+                    for (int h0 = 0; h0 < n_hyp && !warp_done; h0 += 32) {
+                        // ---- level H: lane i tests hyper-cluster h0 + i (8192 spheres) ----
+                        uint32_t hmask = __ballot_sync(0xffffffffu, h0 + lane < n_hyp && (wforce || beam_touches(bm, __ldg(&hypers[min(h0 + lane, n_hyp - 1)]))));
                         n_steps++;
 #pragma unroll 1
-                        while (cmask && !warp_done) {
-                            // ---- level 1, dense: the four lowest surviving leaves, lane i tests sphere i % 8 of leaf i / 8 ----
-                            int mine = -1;
-#pragma unroll
-                            for (int k = 0; k < 4; k++) {
-                                const int c = cmask ? __ffs(cmask) - 1 : -1;
-                                cmask &= cmask - 1;   // (0 & -1 = 0)
-                                if ((lane >> 3) == k) mine = c;
-                            }
-                            const int s_mine = mine >= 0 ? (sup * 32 + mine) * 8 + (lane & 7) : n_sph;
-                            const bool in = s_mine < n_sph;
-                            uint32_t wmask = __ballot_sync(0xffffffffu, in && (wforce || beam_touches(bm, __ldg(&spheres[in ? s_mine : 0]))));
+                        while (hmask && !warp_done) {
+                            const int hyp = h0 + __ffs(hmask) - 1;
+                            hmask &= hmask - 1;
+                            // ---- level S: lane i tests super-cluster hyp * 32 + i ----
+                            const int sl = hyp * 32 + lane;
+                            uint32_t smask = __ballot_sync(0xffffffffu, sl < n_sup && (wforce || beam_touches(bm, __ldg(&supers[min(sl, n_sup - 1)]))));
                             n_steps++;
-                            n_l1 += __popc(wmask);
-                            // ---- level 2: every lane of the group runs its own cone test on the surviving spheres ----
-                            while (wmask) {
-                                const int i = __ffs(wmask) - 1;
-                                wmask &= wmask - 1;
-                                const int s = __shfl_sync(0xffffffffu, s_mine, i);
-                                const float4 q = __ldg(&spheres[s]);
-                                const float lx = start.x - q.x, ly = start.y - q.y, lz = start.z - q.z;
-                                const float LL = fmaf(lz, lz, fmaf(ly, ly, lx * lx));
-                                const float Cm = fmaf(LL, 1.0f - ORE_KAPPA_SHADOW, -(q.w * q.w));
-                                const float sq = Cm * rsqrt_approx(Cm);
-                                const float svu = (EXH || !(Cm > 1e-20f)) ? -ORE_BIG : sq;
-                                uint32_t live = ing ? (~blocked & 0x3ffu) : 0u;
-                                if (!force) {
-                                    const float T = fmaf(ca, svu, -(sa * q.w));
-                                    if (!(fmaf(Ax, lx, fmaf(Ay, ly, fmaf(Az, lz, T))) < 0.f)) live = 0u;
-                                }
-                                if (live) {
-                                    n_l2++;
-                                    const float4 ex4 = __ldg(&prm.sph_xsort[s]);
-                                    // per-ray filter h = D.L + s' < 0 on the 10 rays (shared-memory directions), the "sure
-                                    // hit" shortcut (DESIGN.md 2.5), then the exact sequence on what lies in between
-                                    const float sure_thr = (EXH || force)
-                                                               ? INFINITY
-                                                               : fmaxf(fmaf(LL, 1e-6f, 1e-6f), fmaf(LL, 2e-5f, fmaf(-ex4.w, ex4.w, LL)));
-                                    uint32_t m = 0, sure = 0;
-#pragma unroll
-                                    for (int j = 0; j < 10; j++) {
-                                        const float b = fmaf(dslot[(3 * j) * 32], lx, fmaf(dslot[(3 * j + 1) * 32], ly, dslot[(3 * j + 2) * 32] * lz));
-                                        if (b + svu < 0.f) m |= 1u << j;
-                                        if (b < 0.f && b * b > sure_thr) sure |= 1u << j;
-                                    }
-                                    sure &= m & live;  // only rays the filter lets through, that are still unblocked
-                                    blocked |= sure;
-                                    uint32_t cand = m & live & ~sure;
-                                    while (cand) {
-                                        const int j = __ffs(cand) - 1;
-                                        cand &= cand - 1;
-                                        float t;
-                                        n_exact++;
-                                        if (ref_intersect(start, dir_at(dslot, 32, j), ex4.x, ex4.y, ex4.z, ex4.w, t)) blocked |= 1u << j;
-                                    }
-                                    if (blocked == 0x3ffu) {   // all 10 rays of this light are blocked: the lane drops out
-                                        Ax = Ay = Az = 0.f;
-                                        ca = 0.f;
-                                        sa = 0.f;
-                                        force = false;
-                                    }
-                                }
+#pragma unroll 1
+                            while (smask && !warp_done) {
+                                const int sup = hyp * 32 + __ffs(smask) - 1;
+                                smask &= smask - 1;
+                                open_super(sup);
                             }
-                            if (__all_sync(0xffffffffu, !ing || blocked == 0x3ffu)) warp_done = true;
+                        }
+                    }
+                } else {
+#pragma unroll 1
+                    for (int s0 = 0; s0 < n_sup && !warp_done; s0 += 32) {
+                        // ---- level S: lane i tests super-cluster s0 + i (256 spheres) ----
+                        uint32_t smask = __ballot_sync(0xffffffffu, s0 + lane < n_sup && (wforce || beam_touches(bm, __ldg(&supers[min(s0 + lane, n_sup - 1)]))));
+                        n_steps++;
+#pragma unroll 1
+                        while (smask && !warp_done) {
+                            const int sup = s0 + __ffs(smask) - 1;
+                            smask &= smask - 1;
+                            open_super(sup);
                         }
                     }
                 }
